@@ -2,7 +2,7 @@
 """bench.py — EMIT -> S2 pair synthesis (GLT ortho + SRF + polyfit + apply) on synthetic granules.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--config granule|ortho_srf|tiles|shards|mosaic]
+                    [--config granule|ortho_srf|tiles|shards|mosaic] [--dump-outputs DIR]
 
 Default (`--config granule`) = BASELINE.json configs[1], the configuration the metric is quoted on: one "step" = one pass
 of the hot path over one synthetic EMIT-granule-shaped cube per GPU (raw 1280 x 1242 x 285 fp32, 25-degree GLT ->
@@ -356,7 +356,8 @@ def timed_loop(ctx, run, steps):
 
 
 def capture(ctx, fn):
-    """fn captured into a CUDA graph (warm-up on a side stream first); returns (graph, node counts)."""
+    """fn captured into a CUDA graph (warm-up on a side stream first); returns (graph, node counts, fn's return value,
+    whose tensors every replay rewrites in place)."""
     torch = ctx.torch
     side = torch.cuda.Stream(ctx.device)
     side.wait_stream(torch.cuda.current_stream())
@@ -369,13 +370,32 @@ def capture(ctx, fn):
     except TypeError:                                  # older torch: no node introspection
         g = torch.cuda.CUDAGraph()
     with torch.cuda.graph(g):
-        fn()
+        out = fn()
     counts = graph_node_counts(g)
     try:
         g.instantiate()
     except Exception:
         pass
-    return g, counts
+    return g, counts, out
+
+
+DUMP_SAMPLE_PX = 1 << 18
+
+
+def dump_outputs(out_dir, outputs, grid_hw):
+    """--dump-outputs: each output as out_dir/<name>.npy (float64 stays float64, everything else becomes float32).
+    Per-pixel outputs ([K, Ho, Wo] planes, [Ho, Wo] masks) are kept at the same DUMP_SAMPLE_PX ortho pixels in every
+    array and every run (flat indices drawn by numpy's default_rng(0), sorted): the full planes are 135 MB each."""
+    import torch
+
+    Ho, Wo = grid_hw
+    idx = np.sort(np.random.default_rng(0).choice(Ho * Wo, size=min(Ho * Wo, DUMP_SAMPLE_PX), replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        if tuple(t.shape[-2:]) == (Ho, Wo):
+            t = t[..., torch.from_numpy(idx // Wo).to(t.device), torch.from_numpy(idx % Wo).to(t.device)]
+        a = t.cpu().numpy()
+        np.save(os.path.join(out_dir, f"{name}.npy"), a if a.dtype == np.float64 else a.astype(np.float32))
 
 
 def base_line(ctx, args, value, ms_per_step, scaling, config):
@@ -450,19 +470,29 @@ def run_granule(args, ortho_srf_only=False):
         step(si=i & 1)
     ctx.barrier()
     graphs, counts = None, None
+    coeffs_out = [None, None]      # the coefficients each input set's step returns (rewritten by every replay)
     if not args.no_graph and (not multi or px is not None or ortho_srf_only):
         # the step's launches captured once per input set and replayed: same kernels, same arguments, ~1 us between
         # dependent kernels instead of ~3 us
         graphs = []
         for si in range(2):
-            g, c = capture(ctx, lambda si=si: step(si=si))
+            g, c, coeffs_out[si] = capture(ctx, lambda si=si: step(si=si))
             graphs.append(g)
             counts = c if c is not None else counts
         for i in range(4):
             graphs[i & 1].replay()
         torch.cuda.synchronize()
-    ms_total = timed_loop(ctx, (lambda i: graphs[i & 1].replay()) if graphs is not None
-                          else (lambda i: step(record=True, si=i & 1)), args.steps)
+
+    def eager_step(i):
+        coeffs_out[i & 1] = step(record=True, si=i & 1)
+
+    ms_total = timed_loop(ctx, (lambda i: graphs[i & 1].replay()) if graphs is not None else eager_step, args.steps)
+    if args.dump_outputs and rank == 0:
+        # the last timed step's outputs, before the steps below overwrite the shared buffers
+        outputs = {"bands": bands, "valid": valid_buf, "fit_mask": fit_mask}
+        if not ortho_srf_only:
+            outputs.update(matched=matched, coeffs=coeffs_out[(args.steps - 1) & 1])
+        dump_outputs(args.dump_outputs, outputs, (Ho, Wo))
     if graphs is not None:      # kernel time of the fused gather, from eager steps (events cannot be read from a replay)
         for i in range(30):
             step(record=True, si=i & 1)
@@ -872,7 +902,13 @@ def main():
     ap.add_argument("--collective", choices=["peer", "nccl", "none"], default="peer",
                     help="N > 1: moments over NVLink peer memory fused into the finalize / solve kernels (default) or one "
                          "NCCL all-reduce between them")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="granule / ortho_srf: write what the last timed step computed (rank 0's bands, matched planes, "
+                         "coefficients, valid and fit masks) as DIR/<name>.npy, per-pixel outputs at a fixed sample of "
+                         f"{DUMP_SAMPLE_PX} pixels; the inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config not in ("granule", "ortho_srf")):
+        ap.error("--dump-outputs is available for --impl ours with --config granule or ortho_srf")
     knobs = _env_knobs()
     if knobs and args.impl == "ours":
         raise SystemExit(f"bench.py refuses to run with HSR_* variables set ({', '.join(knobs)}): they select or steer the "

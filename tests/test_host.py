@@ -188,9 +188,11 @@ def test_shard_rows_balanced_by_weights():
         hdist.shard_rows(n, 0, 2, weights=w[:10])
 
 
-def test_moment_allreduce_world_size_2_gloo(tmp_path):
+def test_moment_allreduce_world_size_2_gloo(tmp_path, monkeypatch):
     import torch.multiprocessing as mp
 
+    # the workers are CPU ranks: with a GPU visible, init_from_env would bind rank 1 to cuda:1, absent on a one-GPU box
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     port = 29500 + (os.getpid() % 400)
     mp.spawn(_gloo_worker, args=(2, port, str(tmp_path)), nprocs=2, join=True)
     m0 = np.load(tmp_path / "mom_0.npy")
