@@ -50,6 +50,7 @@ struct SelSeries {
     unsigned long long lt[SEL_QMAX], eqlo[SEL_QMAX], eqhi[SEL_QMAX];
     unsigned long long count, nan;                   // masked samples (NaNs included) and NaNs among them
 };
+static_assert(sizeof(SelSeries) == 96, "tests/test_gpu_select_paths.py and profiles/prof_select.py read this layout");
 
 struct SelParams {
     const float* x[2];     // one or two plane sets (x planes, y planes); series s: set = s / S1, k = (s % S1) / G, g = s % G
@@ -779,8 +780,10 @@ int masked_percentiles_impl(const float* x, long long xks, long long xgs, const 
                             double* out, double* out2, cudaStream_t stream) {
     HSR_REQUIRE(x && q && workspace && out, HSR_EINVAL, "null x / q / workspace / out pointer");
     HSR_REQUIRE((x2 == nullptr) == (out2 == nullptr), HSR_EINVAL, "x2 and out2 must be given together");
-    HSR_REQUIRE(n >= 0 && n < (1LL << 33) && K >= 1 && G >= 1 && (long long)K * G <= 32767, HSR_ERANGE,
-                "bad n = %lld (< 2^33), K = %d or G = %d (K * G <= 32767)", n, K, G);
+    // n < 2^32: the candidate counts (SelSeries::ncand, nc) and the fallback's histogram bins are 32-bit; a wrapped ncand
+    // could pass as <= cap and send the finish kernel to a candidate list it never filled
+    HSR_REQUIRE(n >= 0 && n < (1LL << 32) && K >= 1 && G >= 1 && (long long)K * G <= 32767, HSR_ERANGE,
+                "bad n = %lld (< 2^32), K = %d or G = %d (K * G <= 32767)", n, K, G);
     HSR_REQUIRE(Q >= 1 && Q <= SEL_QMAX, HSR_ERANGE, "Q = %d outside [1, %d]", Q, SEL_QMAX);
     HSR_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(x2)) & 3) == 0, HSR_EALIGN,
                 "x not 4-byte aligned");

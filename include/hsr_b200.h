@@ -319,7 +319,7 @@ HSR_API size_t hsr_workspace_bytes(int op, int64_t n, int K, int deg);
  * masked sample at all, gives NaN (numpy raises IndexError for the empty case; the host wrapper mirrors that).
  *   q              [Q] f64 on the device, fractions in [0, 1] (percent / 100), Q <= HSR_MAX_PERCENTILES.
  *   workspace      hsr_percentiles_workspace_bytes(n, K, G, nsets) bytes, 256-byte aligned (nsets = 1; 2 for the pair).
- * K*G <= 32767.
+ * n < 2^32 (the candidate and histogram counters are 32-bit), K*G <= 32767.
  * hsr_masked_percentiles_pair_f64: the same for TWO plane sets of one shape under one mask — the two images of the
  * stretch (poly_regression.py:126-127) — in the same three launches; out_x, out_y [K*G, Q].
  *

@@ -716,7 +716,8 @@ def test_percentile_stretch_golden_through_reference_call_surface(golden):
     assert t.is_cuda and np.array_equal(bits(t), bits(g["out"]))
 
 
-@pytest.mark.parametrize("n,groups", [(1, 1), (2, 1), (3, 1), (257, 1), (4099, 1), (64 * 64, 4), (300 * 300 + 7, 1)])
+@pytest.mark.parametrize("n,groups", [(1, 1), (2, 1), (3, 1), (257, 1), (4099, 1), (64 * 64, 4), (300 * 300 + 7, 1),
+                                      (10007, 3)])
 def test_masked_percentiles_exact_vs_numpy(n, groups):
     rng = np.random.default_rng(n + groups)
     K = 3
@@ -739,7 +740,7 @@ def test_masked_percentiles_exact_vs_numpy(n, groups):
         for padded in (False, True):
             xt = kernels.alloc_planes(K, (groups, n), DEV) if padded else torch.empty(x.shape, dtype=torch.float32, device=DEV)
             xt.copy_(dev(x))
-            for q in ([2, 98], [0, 100], [50, 99.9]):
+            for q in ([2, 98], [0, 100], [50, 99.9], [98, 2]):
                 got = kernels.masked_percentiles(xt, dev(mask), q, groups=groups).cpu().numpy()
                 for k in range(K):
                     for g_ in range(groups):
@@ -1355,6 +1356,7 @@ def test_abi_argument_errors_are_codes_not_crashes():
     expect(-1, lib.hsr_block_average_f32(p(u8), 3, 1, 8, 8, 64, 2, 0, 0.0, 0, 1.0, p(out), 16, st), "src_dtype")
     wsp = torch.zeros(1 << 20, dtype=torch.uint8, device=DEV)
     expect(-3, lib.hsr_masked_percentiles_f64(p(out), 16, 16, None, 16, 3, 1, p(f64), 3, p(wsp), p(f64), st), "Q = 3")
+    expect(-3, lib.hsr_masked_percentiles_f64(p(out), 16, 16, None, 1 << 32, 3, 1, p(f64), 2, p(wsp), p(f64), st), "2^32")
     expect(-1, lib.hsr_masked_percentiles_pair_f64(p(out), 16, 16, p(out), 16, 16, None, 16, 3, 1, p(f64), 2, p(wsp), p(f64),
                                                    None, st), "together")
     expect(-3, lib.hsr_sinkhorn_barycentric_f64(p(f64), p(f64), 4, 4, 5, 0.05, 10, 1e-6, p(f64), p(f64), None, st), "C = 5")
