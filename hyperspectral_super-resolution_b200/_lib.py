@@ -126,6 +126,11 @@ SIGNATURES = {
     "hsr_masked_percentiles_pair_f64": (_int, [_p, _i64, _i64, _p, _i64, _i64, _p, _i64, _int, _int, _p, _int, _p, _p, _p, _p]),
     "hsr_masked_percentiles_f64": (_int, [_p, _i64, _i64, _p, _i64, _int, _int, _p, _int, _p, _p, _p]),
     "hsr_stretch_f32": (_int, [_p, _i64, _i64, _p, _i64, _int, _int, _p, _i64, _i64, _p]),
+    "hsr_union_select_state_bytes": (_c.c_size_t, [_int, _int]),
+    "hsr_union_select_hist_doubles": (_i64, [_int, _int]),
+    "hsr_union_select_begin": (_int, [_p, _int, _int, _p, _p, _p]),
+    "hsr_union_select_count": (_int, [_p, _i64, _p, _i64, _p, _i64, _int, _int, _int, _p, _p, _p]),
+    "hsr_union_select_step": (_int, [_int, _int, _int, _p, _p, _p, _p, _p]),
 }
 
 _lock = threading.Lock()

@@ -121,6 +121,12 @@ int masked_percentiles_impl(const float*, long long, long long, const float*, lo
                             long long, int, int, const double*, int, void*, double*, double*, cudaStream_t);
 int stretch_impl(const float*, long long, long long, const double*, long long, int, int, float*, long long, long long,
                  cudaStream_t);
+size_t union_state_bytes(int Q, int S);
+long long union_hist_doubles(int Q, int S);
+int union_begin_impl(const double*, int, int, void*, double*, cudaStream_t);
+int union_count_impl(const float*, long long, const float*, long long, const uint8_t*, long long, int, int, int, void*,
+                     double*, cudaStream_t);
+int union_step_impl(int, int, int, void*, double*, double*, int*, cudaStream_t);
 
 size_t compact_workspace(long long n);
 int compact_finite_rows_impl(const float*, const uint8_t*, long long, int, void*, int*, long long*, cudaStream_t);
@@ -259,6 +265,23 @@ int hsr_stretch_f32(const float* x, int64_t x_k_stride, int64_t x_g_stride, cons
                     int G, float* out, int64_t out_k_stride, int64_t out_g_stride, void* stream) {
     return hsr::stretch_impl(x, x_k_stride, x_g_stride, lohi, n, K, G, out, out_k_stride, out_g_stride,
                              (cudaStream_t)stream);
+}
+
+size_t hsr_union_select_state_bytes(int Q, int S) { return hsr::union_state_bytes(Q, S); }
+
+int64_t hsr_union_select_hist_doubles(int Q, int S) { return hsr::union_hist_doubles(Q, S); }
+
+int hsr_union_select_begin(const double* q, int Q, int S, void* state, double* hist, void* stream) {
+    return hsr::union_begin_impl(q, Q, S, state, hist, (cudaStream_t)stream);
+}
+
+int hsr_union_select_count(const float* x, int64_t x_k_stride, const float* y, int64_t y_k_stride, const uint8_t* mask,
+                           int64_t n, int K, int Q, int pass, void* state, double* hist, void* stream) {
+    return hsr::union_count_impl(x, x_k_stride, y, y_k_stride, mask, n, K, Q, pass, state, hist, (cudaStream_t)stream);
+}
+
+int hsr_union_select_step(int Q, int S, int pass, void* state, double* hist, double* out, int* more, void* stream) {
+    return hsr::union_step_impl(Q, S, pass, state, hist, out, more, (cudaStream_t)stream);
 }
 
 size_t hsr_compact_workspace_bytes(int64_t n) { return hsr::compact_workspace(n); }

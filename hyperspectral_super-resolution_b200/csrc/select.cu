@@ -195,6 +195,16 @@ __device__ __forceinline__ void numpy_ranks(long long n, double q, long long& r0
     gamma = vi - prev;
 }
 
+// numpy's "linear" interpolation between the order statistics with keys ka <= kb: the float32 neighbour difference,
+// then float64 without contraction, b - diff (1 - gamma) when gamma >= 0.5
+__device__ __forceinline__ double numpy_lerp(unsigned int ka, unsigned int kb, double gamma) {
+    const float a = value_of(ka), b = value_of(kb);
+    const float diff = __fsub_rn(b, a);
+    double r = __dadd_rn((double)a, __dmul_rn((double)diff, gamma));
+    if (gamma >= 0.5) r = __dsub_rn((double)b, __dmul_rn((double)diff, __dsub_rn(1.0, gamma)));
+    return r;
+}
+
 // ---- 1. brackets from a sample
 __global__ void __launch_bounds__(SEL_BT) select_sample_kernel(const SelParams P) {
     __shared__ unsigned int sk[SEL_SAMPLE];
@@ -562,12 +572,225 @@ __global__ void __launch_bounds__(SEL_BT) select_finish_kernel(const SelParams P
         if (tid < 2) keys[tid] = found[tid];
     }
     __syncthreads();
+    if (tid == 0) *out = numpy_lerp(keys[0], keys[1], gamma);
+}
+
+// ---- exact percentiles of a UNION of units (granules, slabs, ranks): radix select by 4 passes of 8 bits, most
+// significant first.  Each pass every unit adds its counts to a per-series (pass 0) or per-target (passes 1-3) 256-bin
+// histogram; the caller sums the histograms over its processes; a one-block-per-series step picks the digit of every
+// target.  Only integer counts cross units and processes, and integer sums do not depend on the order they are formed
+// in: every process ends with the same keys, and they are those of np.percentile over the concatenation.
+//   state:  UnionSeries[S], then the u64 histograms [S][HS] the counting kernel accumulates into
+//   hist:   the f64 image of the u64 histograms [S][HS] (exact below 2^53): what the processes all-reduce
+// Series s of a unit: set s / K (0: x, 1: y), plane s % K.  Targets per series T = 2Q (ranks r0, r1 per percentile).
+constexpr int UNI_THREADS = 256;
+constexpr int UNI_UNR = 4;      // 16-byte loads in flight per thread
+
+struct UnionSeries {
+    unsigned long long rank[SEL_MAXR];   // target t: rank still to find among the keys that carry prefix[t]
+    unsigned int prefix[SEL_MAXR];       // the key bits found so far (8 per pass)
+    double gamma[SEL_QMAX];
+    unsigned int dead;                   // NaN among the samples, no sample, or counts that do not add up: NaN results
+    unsigned int ticket;                 // blocks of the running count launch that have finished this series
+};
+
+static_assert(sizeof(UnionSeries) == 72, "tests/test_gpu_union_select.py reads this layout");
+
+struct UnionHead {
+    double q[SEL_QMAX];                  // percentile fractions, copied by begin
+};
+
+__host__ __device__ constexpr int union_hist_stride(int Q) { return 2 * Q * 256 + 1; }   // + the NaN count (pass 0)
+
+struct UnionCountParams {
+    const float* x[2];
+    long long xks[2];
+    int vec[2];
+    const uint8_t* mask;    // nullable [n]
+    long long n;
+    int K, S, Q, pass;
+    UnionSeries* ser;
+    unsigned long long* hu;
+    double* hf;
+};
+
+// One streaming pass over one unit's planes: blockIdx.y = series.  Image data in [0, 1] has a handful of distinct top
+// bytes, so a shared-memory atomic per sample would serialise on a few bins: the lanes of a warp that add to the same bin
+// are grouped with __match_any_sync and their leader adds them with one atomic.
+// NR: histograms per series of this pass (1 in pass 0, 2Q after it).
+template <int NR>
+__global__ void __launch_bounds__(UNI_THREADS) union_count_kernel(const UnionCountParams P) {
+    __shared__ unsigned int h[NR][256];
+    __shared__ unsigned int pre_s[NR];
+    __shared__ unsigned int red[UNI_THREADS / 32];
+    __shared__ int last;
+    const int s = blockIdx.y;
+    const int set = s / P.K, k = s - set * P.K;
+    const float* xs = (set ? P.x[1] : P.x[0]) + (long long)k * (set ? P.xks[1] : P.xks[0]);   // (no dynamic param index)
+    const int HS = union_hist_stride(P.Q);
+    constexpr int R = NR;
+    const int shift = 24 - 8 * P.pass;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const bool live = P.ser[s].dead == 0u;
+    for (int i = tid; i < R * 256; i += UNI_THREADS) (&h[0][0])[i] = 0u;
+    if (tid < R) pre_s[tid] = P.ser[s].prefix[tid];
+    __syncthreads();
+    unsigned int pre[R];
+#pragma unroll
+    for (int r = 0; r < R; ++r) pre[r] = pre_s[r];
+    unsigned int nan = 0u;
+    // every lane of the warp calls add() the same number of times (warp-uniform loops below)
+    auto add = [&](float v, bool use) {
+        unsigned int key = 0u;
+        const bool ok = use && key_of(v, key);
+        nan += (use && !ok) ? 1u : 0u;
+        const unsigned int digit = (key >> shift) & 255u;
+#pragma unroll
+        for (int r = 0; r < R; ++r) {
+            const bool hit = ok && (NR == 1 || (key >> (shift + 8)) == pre[r]);
+            if (__ballot_sync(0xffffffffu, hit) == 0u) continue;
+            const unsigned int peers = __match_any_sync(0xffffffffu, hit ? digit : 0x100u);
+            if (hit && lane == __ffs(peers) - 1) atomicAdd(&h[r][digit], (unsigned int)__popc(peers));
+        }
+    };
+    if (live) {
+        const long long n = P.n;
+        const long long gtid = (long long)blockIdx.x * UNI_THREADS + tid;
+        const long long nthreads = (long long)gridDim.x * UNI_THREADS;
+        const long long n4 = (set ? P.vec[1] : P.vec[0]) ? (n >> 2) : 0;
+        const float4* x4 = reinterpret_cast<const float4*>(xs);
+        const unsigned int* m4 = reinterpret_cast<const unsigned int*>(P.mask);
+        for (long long base0 = gtid - lane; base0 < n4; base0 += UNI_UNR * nthreads) {
+            float4 v[UNI_UNR];
+            unsigned int m[UNI_UNR];
+#pragma unroll
+            for (int u = 0; u < UNI_UNR; ++u) {
+                const long long i = base0 + lane + u * nthreads;
+                v[u] = make_float4(0.f, 0.f, 0.f, 0.f);
+                m[u] = 0u;
+                if (i < n4) {
+                    m[u] = P.mask ? __ldg(m4 + i) : 0x01010101u;
+                    if (m[u]) v[u] = __ldcs(x4 + i);
+                }
+            }
+#pragma unroll
+            for (int u = 0; u < UNI_UNR; ++u) {
+                if (__ballot_sync(0xffffffffu, m[u] != 0u) == 0u) continue;   // 128 unmasked samples: skipped whole
+                add(v[u].x, (m[u] & 0xffu) != 0u);
+                add(v[u].y, (m[u] & 0xff00u) != 0u);
+                add(v[u].z, (m[u] & 0xff0000u) != 0u);
+                add(v[u].w, (m[u] & 0xff000000u) != 0u);
+            }
+        }
+        for (long long i0 = (n4 << 2) + gtid - lane; i0 < n; i0 += nthreads) {
+            const long long i = i0 + lane;
+            const bool use = i < n && (P.mask == nullptr || P.mask[i] != 0);
+            add(use ? __ldg(xs + i) : 0.f, use);
+        }
+    }
+    // the block's counts -> the series' u64 histograms
+    __syncthreads();
+    unsigned long long* hu = P.hu + (size_t)s * HS;
+    for (int i = tid; i < R * 256; i += UNI_THREADS)
+        if ((&h[0][0])[i]) atomicAdd(hu + i, (unsigned long long)(&h[0][0])[i]);
+    if (P.pass == 0) {
+        nan = __reduce_add_sync(0xffffffffu, nan);
+        if (lane == 0) red[warp] = nan;
+        __syncthreads();
+        if (tid == 0) {
+            unsigned int t = 0u;
+            for (int w = 0; w < UNI_THREADS / 32; ++w) t += red[w];
+            if (t) atomicAdd(hu + HS - 1, (unsigned long long)t);
+        }
+    }
+    // the series' last block to finish writes the f64 image of its totals (the union so far: one unit after another)
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) last = atomicAdd(&P.ser[s].ticket, 1u) == gridDim.x - 1u;
+    __syncthreads();
+    if (!last) return;
+    __threadfence();
+    double* hf = P.hf + (size_t)s * HS;
+    for (int i = tid; i < R * 256; i += UNI_THREADS) hf[i] = (double)__ldcg(hu + i);
     if (tid == 0) {
-        const float a = value_of(keys[0]), bb = value_of(keys[1]);
-        const float diff = __fsub_rn(bb, a);  // numpy subtracts the two float32 neighbours first
-        double r = __dadd_rn((double)a, __dmul_rn((double)diff, gamma));
-        if (gamma >= 0.5) r = __dsub_rn((double)bb, __dmul_rn((double)diff, __dsub_rn(1.0, gamma)));
-        *out = r;
+        if (P.pass == 0) hf[HS - 1] = (double)__ldcg(hu + HS - 1);
+        P.ser[s].ticket = 0u;
+    }
+}
+
+// One block per series, warp t = target t: reads the SUMMED histograms, picks every target's digit, then clears the
+// histograms for the next pass.  Pass 0 also forms numpy's ranks from the union's sample count; the last pass writes
+// the percentiles.
+__global__ void __launch_bounds__(32 * SEL_MAXR) union_step_kernel(const UnionHead* hd, int Q, int pass, UnionSeries* ser, unsigned long long* hu, double* hf,
+                                                                    double* out) {
+    __shared__ unsigned int dead;
+    const int s = blockIdx.x;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int T = 2 * Q, HS = union_hist_stride(Q);
+    UnionSeries* sr = ser + s;
+    double* hs = hf + (size_t)s * HS;
+    if (tid == 0) dead = sr->dead;
+    __syncthreads();
+    if (pass == 0 && warp == 0) {                            // n = the union's masked non-NaN samples
+        unsigned long long n = 0ull;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) n += (unsigned long long)hs[lane * 8 + j];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
+        if (lane == 0) {
+            if (n == 0ull || hs[HS - 1] != 0.0) {
+                dead = 1u;
+            } else {
+                for (int j = 0; j < Q; ++j) {
+                    long long r0, r1;
+                    double gamma;
+                    numpy_ranks((long long)n, hd->q[j], r0, r1, gamma);
+                    sr->rank[2 * j] = (unsigned long long)r0;
+                    sr->rank[2 * j + 1] = (unsigned long long)r1;
+                    sr->gamma[j] = gamma;
+                }
+            }
+        }
+    }
+    __syncthreads();
+    if (dead == 0u && warp < T) {                            // lane l owns bins 8 l .. 8 l + 7
+        const double* hb = hs + (pass == 0 ? 0 : warp * 256);
+        unsigned long long c[8], local = 0ull;
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+            c[j] = (unsigned long long)hb[lane * 8 + j];
+            local += c[j];
+        }
+        unsigned long long incl = local;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned long long v = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += v;
+        }
+        unsigned long long excl = incl - local;
+        const unsigned long long rk = sr->rank[warp];
+        const unsigned int pre = pass == 0 ? 0u : sr->prefix[warp];
+        const bool mine = rk >= excl && rk < excl + local;
+        if (mine) {
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+                if (rk >= excl && rk < excl + c[j]) {
+                    sr->prefix[warp] = (pre << 8) | (unsigned int)(lane * 8 + j);
+                    sr->rank[warp] = rk - excl;
+                }
+                excl += c[j];
+            }
+        }
+        if (__ballot_sync(0xffffffffu, mine) == 0u && lane == 0) dead = 1u;   // the processes' calls did not match
+    }
+    __syncthreads();
+    if (pass == 3 && tid < Q)
+        out[(size_t)s * Q + tid] = dead ? __longlong_as_double(0x7ff8000000000000LL)
+                                        : numpy_lerp(sr->prefix[2 * tid], sr->prefix[2 * tid + 1], sr->gamma[tid]);
+    if (tid == 0) sr->dead = dead;
+    for (int i = tid; i < HS; i += blockDim.x) {
+        hs[i] = 0.0;
+        hu[(size_t)s * HS + i] = 0ull;
     }
 }
 
@@ -817,6 +1040,90 @@ int masked_percentiles_impl(const float* x, long long xks, long long xgs, const 
     HSR_CUDA(ensure_dynamic_smem(select_finish_kernel, (int)(SEL_CAP * sizeof(unsigned int)), smem_set));
     select_finish_kernel<<<dim3((unsigned int)S, (unsigned int)Q), SEL_BT, fsmem, stream>>>(P);
     HSR_CUDA(cudaGetLastError());
+    return HSR_OK;
+}
+
+// union select state: UnionHead | UnionSeries[S] | u64 histograms [S][HS], each part 256-byte aligned
+static size_t union_head_bytes() { return align_up(sizeof(UnionHead), 256); }
+static size_t union_series_bytes(int S) { return align_up((size_t)S * sizeof(UnionSeries), 256); }
+
+static bool union_args_ok(int Q, int S) { return Q >= 1 && Q <= SEL_QMAX && S >= 1 && S <= 65535; }
+
+size_t union_state_bytes(int Q, int S) {
+    if (!union_args_ok(Q, S)) return 0;
+    return union_head_bytes() + union_series_bytes(S) + (size_t)S * union_hist_stride(Q) * sizeof(unsigned long long);
+}
+
+long long union_hist_doubles(int Q, int S) {
+    return union_args_ok(Q, S) ? (long long)S * union_hist_stride(Q) : 0;
+}
+
+struct UnionState {
+    UnionHead* hd;
+    UnionSeries* ser;
+    unsigned long long* hu;
+};
+
+static UnionState union_state(void* state, int S) {
+    unsigned char* b = reinterpret_cast<unsigned char*>(state);
+    return {reinterpret_cast<UnionHead*>(b), reinterpret_cast<UnionSeries*>(b + union_head_bytes()),
+            reinterpret_cast<unsigned long long*>(b + union_head_bytes() + union_series_bytes(S))};
+}
+
+int union_begin_impl(const double* q, int Q, int S, void* state, double* hist, cudaStream_t stream) {
+    HSR_REQUIRE(q && state && hist, HSR_EINVAL, "null q / state / hist pointer");
+    HSR_REQUIRE(union_args_ok(Q, S), HSR_ERANGE, "Q = %d outside [1, %d] or S = %d outside [1, 65535]", Q, SEL_QMAX, S);
+    HSR_REQUIRE((reinterpret_cast<uintptr_t>(state) & 255) == 0 && (reinterpret_cast<uintptr_t>(hist) & 7) == 0,
+                HSR_EALIGN, "state not 256-byte / hist not 8-byte aligned");
+    HSR_CUDA(cudaMemsetAsync(state, 0, union_state_bytes(Q, S), stream));
+    HSR_CUDA(cudaMemsetAsync(hist, 0, (size_t)union_hist_doubles(Q, S) * sizeof(double), stream));
+    HSR_CUDA(cudaMemcpyAsync(union_state(state, S).hd->q, q, (size_t)Q * sizeof(double), cudaMemcpyDeviceToDevice, stream));
+    return HSR_OK;
+}
+
+int union_count_impl(const float* x, long long xks, const float* y, long long yks, const uint8_t* mask, long long n,
+                     int K, int Q, int pass, void* state, double* hist, cudaStream_t stream) {
+    HSR_REQUIRE(state && hist, HSR_EINVAL, "null state / hist pointer");
+    const long long S = (long long)K * (y ? 2 : 1);
+    // n < 2^32 per unit: the per-block counters are 32-bit (the union's totals are 64-bit)
+    HSR_REQUIRE(n >= 0 && n < (1LL << 32) && K >= 1 && S <= 65535 && union_args_ok(Q, (int)S), HSR_ERANGE,
+                "bad n = %lld (< 2^32), K = %d (K * sets <= 65535) or Q = %d", n, K, Q);
+    HSR_REQUIRE(pass >= 0 && pass <= 3, HSR_ERANGE, "pass = %d outside [0, 3]", pass);
+    HSR_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(y)) & 3) == 0, HSR_EALIGN,
+                "x / y not 4-byte aligned");
+    HSR_REQUIRE((reinterpret_cast<uintptr_t>(state) & 255) == 0, HSR_EALIGN, "state not 256-byte aligned");
+    if (n == 0) return HSR_OK;                       // an empty unit adds nothing (its planes may have no storage)
+    HSR_REQUIRE(x, HSR_EINVAL, "null x pointer");
+    const UnionState us = union_state(state, (int)S);
+    UnionCountParams P{};
+    P.x[0] = x, P.xks[0] = xks, P.x[1] = y, P.xks[1] = yks;
+    P.mask = mask, P.n = n, P.K = K, P.S = (int)S, P.Q = Q, P.pass = pass;
+    P.ser = us.ser, P.hu = us.hu, P.hf = hist;
+    for (int i = 0; i < (y ? 2 : 1); ++i) {
+        const uintptr_t a16 = reinterpret_cast<uintptr_t>(P.x[i]) | (uintptr_t)((K > 1 ? P.xks[i] : 0) * 4);
+        P.vec[i] = ((a16 & 15) == 0 && (reinterpret_cast<uintptr_t>(mask) & 3) == 0) ? 1 : 0;
+    }
+    long long per = (n + (long long)UNI_THREADS * 4 * UNI_UNR - 1) / ((long long)UNI_THREADS * 4 * UNI_UNR);
+    long long cap = (long long)device_sm_count() * 8 / S;
+    if (cap < 1) cap = 1;
+    const dim3 grid((unsigned int)(per < cap ? per : cap), (unsigned int)S);
+    if (pass == 0) union_count_kernel<1><<<grid, UNI_THREADS, 0, stream>>>(P);
+    else if (Q == 1) union_count_kernel<2><<<grid, UNI_THREADS, 0, stream>>>(P);
+    else union_count_kernel<2 * SEL_QMAX><<<grid, UNI_THREADS, 0, stream>>>(P);
+    HSR_CUDA(cudaGetLastError());
+    return HSR_OK;
+}
+
+int union_step_impl(int Q, int S, int pass, void* state, double* hist, double* out, int* more, cudaStream_t stream) {
+    HSR_REQUIRE(state && hist, HSR_EINVAL, "null state / hist pointer");
+    HSR_REQUIRE(union_args_ok(Q, S), HSR_ERANGE, "Q = %d outside [1, %d] or S = %d outside [1, 65535]", Q, SEL_QMAX, S);
+    HSR_REQUIRE(pass >= 0 && pass <= 3, HSR_ERANGE, "pass = %d outside [0, 3]", pass);
+    HSR_REQUIRE(pass < 3 || out, HSR_EINVAL, "null out pointer on the last pass");
+    HSR_REQUIRE((reinterpret_cast<uintptr_t>(state) & 255) == 0, HSR_EALIGN, "state not 256-byte aligned");
+    const UnionState us = union_state(state, S);
+    union_step_kernel<<<(unsigned int)S, 64 * Q, 0, stream>>>(us.hd, Q, pass, us.ser, us.hu, hist, out);
+    HSR_CUDA(cudaGetLastError());
+    if (more) *more = pass < 3 ? 1 : 0;
     return HSR_OK;
 }
 

@@ -23,6 +23,13 @@ def world() -> tuple:
     return 0, 1
 
 
+def group_size(group=None) -> int:
+    """Processes in ``group`` (the default group when None); 1 when torch.distributed is not initialised."""
+    if dist.is_available() and dist.is_initialized():
+        return dist.get_world_size(group)
+    return 1
+
+
 def init_from_env(backend: Optional[str] = None) -> tuple:
     """Initialise torch.distributed from the torchrun environment (RANK / LOCAL_RANK / WORLD_SIZE /
     MASTER_ADDR / MASTER_PORT) and bind this process to its GPU.  Returns (rank, world_size, device)."""

@@ -597,6 +597,26 @@ def poly_solve_apply(x: torch.Tensor, moments: torch.Tensor, mask: Optional[torc
 _Q_CACHE: dict = {}
 
 
+def _percentile_fractions(q):
+    import numpy as np
+
+    qf = np.true_divide(np.asarray(q, dtype=np.float64).reshape(-1), 100)   # as np.percentile does
+    if qf.size < 1 or qf.size > _lib.HSR_MAX_PERCENTILES:
+        raise ValueError(f"between 1 and {_lib.HSR_MAX_PERCENTILES} percentiles per call")
+    if not ((qf >= 0) & (qf <= 1)).all():
+        raise ValueError("Percentiles must be in the range [0, 100]")
+    return qf
+
+
+def _fractions_on(qf, device) -> torch.Tensor:
+    """The fractions on the device, uploaded once per (q, device)."""
+    key = (tuple(qf.tolist()), device)
+    qd = _Q_CACHE.get(key)
+    if qd is None:
+        qd = _Q_CACHE[key] = torch.from_numpy(qf).to(device)
+    return qd
+
+
 def masked_percentiles(x: torch.Tensor, mask: Optional[torch.Tensor], q, *, groups: int = 1,
                        y: Optional[torch.Tensor] = None, _workspace_out: Optional[list] = None):
     """``out[k, g, j] = np.percentile(x[k, g][mask[g]], q[j])`` — exact (sampled brackets, one streaming pass, radix
@@ -607,8 +627,6 @@ def masked_percentiles(x: torch.Tensor, mask: Optional[torch.Tensor], q, *, grou
     masked sample or a NaN among them).  ``y``: a second plane set of x's shape (the reference image of the shared
     stretch) handled in the same three launches: returns ``(out_x, out_y)``.
     """
-    import numpy as np
-
     K = int(x.shape[0])
     G = int(groups)
     n = x.numel() // max(K * G, 1)
@@ -625,17 +643,10 @@ def masked_percentiles(x: torch.Tensor, mask: Optional[torch.Tensor], q, *, grou
         m = m.contiguous()
         if m.numel() != G * n:
             raise ValueError("mask must have one entry per (group, sample)")
-    qf = np.true_divide(np.asarray(q, dtype=np.float64).reshape(-1), 100)   # as np.percentile does
-    if qf.size < 1 or qf.size > _lib.HSR_MAX_PERCENTILES:
-        raise ValueError(f"between 1 and {_lib.HSR_MAX_PERCENTILES} percentiles per call")
-    if not ((qf >= 0) & (qf <= 1)).all():
-        raise ValueError("Percentiles must be in the range [0, 100]")
+    qf = _percentile_fractions(q)
     with torch.cuda.device_of(xv):
-        key = (tuple(qf.tolist()), xv.device)
-        qd = _Q_CACHE.get(key)
-        if qd is None:                       # the fractions live on the device: uploaded once per (q, device)
-            qd = _Q_CACHE[key] = torch.from_numpy(qf).to(xv.device)
-        ws = _lib.lib().hsr_percentiles_workspace_bytes(n, K, G, 2 if yv is not None else 1)
+        qd = _fractions_on(qf, xv.device)
+        ws =_lib.lib().hsr_percentiles_workspace_bytes(n, K, G, 2 if yv is not None else 1)
         work = torch.empty(ws + 256, dtype=torch.uint8, device=xv.device)
         off = (-work.data_ptr()) % 256
         out = torch.empty((K, G, qf.size), dtype=torch.float64, device=xv.device)
@@ -651,6 +662,77 @@ def masked_percentiles(x: torch.Tensor, mask: Optional[torch.Tensor], q, *, grou
                                                               G, qd.data_ptr(), int(qf.size), work.data_ptr() + off,
                                                               out.data_ptr(), out_y.data_ptr(), _stream()))
     return out, out_y
+
+
+def masked_percentiles_union(units, q, *, reduce=None, K: Optional[int] = None, pair: Optional[bool] = None,
+                             device=None, _state_out: Optional[list] = None):
+    """``out[k, 0, j] = np.percentile(concatenation over units of x[k][mask], q[j])`` — the exact percentiles of the
+    UNION of several units (granules, slabs) and, through ``reduce``, of every process's units: a radix select by four
+    8-bit passes whose per-pass histograms are summed over the units and then across processes (hsr_union_select_*).
+    Only integer counts cross units and processes, so the result is bit-identical on every process and to numpy.
+
+    units: a list of ``(x, mask)`` or ``(x, y, mask)``; x, y: [K, ...] f32 planes of one unit, mask: bool/u8 with one
+    entry per sample, or None.  The list may be empty (a process that holds no unit still takes part in the
+    reductions); then ``K``, ``pair`` and ``device`` give the shape.  ``reduce``: callable that sums an f64 CUDA tensor
+    in place across processes, called once per pass; default ``dist.allreduce_moments`` on the default group (a no-op
+    for one process).  Every process must make the call.  Returns [K, 1, Q] f64 (a pair for ``(x, y, mask)`` units;
+    NaN where the union has no sample or a NaN among them).  ``_state_out``: diagnostics (tests) — receives the
+    per-series select state after the last pass."""
+    from . import dist as hdist
+
+    units = [tuple(u) for u in units]
+    if units:
+        arity = {len(u) for u in units}
+        if len(arity) != 1 or arity.pop() not in (2, 3):
+            raise ValueError("units must all be (x, mask) or all be (x, y, mask)")
+        pair = len(units[0]) == 3
+        K = int(units[0][0].shape[0])
+        device = units[0][0].device
+    elif K is None or pair is None or device is None:
+        raise ValueError("an empty unit list needs K=, pair= and device=")
+    K, pair, device = int(K), bool(pair), torch.device(device)
+    qf = _percentile_fractions(q)
+    Q, S = int(qf.size), K * (2 if pair else 1)
+    prepared = []
+    for u in units:
+        x, y, mask = (u[0], u[1], u[2]) if pair else (u[0], None, u[1])
+        if int(x.shape[0]) != K or x.device != device:
+            raise ValueError(f"every unit must hold K = {K} planes on {device}")
+        n = x.numel() // max(K, 1)
+        xv, xks, _ = _grouped(x, "x", K, 1, n)
+        yv, yks = None, 0
+        if y is not None:
+            if int(y.shape[0]) != K or y.numel() != x.numel():
+                raise ValueError("y must have the shape of x")
+            yv, yks, _ = _grouped(y, "y", K, 1, n)
+        m = None
+        if mask is not None:
+            m = mask.view(torch.uint8) if mask.dtype == torch.bool else mask
+            m = _cuda(m, "mask", torch.uint8).contiguous()
+            if m.numel() != n:
+                raise ValueError("mask must have one entry per sample")
+        prepared.append((xv, xks, yv, yks, m, n))
+    reduce = reduce if reduce is not None else hdist.allreduce_moments
+    lib = _lib.lib()
+    with torch.cuda.device(device):
+        qd = _fractions_on(qf, device)
+        state, sp = _aligned_workspace(lib.hsr_union_select_state_bytes(Q, S), device)
+        hist = torch.empty(lib.hsr_union_select_hist_doubles(Q, S), dtype=torch.float64, device=device)
+        out = torch.empty((S, Q), dtype=torch.float64, device=device)
+        _lib.check(lib.hsr_union_select_begin(qd.data_ptr(), Q, S, sp, hist.data_ptr(), _stream()))
+        more, p = ctypes.c_int(1), 0
+        while more.value:
+            for xv, xks, yv, yks, m, n in prepared:
+                _lib.check(lib.hsr_union_select_count(xv.data_ptr(), xks, _ptr(yv), yks, _ptr(m), n, K, Q, p, sp,
+                                                      hist.data_ptr(), _stream()))
+            reduce(hist)
+            _lib.check(lib.hsr_union_select_step(Q, S, p, sp, hist.data_ptr(), out.data_ptr(), ctypes.byref(more),
+                                                 _stream()))
+            p += 1
+        if _state_out is not None:
+            _state_out.append(state[sp - state.data_ptr():])
+    out = out.view(S // K, K, 1, Q)
+    return (out[0], out[1]) if pair else out[0]
 
 
 def stretch_apply(x: torch.Tensor, lohi: torch.Tensor, *, groups: int = 1,

@@ -24,6 +24,11 @@ from ._host import cuda_device, to_device
 from .s2_emit.srf import srf_fold_weights
 
 NO_DATA_VALUE = kernels.NO_DATA_VALUE
+STRETCH_SCOPES = ("granule", "fit")
+
+
+def _no_reduce(t):
+    return t
 
 
 @dataclass
@@ -38,6 +43,7 @@ class PairResult:
     ortho: Optional[torch.Tensor] = None    # [Ho, Wo, B] f32 when materialised
     band_names: Optional[List[str]] = None
     x_limits: Optional[torch.Tensor] = None  # [K, G, 2] f64 (lo, hi) percentile stretch of the planes, if enabled
+                                             # ([K, 1, 2], the same on every rank, for a global fit with stretch_scope="fit")
     y_limits: Optional[torch.Tensor] = None  # ... and of the S2 reference
     raw_rows: Optional[tuple] = None         # synthesize_slab: the [row0, row1) raw rows that were staged
 
@@ -47,11 +53,19 @@ class PairSynthesizer:
 
     def __init__(self, emit_w, srf_dict: Dict[str, tuple], good_mask=None, *, deg: int = 2,
                  fill: float = NO_DATA_VALUE, min_count: int = 200, gate_band: Optional[str] = None,
-                 clip=(0.0, 1.0), y_finite: bool = False, stretch=None, device=None):
+                 clip=(0.0, 1.0), y_finite: bool = False, stretch=None, stretch_scope: str = "granule", device=None):
         """``stretch=(pmin, pmax)`` inserts the shared percentile stretch of s2_emit/color.py:25-34 between the
         SRF synthesis and the fit, as the reference's script does (poly_regression.py:126-127): both images are
         stretched with their own masked percentiles, the fit and the apply then run on the stretched values
-        (applied on the fly; the stretched planes are never written)."""
+        (applied on the fly; the stretched planes are never written).
+
+        ``stretch_scope`` says over which pixels the percentiles are taken.  "granule" (default): per image, and a
+        global fit (``synthesize_sharded``, ``exchange=`` / ``allreduce=True``) with a stretch raises ``ValueError``.
+        "fit": over exactly the pixels the fit is taken over — one granule, each tile of ``synthesize_tiles``, or the
+        union of every granule / slab on every rank of a global fit (exact: np.percentile of the concatenation, the
+        same limits on every rank)."""
+        if stretch_scope not in STRETCH_SCOPES:
+            raise ValueError(f"stretch_scope must be one of {STRETCH_SCOPES}, got {stretch_scope!r}")
         self.device = torch.device(device) if device is not None else cuda_device()
         W, names, none_bands, fill_out = srf_fold_weights(emit_w, srf_dict, good_mask, fill=fill)
         if not names:
@@ -66,6 +80,7 @@ class PairSynthesizer:
         self.clip = clip
         self.y_finite = bool(y_finite)
         self.stretch = None if stretch is None else (float(stretch[0]), float(stretch[1]))
+        self.stretch_scope = stretch_scope
 
     @property
     def K(self) -> int:
@@ -83,17 +98,18 @@ class PairSynthesizer:
                                gate_k=self.gate_k, gate_gt=0.0, raw_row0=raw_row0, raw_rows_total=raw_rows_total,
                                tile_rows=tile_rows, valid_out=valid_out, want_diag=want_diag)
 
-    def fit(self, bands, s2_ref, valid, fit_mask, *, groups=1, exchange=None):
+    def fit(self, bands, s2_ref, valid, fit_mask, *, groups=1, exchange=None, reduce=None):
         """Moments under the fit mask the SRF kernel produced; with ``y_finite`` the mask is rebuilt from the
         planes so that non-finite reference pixels drop out of it as well (poly_regression.py:118).
         Returns ``(moments, fit_mask, x_limits, y_limits)``; the limits ([K, G, 2] f64 (lo, hi), None without a
         stretch) belong to THIS call's data — nothing is kept on the instance, so one synthesizer can serve
-        several streams / threads."""
+        several streams / threads.  With a stretch: mask first, then the limits, then the moments; ``reduce``
+        (a global fit with stretch_scope="fit") sums the percentile histograms across processes, so the limits are
+        those of every process's masked pixels."""
         if self.stretch is not None:
-            if self.y_finite:
-                fit_mask = kernels.fit_mask(bands, valid, gate_k=self.gate_k, gate_gt=0.0, y=s2_ref, groups=groups)
-            xl, yl = kernels.masked_percentiles(bands, fit_mask, self.stretch, groups=groups, y=s2_ref)
-            mom, fm = kernels.fit_moments(bands, s2_ref, fit_mask, self.deg, groups=groups, mask_given=True,
+            fm = self.stretch_mask(bands, s2_ref, valid, fit_mask, groups=groups)
+            xl, yl = self.stretch_limits([(bands, s2_ref, fm)], reduce, groups=groups)
+            mom, fm = kernels.fit_moments(bands, s2_ref, fm, self.deg, groups=groups, mask_given=True,
                                           x_stretch=xl, y_stretch=yl, exchange=exchange)
             return mom, fm, xl, yl
         if self.y_finite:
@@ -104,13 +120,37 @@ class PairSynthesizer:
                                           exchange=exchange)
         return mom, fm, None, None
 
+    def stretch_mask(self, bands, s2_ref, valid, fit_mask, *, groups=1):
+        """The pixels the stretch percentiles and the fit are taken over (with ``y_finite``: rebuilt so that
+        non-finite reference pixels drop out, poly_regression.py:118)."""
+        if self.y_finite:
+            return kernels.fit_mask(bands, valid, gate_k=self.gate_k, gate_gt=0.0, y=s2_ref, groups=groups)
+        return fit_mask
+
+    def stretch_limits(self, units, reduce=None, *, groups=1):
+        """``(x_limits, y_limits)`` over the union of ``units`` ([(bands, s2_ref, mask), ...]) and, when ``reduce`` is
+        given, of every process's units.  One unit on one process takes the one-pass select
+        (``kernels.masked_percentiles``, same bits, faster); anything more the union select."""
+        if reduce is None and len(units) == 1:
+            bands, s2_ref, mask = units[0]
+            return kernels.masked_percentiles(bands, mask, self.stretch, groups=groups, y=s2_ref)
+        return kernels.masked_percentiles_union(units, self.stretch, reduce=reduce or _no_reduce, K=self.K, pair=True,
+                                                device=self.device)
+
+    def _global_reduce(self, group):
+        """The SUM all-reduce of the percentile histograms of a global fit (None for one process)."""
+        if self.stretch is None or hdist.group_size(group) == 1:
+            return None
+        return lambda t: hdist.allreduce_moments(t, group)
+
     def _no_global_stretch(self, what: str) -> None:
-        """The percentile limits are per granule (color.py:30-32 sees one image): moments of differently normalised
-        granules must not be summed into one polynomial."""
-        if self.stretch is not None:
+        """With stretch_scope="granule" the percentile limits are per granule (color.py:30-32 sees one image): moments
+        of differently normalised granules must not be summed into one polynomial."""
+        if self.stretch is not None and self.stretch_scope == "granule":
             raise ValueError(f"stretch=(pmin, pmax) cannot be combined with a global fit ({what}): every granule would be "
-                             "normalised by its own percentiles before the moments are summed; fit per granule, or "
-                             "stretch with limits of your own before calling")
+                             "normalised by its own percentiles before the moments are summed; pass "
+                             "stretch_scope=\"fit\" for limits over the whole fit, fit per granule, or stretch with "
+                             "limits of your own before calling")
 
     def moments(self, bands, s2_ref, fit_mask, mask_rows="auto"):
         return kernels.poly_moments(bands, s2_ref, fit_mask, self.deg, mask_rows=mask_rows)
@@ -124,7 +164,8 @@ class PairSynthesizer:
         Three launches (+ the moment finalize): glt_srf, fit_moments, poly_solve_apply.
         Global fit across ranks: ``exchange`` (a ``dist.PeerExchange``: moments travel over NVLink peer memory
         inside the finalize / solve kernels) or ``allreduce=True`` (one NCCL all-reduce between the two)."""
-        if (exchange is not None and exchange.world > 1) or (allreduce and hdist.world()[1] > 1):
+        global_fit = (exchange is not None and exchange.world > 1) or (allreduce and hdist.world()[1] > 1)
+        if global_fit:
             self._no_global_stretch("exchange= / allreduce=True")
         fm = torch.empty(glt_x.shape, dtype=torch.bool, device=raw.device)
         bands, valid, diag, ortho = self.bands_from_raw(raw, glt_x, glt_y, transpose_raw_yx=transpose_raw_yx,
@@ -132,7 +173,8 @@ class PairSynthesizer:
                                                         fit_mask_out=fm, raw_row0=raw_row0,
                                                         raw_rows_total=raw_rows_total)
         ex = exchange.next() if exchange is not None and exchange.world > 1 else None
-        mom, fm, xl, yl = self.fit(bands, s2_ref, valid, fm, exchange=ex)
+        reduce = self._global_reduce(group) if global_fit else None
+        mom, fm, xl, yl = self.fit(bands, s2_ref, valid, fm, exchange=ex, reduce=reduce)
         if allreduce and ex is None:
             hdist.allreduce_moments(mom, group)
         lo, hi = self.clip if self.clip is not None else (1.0, 0.0)
@@ -210,7 +252,9 @@ class PairSynthesizer:
         """Granules owned by THIS rank (dicts with raw, glt_x, glt_y, s2_ref) — BASELINE configs[3]; the fit is
         GLOBAL: the local moments are summed in a fixed order (``kernels.moments_sum``), summed across ranks once —
         over NVLink peer memory when ``exchange`` (a ``dist.PeerExchange``) is given, else one all-reduce (NCCL /
-        gloo) — and solved redundantly.  A rank that was dealt no granule still takes part in the exchange."""
+        gloo) — and solved redundantly.  A rank that was dealt no granule still takes part in the exchange.
+        With ``stretch_scope="fit"`` the stretch limits are the percentiles of every granule on every rank (their
+        histograms are summed over ``group`` with ``dist.all_reduce`` also when the moments go through ``exchange``)."""
         self._no_global_stretch("synthesize_sharded")
         stage = []
         for g in granules:
@@ -218,12 +262,24 @@ class PairSynthesizer:
             bands, valid, diag, _ = self.bands_from_raw(g["raw"], g["glt_x"], g["glt_y"],
                                                         transpose_raw_yx=g.get("transpose_raw_yx", False),
                                                         fit_mask_out=fm)
-            mom, fm, _, _ = self.fit(bands, g["s2_ref"], valid, fm)
-            stage.append((bands, valid, diag, fm, mom.view(self.K, -1)))
+            if self.stretch is not None:
+                fm = self.stretch_mask(bands, g["s2_ref"], valid, fm)
+            stage.append((bands, valid, diag, fm, g["s2_ref"]))
+        xl = yl = None
+        if self.stretch is not None:
+            xl, yl = self.stretch_limits([(s[0], s[4], s[3]) for s in stage], self._global_reduce(group))
+        moms = []
+        for i, (bands, valid, diag, fm, s2_ref) in enumerate(stage):
+            if self.stretch is not None:
+                mom, _ = kernels.fit_moments(bands, s2_ref, fm, self.deg, mask_given=True, x_stretch=xl, y_stretch=yl)
+            else:
+                mom, fm, _, _ = self.fit(bands, s2_ref, valid, fm)
+            moms.append(mom.view(self.K, -1))
+            stage[i] = (bands, valid, diag, fm)
         ex = exchange.next() if exchange is not None and exchange.world > 1 else None
         like = torch.empty((self.K, 3 * self.deg + 2), dtype=torch.float64, device=self.device)
         with torch.cuda.device(self.device):
-            mom = kernels.moments_sum([s[4] for s in stage], like=like, exchange=ex)
+            mom = kernels.moments_sum(moms, like=like, exchange=ex)
         if ex is None:
             hdist.allreduce_moments(mom, group)
         lo, hi = self.clip if self.clip is not None else (1.0, 0.0)
@@ -234,17 +290,17 @@ class PairSynthesizer:
             x0 = torch.zeros((self.K, 1), dtype=torch.float32, device=self.device)
             m0 = torch.zeros(1, dtype=torch.uint8, device=self.device)
             kernels.poly_solve_apply(x0, mom, m0, self.deg, min_count=self.min_count, lo=lo, hi=hi, exchange=ex)
-        for i, (bands, valid, diag, fm, _) in enumerate(stage):
+        for i, (bands, valid, diag, fm) in enumerate(stage):
             if i == 0 and ex is not None:
                 gmom = torch.empty_like(mom)
                 coeffs, matched = kernels.poly_solve_apply(bands, mom, fm, self.deg, min_count=self.min_count, lo=lo,
-                                                           hi=hi, exchange=ex, moments_out=gmom)
+                                                           hi=hi, x_stretch=xl, exchange=ex, moments_out=gmom)
                 mom = gmom.view(self.K, -1)
             else:
                 coeffs, matched = kernels.poly_solve_apply(bands, mom, fm, self.deg, min_count=self.min_count, lo=lo,
-                                                           hi=hi)
+                                                           hi=hi, x_stretch=xl)
             out.append(PairResult(bands, matched, coeffs.view(self.K, self.deg + 1), valid, fm.view(valid.shape), diag,
-                                  mom, None, self.band_names, None, None))
+                                  mom, None, self.band_names, xl, yl))
         return out
 
 

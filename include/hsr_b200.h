@@ -340,6 +340,49 @@ HSR_API int hsr_stretch_f32(const float* x, int64_t x_k_stride, int64_t x_g_stri
                     void* stream);
 
 /*
+ * Exact masked percentiles of a UNION of units — several granules, row slabs or processes whose samples form one
+ * fit — bit-identical to np.percentile of the concatenated masked samples.  A radix select by 4 passes of 8 bits
+ * (most significant first) over the order-preserving u32 keys of the samples; between passes only integer counts
+ * cross units and processes, and integer sums do not depend on the order they are added in, so every process ends
+ * with the same result.  S series: a unit contributes K planes (x only: S = K) or 2K (x then y: S = 2K).
+ *
+ *   hsr_union_select_state_bytes   bytes of device state for Q percentiles and S series (0 if out of range);
+ *                                  256-byte aligned, reused by every call of one select.
+ *   hsr_union_select_hist_doubles  length of the float64 histogram buffer `hist` (8-byte aligned): the per-series /
+ *                                  per-target counts of the pass, exact integers below 2^53.
+ *   hsr_union_select_begin         starts a select: q [Q] f64 device fractions in [0, 1], Q <= HSR_MAX_PERCENTILES,
+ *                                  S <= 65535.  Clears state and hist.
+ *   hsr_union_select_count         adds ONE unit to the histograms of pass `pass` (0..3): series k of set 0 is
+ *                                  x[k*x_k_stride + i], of set 1 y[k*y_k_stride + i] (y nullable), sample i used iff
+ *                                  mask[i] != 0 (mask nullable [n]); n < 2^32 per unit, the union's counts are 64-bit
+ *                                  on the device.  Pass 0 counts the top byte of every key per series, and the NaNs;
+ *                                  passes 1..3 count the next byte of the keys that carry each target's prefix.
+ *                                  On return the stream has `hist` = the sums of every unit counted so far.
+ *   hsr_union_select_step          consumes the SUMMED `hist` of the pass: picks the digit of the two ranks
+ *                                  (floor / floor + 1 of numpy's virtual index) of every percentile, updates each
+ *                                  target's prefix and remaining rank, and clears hist for the next pass.  Pass 0 forms
+ *                                  the ranks from the union's sample count n.  *more (host, nullable) = 1 while passes
+ *                                  follow; the last pass (3) writes out [S, Q] f64 with numpy's "linear"
+ *                                  interpolation (as hsr_masked_percentiles_f64).  A NaN among the union's masked
+ *                                  samples, or no sample at all, gives NaN.
+ * Sequence, on one stream:
+ *     begin(q, Q, S);
+ *     for pass = 0, 1, 2, 3:  count(unit, pass) for every local unit (any number, any order);
+ *                             SUM all-reduce of hist (hsr_union_select_hist_doubles(Q, S) f64) across processes —
+ *                             any f64 SUM all-reduce, e.g. hsr_allreduce_moments; skip it with one process;
+ *                             step(pass, &more)
+ * Every process makes the same begin / all-reduce / step calls (a process with no unit skips only the counts).
+ */
+HSR_API size_t hsr_union_select_state_bytes(int Q, int S);
+HSR_API int64_t hsr_union_select_hist_doubles(int Q, int S);
+HSR_API int hsr_union_select_begin(const double* q, int Q, int S, void* state, double* hist, void* stream);
+HSR_API int hsr_union_select_count(const float* x, int64_t x_k_stride, const float* y, int64_t y_k_stride,
+                           const uint8_t* mask, int64_t n, int K, int Q, int pass, void* state, double* hist,
+                           void* stream);
+HSR_API int hsr_union_select_step(int Q, int S, int pass, void* state, double* hist, double* out, int* more,
+                          void* stream);
+
+/*
  * Optimal-transport targets of fit_ot_poly_rgb, s2_emit/poly_regression.py:31-60.  POT (`import ot`) is an
  * un-vendored, un-pinned dependency of the reference; these entry points follow its published algorithms
  * (ot.dist "sqeuclidean" = |x|^2 + |y|^2 - 2 x.y clamped at 0; ot.sinkhorn = sinkhorn_knopp), all in fp64.
