@@ -14,9 +14,6 @@ import threading
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC_DIR = os.path.join(_HERE, "csrc")
 LIB_PATH = os.path.join(CSRC_DIR, "libhsr_b200.so")
-# profiles/ only: the -DHSR_EXPERIMENTS build (make EXPERIMENTS=1), the one that reads HSR_* tuning / dry-run knobs.
-# Selected with HSR_B200_EXPERIMENTAL_LIB=1; bench.py refuses to run with any HSR_* variable set.
-EXP_LIB_PATH = os.path.join(CSRC_DIR, "libhsr_b200_exp.so")
 ABI_VERSION = 6
 HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "hsr_b200.h")
 
@@ -137,22 +134,14 @@ _lock = threading.Lock()
 _handle = None
 
 
-def build(verbose: bool = False, experiments: bool = False) -> str:
-    """Compile every CUDA source for sm_100a into ``csrc/libhsr_b200.so`` (nvcc cross-compiles without a GPU).
-    ``experiments=True`` builds ``libhsr_b200_exp.so`` (-DHSR_EXPERIMENTS) beside it instead."""
-    cmd = ["make", "-C", CSRC_DIR, "-j8"] + (["EXPERIMENTS=1"] if experiments else [])
-    proc = subprocess.run(cmd, capture_output=True, text=True)
+def build(verbose: bool = False) -> str:
+    """Compile every CUDA source for sm_100a into ``csrc/libhsr_b200.so`` (nvcc cross-compiles without a GPU)."""
+    proc = subprocess.run(["make", "-C", CSRC_DIR, "-j8"], capture_output=True, text=True)
     if verbose or proc.returncode != 0:
         print(proc.stdout)
         print(proc.stderr)
     if proc.returncode != 0:
         raise HsrLibraryError(f"building libhsr_b200.so failed (exit {proc.returncode})")
-    return EXP_LIB_PATH if experiments else LIB_PATH
-
-
-def _selected_path() -> str:
-    if os.environ.get("HSR_B200_EXPERIMENTAL_LIB", "") not in ("", "0"):
-        return EXP_LIB_PATH
     return LIB_PATH
 
 
@@ -163,7 +152,7 @@ def lib() -> ctypes.CDLL:
         return _handle
     with _lock:
         if _handle is None:
-            path = _selected_path()
+            path = LIB_PATH  # the module global, read at call time
             if not os.path.exists(path):
                 raise HsrLibraryError(
                     f"{path} not found — build it with `python -c 'import __graft_entry__ as g; g.build()'` "

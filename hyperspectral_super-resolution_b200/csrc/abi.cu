@@ -2,7 +2,6 @@
 // thread-local error string.  Everything here is argument plumbing; kernels live in
 // glt_stream.cu and poly.cu.
 #include <stdarg.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "hsr_common.cuh"
@@ -52,15 +51,6 @@ int device_max_smem_optin() {
     static int cache[HSR_MAX_DEVICES];
     return cached_attr(cudaDevAttrMaxSharedMemoryPerBlockOptin, cache, 0);
 }
-
-#ifdef HSR_EXPERIMENTS
-int exp_int(const char* name, int dflt, int lo, int hi) {
-    const char* v = getenv(name);
-    if (!v || !*v) return dflt;
-    const int x = atoi(v);
-    return x < lo ? lo : (x > hi ? hi : x);
-}
-#endif
 
 int glt_ortho_impl(const float*, long long, long long, int, long long, int, const int32_t*, const int32_t*, long long,
                    long long, long long, float, float*, long long, uint8_t*, unsigned long long*, const hsr_raw_view_t*,

@@ -4,8 +4,9 @@
 // One persistent CTA per SM, warp-specialised around a ring of shared-memory stages, one
 // 32-pixel ortho tile per stage:
 //   PRODUCER warps (nprod; producer w owns stages w, w + nprod, ...): lane i owns pixel i of the
-//   tile.  The GLT entries come from a per-producer shared-memory ring filled by 1-D bulk copies
-//   (TMA, SASS UBLKCP) GLT_DEPTH tiles ahead.  The lanes evaluate the validity rule of
+//   tile.  The GLT entries come from a per-producer shared-memory ring filled by 16-byte cp.async
+//   copies GLT_DEPTH tiles ahead (when the GLT planes are contiguous and 16-byte aligned; otherwise
+//   each lane loads its own entries).  The lanes evaluate the validity rule of
 //   EMIT_data/emit_proj.py:691-703, then MERGE lanes whose source pixels are the same or adjacent
 //   in memory (q[l] - q[l-1] in {0, 1}) into runs: one bulk copy per run brings the 16-byte
 //   aligned window covering the run's spectra (n * 1140 B for 285 bands) into the stage, runs
@@ -56,9 +57,7 @@ struct StreamParams {
     const int32_t* glt_x;
     const int32_t* glt_y;
     long long out_w, glt_row_stride, npix, ntiles;
-    int glt_tma;  // GLT planes contiguous and 16-byte aligned -> staged ahead in shared memory: 2 cp.async, 1 bulk copies
-    int l2_stream;  // raw-cube bulk copies carry an L2 evict-first policy
-    int dry;        // -DHSR_EXPERIMENTS builds only (HSR_DRY_CONSUMER bit flags); the product library ignores it
+    int glt_ring;  // GLT planes contiguous and 16-byte aligned -> staged ahead in shared memory by cp.async
     float fill;
     float* ortho;
     long long out_pix_stride;
@@ -93,7 +92,6 @@ struct StreamParams {
 struct SmemHeader {
     uint64_t full[MAX_STAGES];
     uint64_t empty[MAX_STAGES];
-    uint64_t glt_full[MAX_PRODUCERS][GLT_DEPTH];
     int meta[MAX_STAGES][TILE];  // >= 0: word offset of the pixel's spectrum inside its stage
     int glt[MAX_PRODUCERS][GLT_DEPTH][2][TILE];
     int fill_f4[MAX_STAGES];                // float4 of the stage the tile's runs occupy (gaps included)
@@ -107,18 +105,10 @@ struct SmemHeader {
     int kcount[MAX_CPS];
     float fill_out[MAXK];
 };
-static_assert(offsetof(SmemHeader, glt) % 16 == 0, "GLT ring must be 16-byte aligned for bulk copies");
+static_assert(offsetof(SmemHeader, glt) % 16 == 0, "GLT ring must be 16-byte aligned for 16-byte cp.async");
 static_assert(offsetof(SmemHeader, kparam) % 16 == 0, "kparam is read with 16-byte loads");
 
 __host__ __device__ inline int header_bytes() { return (int)((sizeof(SmemHeader) + 127) / 128 * 128); }
-
-// Work-skipping diagnostics exist only in -DHSR_EXPERIMENTS builds; in the product library DRY() is the constant 0
-// and the code it guards is compiled out.
-#ifdef HSR_EXPERIMENTS
-#define HSR_DRY(P, bit) ((P).dry & (bit))
-#else
-#define HSR_DRY(P, bit) 0
-#endif
 
 // Fused SRF without a materialised cube: a tile that holds no valid pixel is finished BY ITS PRODUCER (K fill stores, a
 // zero fit-mask word) and never enters the ring — a nodata tile through the ring costs a whole stage round trip
@@ -268,43 +258,40 @@ __device__ __forceinline__ void srf_tile(const StreamParams& P, SmemHeader* hd, 
     const float* xs = reinterpret_cast<const float*>(w4) + sp;
 
     // ---- 1. non-finite scan of this warp's part of the occupied stage (result needed only after step 2)
-    float z = 0.f;
-    if (!HSR_DRY(P, 2)) {
-        const int n4 = hd->fill_f4[stage];
-        const int per = (n4 + CPS - 1) / CPS;
-        const int lo = half * per, hi = (lo + per < n4) ? lo + per : n4;
-        unsigned long long zz0 = 0ull, zz1 = 0ull, zz2 = 0ull, zz3 = 0ull;
-        int i = lo + lane;
-        for (; i + 96 < hi; i += 128) {
-            const float4 a = st4[i], b = st4[i + 32], c = st4[i + 64], d = st4[i + 96];
-            scan2(zz0, a.x, a.y);
-            scan2(zz1, a.z, a.w);
-            scan2(zz2, b.x, b.y);
-            scan2(zz3, b.z, b.w);
-            scan2(zz0, c.x, c.y);
-            scan2(zz1, c.z, c.w);
-            scan2(zz2, d.x, d.y);
-            scan2(zz3, d.z, d.w);
-        }
-        for (; i < hi; i += 32) {
-            const float4 a = st4[i];
-            scan2(zz0, a.x, a.y);
-            scan2(zz1, a.z, a.w);
-        }
-        float y0, y1, y2, y3, y4, y5, y6, y7;
-        asm("mov.b64 {%0, %1}, %2;" : "=f"(y0), "=f"(y1) : "l"(zz0));
-        asm("mov.b64 {%0, %1}, %2;" : "=f"(y2), "=f"(y3) : "l"(zz1));
-        asm("mov.b64 {%0, %1}, %2;" : "=f"(y4), "=f"(y5) : "l"(zz2));
-        asm("mov.b64 {%0, %1}, %2;" : "=f"(y6), "=f"(y7) : "l"(zz3));
-        z = ((y0 + y1) + (y2 + y3)) + ((y4 + y5) + (y6 + y7));
+    const int n4 = hd->fill_f4[stage];
+    const int per = (n4 + CPS - 1) / CPS;
+    const int lo = half * per, hi = (lo + per < n4) ? lo + per : n4;
+    unsigned long long zz0 = 0ull, zz1 = 0ull, zz2 = 0ull, zz3 = 0ull;
+    int i = lo + lane;
+    for (; i + 96 < hi; i += 128) {
+        const float4 a = st4[i], b = st4[i + 32], c = st4[i + 64], d = st4[i + 96];
+        scan2(zz0, a.x, a.y);
+        scan2(zz1, a.z, a.w);
+        scan2(zz2, b.x, b.y);
+        scan2(zz3, b.z, b.w);
+        scan2(zz0, c.x, c.y);
+        scan2(zz1, c.z, c.w);
+        scan2(zz2, d.x, d.y);
+        scan2(zz3, d.z, d.w);
     }
+    for (; i < hi; i += 32) {
+        const float4 a = st4[i];
+        scan2(zz0, a.x, a.y);
+        scan2(zz1, a.z, a.w);
+    }
+    float y0, y1, y2, y3, y4, y5, y6, y7;
+    asm("mov.b64 {%0, %1}, %2;" : "=f"(y0), "=f"(y1) : "l"(zz0));
+    asm("mov.b64 {%0, %1}, %2;" : "=f"(y2), "=f"(y3) : "l"(zz1));
+    asm("mov.b64 {%0, %1}, %2;" : "=f"(y4), "=f"(y5) : "l"(zz2));
+    asm("mov.b64 {%0, %1}, %2;" : "=f"(y6), "=f"(y7) : "l"(zz3));
+    const float z = ((y0 + y1) + (y2 + y3)) + ((y4 + y5) + (y6 + y7));
 
     // ---- 2. per-band FMA over the non-zero run of the folded weights: 16-byte broadcast loads of four
     //         weights, four independent accumulators.  The run bounds are multiples of 4 inside the
     //         spectrum (zero weights pad them); the rare tail past bands & ~3 is scalar.  Independent of the
     //         scan, so the two interleave; pixels the scan flags are redone below.
     bool fit = ok;  // this warp's share of the fit mask: my bands are finite (and the gate band > gate_gt)
-    for (int j = 0; j < (HSR_DRY(P, 4) ? 0 : nk); ++j) {
+    for (int j = 0; j < nk; ++j) {
         const int4 kq = kp[j];
         const int k = kq.x, b0 = kq.y, b1v = kq.z, b1 = kq.w;
         const float* wk = wt + k * P.wt_pitch;
@@ -569,8 +556,6 @@ __global__ void __launch_bounds__(nthreads_of(MODE), 1) glt_stream_kernel(const 
             mbar_init(&hd->full[s], 1);
             mbar_init(&hd->empty[s], CPS);
         }
-        for (int w = 0; w < MAX_PRODUCERS; ++w)
-            for (int g = 0; g < GLT_DEPTH; ++g) mbar_init(&hd->glt_full[w][g], 1);
         fence_mbar_init();
     }
     if ((MODE & MODE_SRF) && tid < P.K) hd->fill_out[tid] = P.fill_out ? P.fill_out[tid] : 0.f;
@@ -656,28 +641,19 @@ __global__ void __launch_bounds__(nthreads_of(MODE), 1) glt_stream_kernel(const 
         const int npix = (int)P.npix, ntiles = (int)P.ntiles, igrid = (int)grid, ibid = (int)bid;
         const int raw_w = (int)P.raw_w, raw_h = (int)P.raw_h;
         const bool contiguous = P.glt_row_stride == P.out_w;
-        const bool glt_ring = P.glt_tma && !P.identity;
+        const bool glt_ring = P.glt_ring && !P.identity;
         int(*gring)[2][TILE] = hd->glt[warp];
-        uint64_t* gbar = hd->glt_full[warp];
         auto tile_is_full = [&](int tile) { return tile * TILE + TILE <= npix; };
-        // The 2 x 128 bytes of a tile's GLT entries are staged GLT_DEPTH tiles ahead.  glt_tma == 2 (default): sixteen
-        // lanes issue one 16-byte cp.async each and every lane commits one group per iteration (an empty one when nothing
-        // was issued), so "the oldest group has landed" is cp.async.wait_group GLT_DEPTH - 1 — no mbarrier, no elected
-        // lane, no entry in the SM's bulk-copy queue.  Against 1-D bulk copies (glt_tma == 1, the round-1 path, kept
-        // for the experiment build): all-nodata grid 0.107 -> 0.098 ms, granule 0.3316 -> 0.3289 ms
-        // (profiles/r2/nodata/invalid_knobs_producer.log).
-        const bool glt_async = P.glt_tma == 2;
+        // The 2 x 128 bytes of a tile's GLT entries are staged GLT_DEPTH tiles ahead: sixteen lanes issue one 16-byte
+        // cp.async each and every lane commits one group per iteration (an empty one when nothing was issued), so "the
+        // oldest group has landed" is cp.async.wait_group GLT_DEPTH - 1 — no mbarrier, no elected lane, no entry in the
+        // SM's bulk-copy queue.  Faster than 1-D bulk copies into the same ring: all-nodata grid 0.107 -> 0.098 ms,
+        // granule 0.3316 -> 0.3289 ms (profiles/r2/nodata/invalid_knobs_producer.log).
         auto issue_glt = [&](int g, int tile, bool on) {  // all lanes; on = warp-uniform "this tile's GLT is staged"
-            if (glt_async) {
-                if (on && lane < 16)
-                    glt_cp_async16(&gring[g][lane >> 3][(lane & 7) << 2],
-                                   (lane < 8 ? P.glt_x : P.glt_y) + (long long)tile * TILE + ((lane & 7) << 2));
-                glt_cp_async_commit();
-            } else if (on && lane == 0) {
-                mbar_arrive_expect_tx(&gbar[g], 2 * TILE * 4);
-                bulk_g2s(&gring[g][0][0], P.glt_x + (long long)tile * TILE, TILE * 4, &gbar[g]);
-                bulk_g2s(&gring[g][1][0], P.glt_y + (long long)tile * TILE, TILE * 4, &gbar[g]);
-            }
+            if (on && lane < 16)
+                glt_cp_async16(&gring[g][lane >> 3][(lane & 7) << 2],
+                               (lane < 8 ? P.glt_x : P.glt_y) + (long long)tile * TILE + ((lane & 7) << 2));
+            glt_cp_async_commit();
         };
         // A stage has ONE producer (a single waiter per `empty` barrier keeps the phase parity
         // unambiguous): this warp walks its stages w, w + nprod, ... round-robin; use `u` of stage
@@ -708,7 +684,6 @@ __global__ void __launch_bounds__(nthreads_of(MODE), 1) glt_stream_kernel(const 
         const bool fill_vec = pfill && (reinterpret_cast<uintptr_t>(P.bands_out) & 15) == 0 && (P.plane_stride & 3) == 0;
         unsigned int fills = 0;  // pfill: how often this producer has filled its (one) stage
         int g = 0;
-        unsigned int gphase = 0;
         const unsigned int le = FULLM >> (31 - lane);  // lanes <= this one
         const int tbank = (P.bank_step * lane) & 31;
         if (warp < nstage)
@@ -722,13 +697,9 @@ __global__ void __launch_bounds__(nthreads_of(MODE), 1) glt_stream_kernel(const 
             int gx = 0, gy = 0;
             if (!P.identity) {
                 if (glt_ring) {
-                    if (glt_async && !HSR_DRY(P, 32)) {
-                        glt_cp_async_wait<GLT_DEPTH - 1>();   // my own copies of the oldest group ...
-                        __syncwarp();                         // ... and every other lane's
-                    }
-                    if (HSR_DRY(P, 32)) {
-                    } else if (tile_is_full(tile)) {
-                        if (!glt_async) mbar_wait(&gbar[g], gphase);
+                    glt_cp_async_wait<GLT_DEPTH - 1>();   // my own copies of the oldest group ...
+                    __syncwarp();                         // ... and every other lane's
+                    if (tile_is_full(tile)) {
                         gx = gring[g][0][lane];
                         gy = gring[g][1][lane];
                         __syncwarp();
@@ -737,12 +708,9 @@ __global__ void __launch_bounds__(nthreads_of(MODE), 1) glt_stream_kernel(const 
                         gy = __ldg(P.glt_y + p);
                     }
                     const long long nt = tile_of(ps, pu);
-                    issue_glt(g, (int)nt, nt < ntiles && tile_is_full((int)nt) && !HSR_DRY(P, 64));
+                    issue_glt(g, (int)nt, nt < ntiles && tile_is_full((int)nt));
                     advance(ps, pu);
-                    if (++g == GLT_DEPTH) {
-                        g = 0;
-                        gphase ^= 1u;
-                    }
+                    if (++g == GLT_DEPTH) g = 0;
                 } else if (inb) {
                     const long long gi = contiguous ? (long long)p
                                                     : (long long)(p / (int)P.out_w) * P.glt_row_stride + (p % (int)P.out_w);
@@ -771,7 +739,7 @@ __global__ void __launch_bounds__(nthreads_of(MODE), 1) glt_stream_kernel(const 
                 q = p;
             }
             if (inb && !P.identity) {
-                if (P.valid && !HSR_DRY(P, 16)) P.valid[p] = ib ? 1 : 0;
+                if (P.valid) P.valid[p] = ib ? 1 : 0;
                 cnt_nz += nz ? 1u : 0u;
                 cnt_ib += ib ? 1u : 0u;
                 cnt_ow += (ib && !in_win) ? 1u : 0u;
@@ -782,8 +750,7 @@ __global__ void __launch_bounds__(nthreads_of(MODE), 1) glt_stream_kernel(const 
 
             const unsigned int vmask = __ballot_sync(FULLM, ib);
             if (pfill && vmask == 0u && tile_is_full(tile)) {  // nodata tile: finished here, the ring never sees it
-                if (HSR_DRY(P, 8)) {
-                } else if (fill_vec) {  // 8 lanes x 16 bytes cover a plane's 32 pixels: four planes per store instruction
+                if (fill_vec) {  // 8 lanes x 16 bytes cover a plane's 32 pixels: four planes per store instruction
                     for (int k = lane >> 3; k < P.K; k += 4) {
                         const float f = hd->fill_out[k];
                         *reinterpret_cast<float4*>(P.bands_out + (long long)k * P.plane_stride + (long long)tile * TILE +
@@ -792,7 +759,7 @@ __global__ void __launch_bounds__(nthreads_of(MODE), 1) glt_stream_kernel(const 
                 } else {
                     for (int k = 0; k < P.K; ++k) P.bands_out[(long long)k * P.plane_stride + p] = hd->fill_out[k];
                 }
-                if (P.fit_mask && !HSR_DRY(P, 16)) P.fit_mask[p] = 0;
+                if (P.fit_mask) P.fit_mask[p] = 0;
                 advance(stage, use);
                 continue;
             }
@@ -867,12 +834,12 @@ __global__ void __launch_bounds__(nthreads_of(MODE), 1) glt_stream_kernel(const 
             __syncwarp();
             if (lane == 0) mbar_arrive_expect_tx(&hd->full[stage], tx);
             if (tma_bytes) {
-                if (P.l2_stream)
-                    bulk_g2s_hint(sbase + base + cut_front, reinterpret_cast<const void*>(lo + cut_front), tma_bytes,
-                                  &hd->full[stage], evict_first);
-                else
+                if (P.identity)  // un-fused SRF: no hint (its L2 behaviour with evict-first has not been measured)
                     bulk_g2s(sbase + base + cut_front, reinterpret_cast<const void*>(lo + cut_front), tma_bytes,
                              &hd->full[stage]);
+                else
+                    bulk_g2s_hint(sbase + base + cut_front, reinterpret_cast<const void*>(lo + cut_front), tma_bytes,
+                                  &hd->full[stage], evict_first);
             }
 
             advance(stage, use);
@@ -909,13 +876,11 @@ __global__ void __launch_bounds__(nthreads_of(MODE), 1) glt_stream_kernel(const 
                 if (tile < 0) break;
             }
             const int m = hd->meta[stage][lane];
-            if (!HSR_DRY(P, 1)) {
-                if (MODE & MODE_COPY) copy_tile<CPS>(P, st4, m, tile, lane, half);
-                if (MODE & MODE_SRF) srf_tile<CPS>(P, hd, wt, st4, m, tile, lane, stage, half);
-                if (MODE & MODE_Q16) {
-                    if (P.q16_pair) q16_tile2<CPS>(P, hd, st4, m, tile, lane, stage, half);
-                    else q16_tile<CPS>(P, hd, st4, m, tile, lane, stage, half);
-                }
+            if (MODE & MODE_COPY) copy_tile<CPS>(P, st4, m, tile, lane, half);
+            if (MODE & MODE_SRF) srf_tile<CPS>(P, hd, wt, st4, m, tile, lane, stage, half);
+            if (MODE & MODE_Q16) {
+                if (P.q16_pair) q16_tile2<CPS>(P, hd, st4, m, tile, lane, stage, half);
+                else q16_tile<CPS>(P, hd, st4, m, tile, lane, stage, half);
             }
             __syncwarp();
             if (lane == 0) mbar_arrive(&hd->empty[stage]);
@@ -998,7 +963,7 @@ __global__ void __launch_bounds__(256) glt_row_range_kernel(const int32_t* __res
 // Run merging needs adjacent source pixels contiguous in memory (pixel stride == bands) and pays off only
 // when spectra `bands` words apart fall into different banks (bands = 285: 29 mod 32, all 32 distinct).
 bool merge_ok(int bands, long long pix_stride) {
-    return pix_stride == bands && (bands & 3) != 0 && exp_int("HSR_NO_MERGE", 0, 0, 1) == 0;
+    return pix_stride == bands && (bands & 3) != 0;
 }
 
 int plan_smem(StreamParams& P, int mode, size_t* smem_bytes) {
@@ -1029,9 +994,8 @@ int plan_smem(StreamParams& P, int mode, size_t* smem_bytes) {
     long long ns = (long long)((cap - fixed - 128) / stage_bytes);
     if (ns > MAX_STAGES) ns = MAX_STAGES;
     if (ns < 2) return HSR_ENOSMEM;
-    P.nstage = exp_int("HSR_STAGES", (int)ns, 2, (int)ns);
-    P.nprod = exp_int("HSR_PRODUCERS", MAX_PRODUCERS, 1, MAX_PRODUCERS);
-    if (P.nprod > P.nstage) P.nprod = P.nstage;
+    P.nstage = (int)ns;
+    P.nprod = P.nstage < MAX_PRODUCERS ? P.nstage : MAX_PRODUCERS;
     *smem_bytes = fixed + (size_t)P.nstage * stage_bytes;
     return HSR_OK;
 }
@@ -1103,13 +1067,9 @@ void fill_common(StreamParams& P, const float* raw, long long raw_h, long long r
     P.glt_row_stride = glt_row_stride;
     P.npix = out_h * out_w;
     P.ntiles = (P.npix + TILE - 1) / TILE;
-    P.glt_tma = (glt_row_stride == out_w || out_h <= 1) &&
-                ((reinterpret_cast<uintptr_t>(glt_x) | reinterpret_cast<uintptr_t>(glt_y)) & 15) == 0 &&
-                exp_int("HSR_GLT_NO_RING", 0, 0, 1) == 0;
-    if (P.glt_tma) P.glt_tma = exp_int("HSR_GLT_BULK", 0, 0, 1) ? 1 : 2;   // 2: cp.async ring (default), 1: bulk copies
+    P.glt_ring = (glt_row_stride == out_w || out_h <= 1) &&
+                 ((reinterpret_cast<uintptr_t>(glt_x) | reinterpret_cast<uintptr_t>(glt_y)) & 15) == 0;
     P.fill = fill;
-    P.l2_stream = exp_int("HSR_L2_STREAM", 1, 0, 1);
-    P.dry = exp_int("HSR_DRY_CONSUMER", 0, 0, 127);   // bits 8 / 16 / 32 / 64: producer-side experiments
     const long long slow_n = transpose ? raw_w : raw_h, fast_n = transpose ? raw_h : raw_w;
     long long held = slow_n;
     P.win_lo = 0u;
@@ -1197,7 +1157,7 @@ int glt_ortho_u16_impl(const float* raw, long long raw_h, long long raw_w, int b
     P.diag = diag;
     P.q16 = out;
     P.q16_plane_stride = plane_stride;
-    P.q16_pair = ((reinterpret_cast<uintptr_t>(out) & 3) == 0 && (plane_stride & 1) == 0) ? exp_int("HSR_Q16_PAIR", 1, 0, 1) : 0;
+    P.q16_pair = (reinterpret_cast<uintptr_t>(out) & 3) == 0 && (plane_stride & 1) == 0;
     P.q_scale = scale, P.q_nodata = nodata, P.q_hi = (float)(nodata_u16 - 1), P.q_has_nodata = has_nodata ? 1 : 0;
     P.q_nd = (unsigned short)nodata_u16;
     P.black = black;

@@ -59,15 +59,6 @@ inline int resident_blocks_cached(Kern kern, int threads, int* cache) {
     return r;
 }
 
-// Experiment knobs (profiles/ only).  The shipped library reads NO environment variable: every knob folds to
-// its default at compile time unless the library is built with -DHSR_EXPERIMENTS (`make EXPERIMENTS=1`, which
-// produces libhsr_b200_exp.so beside the product library).
-#ifdef HSR_EXPERIMENTS
-int exp_int(const char* name, int dflt, int lo, int hi);
-#else
-constexpr int exp_int(const char*, int dflt, int, int) { return dflt; }
-#endif
-
 // ---------------------------------------------------------------- PTX wrappers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));

@@ -600,8 +600,7 @@ int sinkhorn_barycentric_impl(const double* X, const double* Y, int ns, int nt, 
     int fgrid = device_sm_count();
     if (fgrid > OT_PARTS_MAX) fgrid = OT_PARTS_MAX;
     if (fgrid > ns) fgrid = ns;
-    const bool fused = (nt % 2 == 0) && nt <= FUSE_NCMAX * FUSE_THREADS && fuse_smem <= (size_t)device_max_smem_optin() &&
-                       exp_int("HSR_OT_UNFUSED", 0, 0, 1) == 0;
+    const bool fused = (nt % 2 == 0) && nt <= FUSE_NCMAX * FUSE_THREADS && fuse_smem <= (size_t)device_max_smem_optin();
     if (fused)
     {
         static int set__[HSR_MAX_DEVICES];
@@ -609,7 +608,7 @@ int sinkhorn_barycentric_impl(const double* X, const double* Y, int ns, int nt, 
     }
     int nparts = nchunks;
     bool looped = false;
-    if (fused && num_iter_max > 0 && exp_int("HSR_OT_NO_GRAPH", 0, 0, 1) == 0) {
+    if (fused && num_iter_max > 0) {
         // Device-side loop: a CUDA-graph WHILE node whose body is {v-update, fused sweep, step}; the step kernel ends
         // the loop as soon as the marginal error is below stopThr (or after numItermax iterations), so nothing is
         // enqueued for iterations that never run.  The first column pass (u_0) fills nchunks partial rows; the rest

@@ -75,9 +75,9 @@ struct MomParams {
     const double* yst;
     long long n;
     int G;
-    int reverse;  // walk the samples from the end: the planes were just written front to back by the producer
-                  // kernel, so their tail is what is still in L2 (a forward scan of 135 MB through a 126 MB LRU
-                  // cache would miss everywhere)
+    int reverse;  // hsr_fit_moments_f64 walks the samples from the end: the planes were just written front to back
+                  // by the producer kernel, so their tail is what is still in L2 (a forward scan of 135 MB through a
+                  // 126 MB LRU cache would miss everywhere).  hsr_poly_moments_f64 walks forward.
     double* partial;
 };
 
@@ -838,7 +838,7 @@ int fit_moments_impl(const float* x, long long xks, long long xgs, const float* 
     P.mask = fm, P.mdiv = 1, P.mmod = G;  // series s = k * G + g uses mask row g
     P.xst = x_stretch, P.yst = y_stretch;
     P.n = n, P.G = G, P.partial = partial;
-    P.reverse = exp_int("HSR_FIT_REVERSE", 1, 0, 1);
+    P.reverse = 1;
     return launch_moments(P, (long long)K * G, deg, moments, stream, ex);
 }
 

@@ -52,14 +52,7 @@ struct WarpParams {
     unsigned long long* redo_list;   // warp_quad_kernel -> warp_fixup_kernel: (pixel << 8 | band group) of ill-conditioned quotients
     unsigned int* redo_count;
     unsigned int redo_cap;
-    int dry;                    // -DHSR_EXPERIMENTS builds only (HSR_WARP_DRY bit flags: 1 no taps, 2 no stores, 4 no staging)
 };
-
-#ifdef HSR_EXPERIMENTS
-#define HSR_WDRY(P, bit) ((P).dry & (bit))
-#else
-#define HSR_WDRY(P, bit) 0
-#endif
 
 __host__ __device__ __forceinline__ double taup_of(double tau, double e) {
     const double s1 = sqrt(1.0 + tau * tau);
@@ -1533,7 +1526,7 @@ __global__ void __launch_bounds__(256, 2) warp_quad_kernel(const __grid_constant
                 dirty = nonfinite || (has_nd && pm == 0.f);
                 notfill = !has_nd || nonfinite || !((sa + sb) + (sc + sd) == 0.f);
             }
-            const bool clean = __syncthreads_or(dirty && !HSR_WDRY(P, 16)) == 0;
+            const bool clean = __syncthreads_or(dirty) == 0;
             const bool allfill = staged && !clean && __syncthreads_or(notfill) == 0;
             // a dirty box (the swath's edge): classify every box pixel — clean, FILL (all bands of the group are nodata: the
             // usual case outside the swath) or mixed.  Without mixed pixels and non-finite samples the group takes the
@@ -1669,7 +1662,7 @@ __global__ void __launch_bounds__(256, 2) warp_quad_kernel(const __grid_constant
 #pragma unroll
                     for (int p = 0; p < 4; ++p) {
                         if (!((doing >> p) & 1u)) continue;
-                        if (winv[p] > 33.f && !HSR_WDRY(P, 8)) list_px(p);    // weight sum < 0.03 (taps beyond the source's border)
+                        if (winv[p] > 33.f) list_px(p);    // weight sum < 0.03 (taps beyond the source's border)
                         float4 o = fillq;
                         if (winv[p] != 0.f) {
                             const unsigned long long iv = pack2(winv[p], winv[p]);
@@ -1726,7 +1719,7 @@ __global__ void __launch_bounds__(256, 2) warp_quad_kernel(const __grid_constant
                         if (!((doing >> p) & 1u)) continue;
                         // few valid taps left: fixed up exactly afterwards (a sum <= -1e-3 is clearly below GDAL's 1e-6
                         // threshold, 0 means no valid tap at all: both are nodata without a second look)
-                        if (((insb >> p) & 1u) && ms[p] > -1e-3f && ms[p] != 0.f && ms[p] < 0.03f && !HSR_WDRY(P, 8)) list_px(p);
+                        if (((insb >> p) & 1u) && ms[p] > -1e-3f && ms[p] != 0.f && ms[p] < 0.03f) list_px(p);
                         float4 o = fillq;
                         if (((insb >> p) & 1u) && ms[p] >= 1e-6f) {
                             const float inv = 1.f / ms[p];
@@ -1746,7 +1739,7 @@ __global__ void __launch_bounds__(256, 2) warp_quad_kernel(const __grid_constant
                     for (int p = 0; p < 4; ++p)
                         if ((redo >> p) & 1u) {
                             const bool ill = exact_px(p);
-                            if ((__ballot_sync(gm, ill) & gm) != 0u && !HSR_WDRY(P, 8)) list_px(p);
+                            if ((__ballot_sync(gm, ill) & gm) != 0u) list_px(p);
                         }
                 }
             }
@@ -1873,7 +1866,6 @@ int warp_impl(const float* src, long long Hs, long long Ws, int bands, long long
     P.has_nodata = has_nodata ? 1 : 0;
     P.nodata = nodata;
     P.dst_nodata = dst_nodata;
-    P.dry = exp_int("HSR_WARP_DRY", 0, 0, 31);
     if (kernel == 0 || kernel == 3) {   // nearest / average: every pixel transforms its own centre or corners
         long long pb = (Hd * Wd + 255) / 256;
         const long long pcap = (long long)device_sm_count() * 16;
@@ -1914,9 +1906,8 @@ int warp_impl(const float* src, long long Hs, long long Ws, int bands, long long
     const bool dst_vec = (dst_pix_stride & 3) == 0 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0;
     const bool fast = P.coords && 4 * P.rx * P.ry <= PTAPS && P.tile_w * P.tile_h <= PTILE && Ws < 2147483647LL &&
                       Hs < 2147483647LL;
-    if (P.coords && P.rx <= 4 && P.ry <= 4 && Hs * Ws < 4294967295LL && Hs < 2147483000LL && Ws < 2147483000LL &&
-        exp_int("HSR_WARP_NO_LANE", 0, 0, 1) == 0) {
-        if (src_vec && dst_vec && exp_int("HSR_WARP_NO_QUAD", 0, 0, 1) == 0) {
+    if (P.coords && P.rx <= 4 && P.ry <= 4 && Hs * Ws < 4294967295LL && Hs < 2147483000LL && Ws < 2147483000LL) {
+        if (src_vec && dst_vec) {
             // 2 x 2 block kernel, TMA-staged.  TMA box = the tile's windows estimated from the scales (+ 1 of slack per
             // axis for rotation / rounding; a tile that needs more reads its taps from global memory)
             const double xs = geo->xscale > 0.0 ? geo->xscale : 1.0, ys = geo->yscale > 0.0 ? geo->yscale : 1.0;

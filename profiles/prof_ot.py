@@ -48,7 +48,7 @@ for iters in (300,):
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
-    passes = 2 if os.environ.get("HSR_OT_UNFUSED") else 1          # sweeps of K per iteration
+    passes = 1                                                     # sweeps of K per iteration
     nbytes = 5000 * 5000 * 8 * (passes * iters + 3)
     print(f"sinkhorn 5000x5000, {iters} iterations (stopThr 0)              {ms:9.3f} ms   {nbytes / ms / 1e6:8.1f} GB/s of K traffic"
           f"   ({ms / iters * 1e3:.1f} us / iteration, {passes} sweep(s) of K each)")

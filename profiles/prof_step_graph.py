@@ -1,6 +1,6 @@
 """The benchmark step (glt_stream<SRF>, poly_moments, moments_finalize, solve_apply) captured into a CUDA graph and
-replayed — for A/B runs of the experiment build's knobs (bench.py refuses to run with HSR_* set).
-    [HSR_B200_EXPERIMENTAL_LIB=1 HSR_...=..] python profiles/prof_step_graph.py [reps]"""
+replayed, without the host's launch overhead.
+    python profiles/prof_step_graph.py [reps]"""
 import os
 import sys
 
@@ -52,5 +52,4 @@ for i in range(reps):
     graphs[i & 1].replay()
 e1.record()
 torch.cuda.synchronize()
-knobs = " ".join(f"{k}={v}" for k, v in sorted(os.environ.items()) if k.startswith("HSR_"))
-print(f"{knobs or '(product library)':60s} {e0.elapsed_time(e1) / reps:.4f} ms per step", flush=True)
+print(f"{e0.elapsed_time(e1) / reps:.4f} ms per step", flush=True)

@@ -58,8 +58,8 @@ def test_missing_library_fails_loudly(monkeypatch, tmp_path):
 
 
 def test_product_library_reads_no_environment_variable():
-    """VERDICT r1: work-skipping / tuning knobs must not ship.  The product library has no getenv at all (the knobs
-    exist only in the -DHSR_EXPERIMENTS build, libhsr_b200_exp.so)."""
+    """VERDICT r1: work-skipping / tuning knobs must not ship.  The library has no getenv at all, and none of the knob
+    names INTEGRATION.md lists appears in it."""
     import subprocess
 
     if not os.path.exists(_lib.LIB_PATH):
@@ -68,7 +68,10 @@ def test_product_library_reads_no_environment_variable():
     names = {ln.split()[-1].split("@")[0] for ln in und.splitlines() if ln.strip()}
     assert "getenv" not in names and "secure_getenv" not in names
     strings = subprocess.run(["strings", "-n", "6", _lib.LIB_PATH], capture_output=True, text=True, check=True).stdout
-    assert "HSR_DRY_CONSUMER" not in strings and "HSR_L2_STREAM" not in strings and "HSR_OT_NO_GRAPH" not in strings
+    knobs = ("HSR_DRY_CONSUMER", "HSR_WARP_DRY", "HSR_STAGES", "HSR_PRODUCERS", "HSR_NO_MERGE", "HSR_GLT_NO_RING",
+             "HSR_GLT_BULK", "HSR_L2_STREAM", "HSR_FIT_REVERSE", "HSR_OT_UNFUSED", "HSR_OT_NO_GRAPH", "HSR_WARP_NO_QUAD",
+             "HSR_WARP_NO_LANE", "HSR_Q16_PAIR")
+    assert [k for k in knobs if k in strings] == []
 
 
 def test_exchange_descriptor_must_alternate_fit_then_solve():
