@@ -14,7 +14,7 @@ are); or one shared CRS (affine only).  Parity with GDAL / PROJ is unpinned — 
 from __future__ import annotations
 
 import math
-from dataclasses import dataclass
+from dataclasses import dataclass, field
 from typing import Optional, Sequence, Tuple
 
 import numpy as np
@@ -249,3 +249,57 @@ def warp_to_s2_grid(cube, src_gt, s2, xres: float = 60.0, yres: float = 60.0, *,
     dst_gt, dst_shape, rec = target_grid(src_gt, shape[:2], s2, xres, yres)
     out = warp_to_grid(cube, src_gt, dst_gt, dst_shape, epsg=s2.epsg, kernel=kernel, nodata=nodata, dst_nodata=nodata)
     return out, dst_gt, rec
+
+
+warp_planes = kernels.warp_planes
+
+
+@dataclass
+class S2Target:
+    """The Sentinel-2 grid a pair is synthesised on (``PairSynthesizer.synthesize_on_s2_grid``): the grid
+    ``nc_to_envi`` warps the ortho cube onto, with what the plane warp needs to reach it.
+
+    ``s2_window`` = (row, col): where the target's top-left pixel sits in the S2 grid counted in target pixels
+    (xres / yres), so that ``s2_stack_at_target_res[:, row:row + shape[0], col:col + shape[1]]`` is the reference on
+    the target grid.  :meth:`coords` runs the fp64 inverse transverse Mercator once per device and keeps the result,
+    so repeated syntheses on one geometry skip it."""
+    src_gt: Tuple[float, ...]
+    dst_gt: Tuple[float, ...]
+    shape: Tuple[int, int]
+    rec: dict
+    zone: int
+    south: bool
+    scales: Tuple[float, float]
+    s2_window: Tuple[int, int]
+    kernel: str = "cubic"
+    _coords: dict = field(default_factory=dict, repr=False, compare=False)
+
+    def coords(self, device=None) -> torch.Tensor:
+        """[Hd, Wd, 2] f64 source pixel coordinates of the target's pixel centres on ``device`` (cached)."""
+        dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
+        if dev.type == "cuda" and dev.index is None:
+            dev = torch.device("cuda", torch.cuda.current_device())
+        c = self._coords.get(dev)
+        if c is None:
+            c = kernels.warp_coords(self.src_gt, self.dst_gt, self.shape, utm_zone=self.zone, south=self.south,
+                                    device=dev)
+            self._coords[dev] = c
+        return c
+
+
+def s2_target(glt_gt, ortho_shape, s2, xres: float = 60.0, yres: float = 60.0, kernel: str = "cubic") -> S2Target:
+    """The S2 target of an ortho (GLT) grid with geotransform ``glt_gt`` and shape ``ortho_shape`` = (Ho, Wo): the
+    snapped extent of ``target_grid`` (reference :354-382, :886-908), the UTM zone of the S2 CRS, the filter scales of
+    ``warp_scales`` and the integer offset of the target in the S2 grid at (xres, yres).  Raises ``ValueError`` when
+    the grids do not overlap, when xres / yres is not an integer multiple of the S2 pixel size, or for a kernel other
+    than "cubic" / "bilinear"."""
+    if kernel not in kernels.PLANE_WARP_KERNELS:
+        raise ValueError(f"kernel must be one of {sorted(kernels.PLANE_WARP_KERNELS)}, got {kernel!r}")
+    s2 = S2Grid.coerce(s2)
+    zone, south = epsg_to_utm(s2.epsg)
+    glt_gt = tuple(float(v) for v in glt_gt)
+    dst_gt, shape, rec = target_grid(glt_gt, ortho_shape, s2, xres, yres)
+    # compute_te snaps the extent to whole steps from the S2 origin: the offsets are integers up to rounding
+    window = (int(round((s2.y0 - rec["top"]) / yres)), int(round((rec["left"] - s2.x0) / xres)))
+    scales = warp_scales(dst_gt, glt_gt, shape, zone, south)
+    return S2Target(glt_gt, tuple(dst_gt), tuple(shape), rec, zone, south, scales, window, kernel)

@@ -1752,6 +1752,88 @@ __global__ void __launch_bounds__(256, 2) warp_quad_kernel(const __grid_constant
     }
 }
 
+// ---------------------------------------------------------------------------- K planes, lane per pixel
+// hsr_warp_planes_f32: K <= 16 planar images (the pseudo-S2 planes of the SRF pass) resampled with the taps of
+// hsr_warp_f32, validity per SOURCE PIXEL (src_valid) instead of per band and value.  One thread per destination pixel
+// of a 32 x 8 tile; the K accumulators are fp64 registers (K is a template parameter, every loop over it unrolled), so
+// the quotient is formed as warp_fixup_kernel forms it and there is no fix-up pass.  Tap weights: the fp32 rounding of
+// the fp64 product wy * wx (oracle/warp.py); zero weights, taps outside the source and invalid source pixels skipped.
+constexpr int PL_COLS = 32, PL_ROWS = 8;
+
+struct PlaneParams {
+    const float* src;
+    const uint8_t* src_valid;
+    long long Hs, Ws, src_plane_stride;
+    const double* coords;
+    long long Hd, Wd;
+    int kind, rx, ry;
+    double fx, fy;
+    const float* fill_out;
+    int gate_k;
+    float gate_gt;
+    float* dst;
+    long long dst_plane_stride;
+    uint8_t* dst_valid;
+    uint8_t* fit_mask;
+};
+
+template <int K>
+__global__ void __launch_bounds__(PL_COLS * PL_ROWS) warp_planes_kernel(const PlaneParams P) {
+    const long long c = (long long)blockIdx.x * PL_COLS + threadIdx.x;
+    if (c >= P.Wd) return;
+    const long long tiles_y = (P.Hd + PL_ROWS - 1) / PL_ROWS;
+    for (long long ty = blockIdx.y; ty < tiles_y; ty += gridDim.y) {
+        const long long r = ty * PL_ROWS + threadIdx.y;
+        if (r >= P.Hd) return;
+        const long long o = r * P.Wd + c;
+        const double2 xy = __ldg(reinterpret_cast<const double2*>(P.coords) + o);
+        const double px = xy.x, py = xy.y;
+        double acc[K];
+#pragma unroll
+        for (int k = 0; k < K; ++k) acc[k] = 0.0;
+        double ws = 0.0;
+        const bool inside = px >= 0.0 && px < (double)P.Ws && py >= 0.0 && py < (double)P.Hs;
+        if (inside) {
+            const double fxp = floor(px - 0.5), fyp = floor(py - 0.5);
+            const long long x0 = (long long)fxp + 1 - P.rx, y0 = (long long)fyp + 1 - P.ry;
+            const double ddx = px - 0.5 - fxp, ddy = py - 0.5 - fyp;
+            for (int j = 0; j < 2 * P.ry; ++j) {
+                const long long yy = y0 + j;
+                if (yy < 0 || yy >= P.Hs) continue;
+                const double wy = tap_weight(P.kind, ((double)(j + 1 - P.ry) - ddy) * P.fy);
+                if (wy == 0.0) continue;
+                for (int i = 0; i < 2 * P.rx; ++i) {
+                    const long long xx = x0 + i;
+                    if (xx < 0 || xx >= P.Ws) continue;
+                    const double w = (double)(float)(wy * tap_weight(P.kind, ((double)(i + 1 - P.rx) - ddx) * P.fx));
+                    const long long s = yy * P.Ws + xx;
+                    if (w == 0.0 || !__ldg(P.src_valid + s)) continue;
+                    ws += w;
+                    const float* sp = P.src + s;
+#pragma unroll
+                    for (int k = 0; k < K; ++k) acc[k] = fma(w, (double)__ldg(sp + k * P.src_plane_stride), acc[k]);
+                }
+            }
+        }
+        const bool covered = inside && ws >= 1e-6;
+        bool fit = covered;
+        float* dp = P.dst + o;
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            const float v = covered ? (float)(acc[k] / ws) : __ldg(P.fill_out + k);
+            dp[k * P.dst_plane_stride] = v;
+            fit = fit && isfinite(v) && (k != P.gate_k || v > P.gate_gt);
+        }
+        if (P.dst_valid) P.dst_valid[o] = covered ? 1 : 0;
+        if (P.fit_mask) P.fit_mask[o] = fit ? 1 : 0;
+    }
+}
+
+template <int K>
+void launch_warp_planes(dim3 grid, cudaStream_t stream, const PlaneParams& P) {
+    warp_planes_kernel<K><<<grid, dim3(PL_COLS, PL_ROWS), 0, stream>>>(P);
+}
+
 // ---------------------------------------------------------------------------- host side
 int fill_params(WarpParams& P, const hsr_warp_geo_t* geo, long long Hs, long long Ws, long long Hd, long long Wd,
                 int kernel) {
@@ -2059,6 +2141,59 @@ int warp_coords_impl(const hsr_warp_geo_t* geo, long long Hd, long long Wd, doub
     const long long cap = (long long)device_sm_count() * 8;
     if (blocks > cap) blocks = cap;
     warp_coords_kernel<<<(unsigned int)blocks, 32 * WARPS, 0, stream>>>(P);
+    HSR_CUDA(cudaGetLastError());
+    return HSR_OK;
+}
+
+int warp_planes_impl(const float* src, long long Hs, long long Ws, int K, long long src_plane_stride,
+                     const uint8_t* src_valid, const double* coords, const hsr_warp_geo_t* geo, int kernel,
+                     const float* fill_out, int gate_k, float gate_gt, long long Hd, long long Wd, float* dst,
+                     long long dst_plane_stride, uint8_t* dst_valid, uint8_t* fit_mask, cudaStream_t stream) {
+    HSR_REQUIRE(src && dst && src_valid && fill_out, HSR_EINVAL, "null src / dst / src_valid / fill_out pointer");
+    HSR_REQUIRE(coords, HSR_EINVAL, "null coords pointer: pass hsr_warp_coords_f64's output");
+    HSR_REQUIRE(geo, HSR_EINVAL, "null geo pointer");
+    HSR_REQUIRE(K >= 1 && K <= HSR_MAX_SRF_BANDS, HSR_EINVAL, "K = %d outside [1, %d]", K, HSR_MAX_SRF_BANDS);
+    HSR_REQUIRE(kernel == 1 || kernel == 2, HSR_EINVAL, "kernel must be 1 (bilinear) or 2 (cubic), got %d", kernel);
+    HSR_REQUIRE(Hs > 0 && Ws > 0 && Hd >= 0 && Wd >= 0, HSR_EINVAL, "bad shape");
+    HSR_REQUIRE(Hs * Ws < (1LL << 40) && Hd * Wd < (1LL << 40), HSR_EINVAL, "grid too large (limit 2^40 pixels)");
+    HSR_REQUIRE((K == 1 || src_plane_stride >= Hs * Ws) && (K == 1 || dst_plane_stride >= Hd * Wd) &&
+                    src_plane_stride >= 0 && dst_plane_stride >= 0,
+                HSR_EINVAL, "plane stride below the plane size");
+    HSR_REQUIRE((reinterpret_cast<uintptr_t>(coords) & 15) == 0, HSR_EALIGN, "coords not 16-byte aligned");
+    HSR_REQUIRE(gate_k < K, HSR_EINVAL, "gate_k = %d >= K = %d", gate_k, K);
+    PlaneParams P{};
+    const int r0 = kernel == 2 ? 2 : 1;
+    const double xs = geo->xscale > 0.0 ? geo->xscale : 1.0, ys = geo->yscale > 0.0 ? geo->yscale : 1.0;
+    const double rxd = xs < 1.0 ? ceil(r0 / xs) : (double)r0, ryd = ys < 1.0 ? ceil(r0 / ys) : (double)r0;
+    HSR_REQUIRE(rxd <= MAX_TAPS / 2 && ryd <= MAX_TAPS / 2, HSR_EINVAL,
+                "scale (%g, %g) needs a filter radius beyond %d taps", xs, ys, MAX_TAPS / 2);
+    if (Hd == 0 || Wd == 0) return HSR_OK;
+    P.src = src;
+    P.src_valid = src_valid;
+    P.Hs = Hs, P.Ws = Ws, P.src_plane_stride = src_plane_stride;
+    P.coords = coords;
+    P.Hd = Hd, P.Wd = Wd;
+    P.kind = kernel;
+    P.rx = (int)rxd, P.ry = (int)ryd;
+    P.fx = xs < 1.0 ? xs : 1.0;
+    P.fy = ys < 1.0 ? ys : 1.0;
+    P.fill_out = fill_out;
+    P.gate_k = gate_k;
+    P.gate_gt = gate_gt;
+    P.dst = dst;
+    P.dst_plane_stride = dst_plane_stride;
+    P.dst_valid = dst_valid;
+    P.fit_mask = fit_mask;
+    const long long tiles_x = (Wd + PL_COLS - 1) / PL_COLS, tiles_y = (Hd + PL_ROWS - 1) / PL_ROWS;
+    HSR_REQUIRE(tiles_x < 2147483647LL, HSR_EINVAL, "destination too wide");
+    const dim3 grid((unsigned int)tiles_x, (unsigned int)(tiles_y < 65535 ? tiles_y : 65535));
+    typedef void (*launch_fn)(dim3, cudaStream_t, const PlaneParams&);
+    static const launch_fn launch[HSR_MAX_SRF_BANDS] = {
+        launch_warp_planes<1>,  launch_warp_planes<2>,  launch_warp_planes<3>,  launch_warp_planes<4>,
+        launch_warp_planes<5>,  launch_warp_planes<6>,  launch_warp_planes<7>,  launch_warp_planes<8>,
+        launch_warp_planes<9>,  launch_warp_planes<10>, launch_warp_planes<11>, launch_warp_planes<12>,
+        launch_warp_planes<13>, launch_warp_planes<14>, launch_warp_planes<15>, launch_warp_planes<16>};
+    launch[K - 1](grid, stream, P);
     HSR_CUDA(cudaGetLastError());
     return HSR_OK;
 }

@@ -1157,3 +1157,53 @@ def warp_coords(src_gt, dst_gt, dst_shape, *, utm_zone: int = 0, south: bool = F
         out = torch.empty((Hd, Wd, 2), dtype=torch.float64, device=dev)
         _lib.check(_lib.lib().hsr_warp_coords_f64(ctypes.addressof(geo), Hd, Wd, out.data_ptr(), _stream()))
     return out
+
+
+PLANE_WARP_KERNELS = {"bilinear": 1, "cubic": 2}
+
+
+def warp_planes(planes: torch.Tensor, src_valid: torch.Tensor, coords: torch.Tensor, scales, *, kernel: str,
+                fill_out: torch.Tensor, gate_k: int = 0, gate_gt: float = 0.0, out: Optional[torch.Tensor] = None,
+                valid_out: Optional[torch.Tensor] = None, fit_mask_out: Optional[torch.Tensor] = None):
+    """Warp K planar images ``planes`` [K, Hs, Ws] f32 (any plane stride, as ``alloc_planes`` pads them) onto the grid
+    of ``coords`` [Hd, Wd, 2] f64 (:func:`warp_coords`) with the taps of :func:`warp` (``hsr_warp_planes_f32``).
+    ``src_valid`` [Hs, Ws] bool/u8: source pixels whose taps may be used (the GLT valid mask); ``scales`` = (xscale,
+    yscale) of ``EMIT_data.warp.warp_scales``; ``fill_out`` [K] f32: written where the destination is not covered.
+    Returns ``(planes [K, Hd, Wd] f32, dst_valid [Hd, Wd] bool, fit_mask [Hd, Wd] bool)``, the fit mask being
+    ``dst_valid & isfinite(planes).all(0) & (planes[gate_k] > gate_gt)`` (gate_k < 0: no gate)."""
+    code = PLANE_WARP_KERNELS.get(kernel)
+    if code is None:
+        raise ValueError(f"kernel must be one of {sorted(PLANE_WARP_KERNELS)} for a plane warp, got {kernel!r}")
+    p = _cuda(planes, "planes", torch.float32)
+    if p.dim() != 3:
+        raise ValueError(f"planes must be [K, Hs, Ws], got shape {tuple(p.shape)}")
+    K, Hs, Ws = (int(d) for d in p.shape)
+    ps = _plane_stride(p, K, Hs * Ws, "planes")
+    sv = src_valid.view(torch.uint8) if src_valid.dtype == torch.bool else src_valid
+    sv = _cuda(sv, "src_valid", torch.uint8).contiguous()
+    if sv.numel() != Hs * Ws:
+        raise ValueError(f"src_valid must have one entry per source pixel ({Hs} x {Ws}), got shape {tuple(sv.shape)}")
+    co = _cuda(coords, "coords", torch.float64)
+    if co.dim() != 3 or co.shape[2] != 2 or not co.is_contiguous():
+        raise ValueError(f"coords must be a contiguous [Hd, Wd, 2] tensor, got shape {tuple(co.shape)}")
+    Hd, Wd = int(co.shape[0]), int(co.shape[1])
+    fo = _cuda(fill_out, "fill_out", torch.float32).contiguous()
+    if fo.numel() != K:
+        raise ValueError(f"fill_out must have K = {K} entries, got {fo.numel()}")
+    geo = _lib.WarpGeo()
+    geo.xscale, geo.yscale = float(scales[0]), float(scales[1])
+    with torch.cuda.device_of(p):
+        if out is None:
+            out = alloc_planes(K, (Hd, Wd), p.device)
+        else:
+            _cuda(out, "out", torch.float32)
+        ops = _plane_stride(out, K, Hd * Wd, "out")
+        valid = (_mask_out(valid_out, Hd * Wd) if valid_out is not None
+                 else torch.empty(Hd * Wd, dtype=torch.uint8, device=p.device))
+        fm = (_mask_out(fit_mask_out, Hd * Wd) if fit_mask_out is not None
+              else torch.empty(Hd * Wd, dtype=torch.uint8, device=p.device))
+        _lib.check(_lib.lib().hsr_warp_planes_f32(p.data_ptr(), Hs, Ws, K, ps, sv.data_ptr(), co.data_ptr(),
+                                                  ctypes.addressof(geo), code, fo.data_ptr(), int(gate_k),
+                                                  float(gate_gt), Hd, Wd, out.data_ptr(), ops, valid.data_ptr(),
+                                                  fm.data_ptr(), _stream()))
+    return out, valid.view(torch.bool).view(Hd, Wd), fm.view(torch.bool).view(Hd, Wd)

@@ -10,6 +10,9 @@ from HBM once:
     fit_moments      fp64 normal equations of the planes vs the S2 reference under that mask
                      [+ all-reduce across ranks]
     poly_solve_apply (K, deg+1) coefficients and the colour-matched planes, clipped to [0, 1]
+
+``synthesize_on_s2_grid`` runs the same pass on the Sentinel-2 UTM grid, where the reference fits: glt_srf, then a warp
+of the K planes onto the S2 grid (``warp_planes``), then the same fit and solve / apply.
 """
 from __future__ import annotations
 
@@ -21,6 +24,7 @@ import torch
 from . import dist as hdist
 from . import kernels
 from ._host import cuda_device, to_device
+from .EMIT_data.warp import S2Target, s2_target, warp_planes  # noqa: F401  (the building blocks of synthesize_on_s2_grid)
 from .s2_emit.srf import srf_fold_weights
 
 NO_DATA_VALUE = kernels.NO_DATA_VALUE
@@ -46,6 +50,7 @@ class PairResult:
                                              # ([K, 1, 2], the same on every rank, for a global fit with stretch_scope="fit")
     y_limits: Optional[torch.Tensor] = None  # ... and of the S2 reference
     raw_rows: Optional[tuple] = None         # synthesize_slab: the [row0, row1) raw rows that were staged
+    grid: Optional[S2Target] = None          # synthesize_on_s2_grid: the S2 grid of bands / matched / valid / fit_mask
 
 
 class PairSynthesizer:
@@ -174,6 +179,12 @@ class PairSynthesizer:
                                                         raw_rows_total=raw_rows_total)
         ex = exchange.next() if exchange is not None and exchange.world > 1 else None
         reduce = self._global_reduce(group) if global_fit else None
+        return self._fit_apply(bands, s2_ref, valid, fm, diag, matched_out=matched_out, ex=ex, reduce=reduce,
+                               allreduce=allreduce, group=group, ortho=ortho)
+
+    def _fit_apply(self, bands, s2_ref, valid, fm, diag, *, matched_out=None, ex=None, reduce=None,
+                   allreduce=False, group=None, ortho=None, grid=None) -> PairResult:
+        """The tail of one image: fit (+ all-reduce), then solve / apply."""
         mom, fm, xl, yl = self.fit(bands, s2_ref, valid, fm, exchange=ex, reduce=reduce)
         if allreduce and ex is None:
             hdist.allreduce_moments(mom, group)
@@ -184,7 +195,31 @@ class PairSynthesizer:
         if gmom is not None:
             mom = gmom
         return PairResult(bands, matched, coeffs.view(self.K, self.deg + 1), valid, fm.view(valid.shape), diag,
-                          mom.view(self.K, -1), ortho, self.band_names, xl, yl)
+                          mom.view(self.K, -1), ortho, self.band_names, xl, yl, grid=grid)
+
+    # ------------------------------------------------------------------ one granule on the Sentinel-2 grid
+    def synthesize_on_s2_grid(self, raw: torch.Tensor, glt_x: torch.Tensor, glt_y: torch.Tensor, s2_ref: torch.Tensor,
+                              target: S2Target, *, transpose_raw_yx: bool = False, bands_out=None,
+                              matched_out=None) -> PairResult:
+        """The pair on the Sentinel-2 UTM grid ``target`` (:func:`hsr_b200.EMIT_data.warp.s2_target`), where the
+        reference fits: ``s2_ref`` [K, Hd, Wd] f32 is the S2 stack on that grid.  Instead of warping the B-band ortho
+        cube and integrating the SRF over it (nc_to_envi's gdalwarp, then synth.py:9-45), the K pseudo-S2 planes of
+        the fused GLT + SRF pass are warped (``kernels.warp_planes``, GLT-valid pixels only): both steps are linear and
+        the warp's tap weights are the same for every band, so the result is the same up to fp rounding.
+        Stages: glt_srf, the target's cached coordinates, warp_planes, then the fit and solve / apply of
+        :meth:`synthesize` (stretch, ``y_finite``, gate band and clip as there, on the S2-grid planes).
+        ``bands``, ``matched``, ``valid`` and ``fit_mask`` of the result are on the target grid, ``diag`` is the GLT
+        diagnostics of the source pass and ``grid`` is ``target``.  Deviation from the reference: a GLT-valid raw
+        spectrum holding the nodata value in some or all of its bands is used as data (DESIGN section 7)."""
+        Hd, Wd = target.shape
+        if tuple(s2_ref.shape) != (self.K, Hd, Wd):
+            raise ValueError(f"s2_ref must be [K={self.K}, {Hd}, {Wd}] on the target grid, got {tuple(s2_ref.shape)}")
+        src, valid, diag, _ = self.bands_from_raw(raw, glt_x, glt_y, transpose_raw_yx=transpose_raw_yx)
+        fm = torch.empty((Hd, Wd), dtype=torch.bool, device=src.device)
+        bands, dvalid, fm = kernels.warp_planes(src, valid, target.coords(src.device), target.scales,
+                                                kernel=target.kernel, fill_out=self.fill_out, gate_k=self.gate_k,
+                                                gate_gt=0.0, out=bands_out, fit_mask_out=fm)
+        return self._fit_apply(bands, s2_ref, dvalid, fm, diag, matched_out=matched_out, grid=target)
 
     # ------------------------------------------------------------------ a row slab of a mosaic
     def synthesize_slab(self, raw, glt_x: torch.Tensor, glt_y: torch.Tensor, s2_ref: torch.Tensor, *,

@@ -557,6 +557,34 @@ HSR_API size_t hsr_warp_workspace_bytes(int64_t Hd, int64_t Wd);
 /* coords[Hd, Wd, 2] = source pixel coordinates (x, y; pixel (i, j) has its centre at (i + 0.5, j + 0.5)) of every
  * destination pixel centre — the transformer of hsr_warp_f32 on its own (tests, diagnostics, footprints). */
 HSR_API int hsr_warp_coords_f64(const hsr_warp_geo_t* geo, int64_t Hd, int64_t Wd, double* coords, void* stream);
+/*
+ * Warp of K planar images onto the Sentinel-2 grid: the pseudo-S2 planes of hsr_glt_srf_f32 instead of the B-band
+ * ortho cube.  The SRF contraction and the warp are both linear, and the warp's tap weights are the same for every
+ * band wherever a source pixel is all data or all nodata, which the GLT fill is; so warping the K planes gives
+ * SRF(warp(cube)).  Tap rule of hsr_warp_f32 (kernel 1 bilinear, 2 cubic; radius ceil(r / scale) per axis below
+ * scale 1 with the argument scaled; tap weight = fp32 rounding of the fp64 product wy * wx), except that validity is
+ * per source pixel: a tap is skipped when its weight is 0 (even over a NaN), when it is outside the source or when
+ * src_valid is 0.  The K sums and the weight sum are accumulated in fp64 and dst[k] = f32(acc[k] / ws).  A centre
+ * outside the source or ws < 1e-6: dst[k] = fill_out[k] and dst_valid = 0.  Non-finite values propagate as in the
+ * per-band warp.  fit_mask = dst_valid & all_k isfinite(dst[k]) & (dst[gate_k] > gate_gt) (gate_k < 0: no gate),
+ * the rule hsr_glt_srf_f32 writes.
+ *   src       [K] planes of Hs * Ws f32, plane k at src + k * src_plane_stride (>= Hs * Ws unless K == 1);
+ *   src_valid [Hs, Ws] u8, 1 = the pixel's taps may be used (the GLT valid mask);
+ *   coords    [Hd, Wd, 2] f64 from hsr_warp_coords_f64 (16-byte aligned); required;
+ *   geo       only xscale / yscale are read (<= 0 reads as 1);
+ *   fill_out  [K] f32 device; dst [K] planes of Hd * Wd with dst_plane_stride; dst_valid, fit_mask [Hd, Wd] u8,
+ *             both nullable.
+ * Exactness: equal to pseudo_s2_srf_integral(warp(glt_ortho(raw))) in exact arithmetic; in fp, planes within
+ * 1e-5 * C_k + 1e-7 where C_k = sum_t |w_t| |v_tk| / |sum_t w_t| (the conditioning of the renormalised sum), identical
+ * coverage and NaN / Inf patterns, fill_out where uncovered.  Deviation: a GLT-valid raw spectrum holding the nodata
+ * value in some or all of its bands is used as data (the per-band warp skips it for those bands).
+ * HSR_EINVAL: K outside 1..16, NULL coords (or src / dst / src_valid / fill_out / geo), kernel not 1 / 2, a filter
+ * radius beyond 8 taps (scale < 0.25 cubic, < 0.125 bilinear), plane strides below the plane size, gate_k >= K.
+ */
+HSR_API int hsr_warp_planes_f32(const float* src, int64_t Hs, int64_t Ws, int K, int64_t src_plane_stride,
+                                const uint8_t* src_valid, const double* coords, const hsr_warp_geo_t* geo, int kernel,
+                                const float* fill_out, int gate_k, float gate_gt, int64_t Hd, int64_t Wd, float* dst,
+                                int64_t dst_plane_stride, uint8_t* dst_valid, uint8_t* fit_mask, void* stream);
 
 /*
  * Peer blocks for hsr_exchange_t.  hsr_peer_alloc creates (cudaMalloc + zero) this rank's block — the one
