@@ -14,7 +14,7 @@ import threading
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC_DIR = os.path.join(_HERE, "csrc")
 LIB_PATH = os.path.join(CSRC_DIR, "libhsr_b200.so")
-ABI_VERSION = 6
+ABI_VERSION = 7
 HEADER_PATH = os.path.join(os.path.dirname(_HERE), "include", "hsr_b200.h")
 
 HSR_OP_POLY_MOMENTS = 1

@@ -10,11 +10,12 @@
 //     scaled where the destination is coarser than the source; taps outside the source or equal to nodata are
 //     skipped PER BAND and the sum is divided by the accumulated weight; centre outside the source or accumulated
 //     weight < 1e-6 -> dst_nodata.  NaN is an ordinary value.
-// Default kernel: warp_lane_kernel (lanes across destination pixels, the tap box of a 16 x 8 tile staged transposed in
-// shared memory, per-pixel weights in registers for the whole spectrum).  The band-per-lane kernels it replaced remain
-// as fall-backs: warp_pipe_kernel (filter radii beyond 4) and warp_tile_kernel (no coordinate workspace).  All of them
-// classify what they stage: no nodata -> plain FMAs under a uniform weight sum; all nodata -> skipped; band-specific
-// nodata -> exact per-element weights.
+// Kernels 1 and 2 (bilinear, cubic) take the source coordinates of every destination pixel from the caller's workspace
+// (warp_coords_kernel) and then run one of three kernels: warp_quad_kernel (TMA-staged 2 x 2 pixel blocks, the default)
+// or warp_lane_kernel (records that are not 16-byte aligned) for filter radii up to 4; warp_exact_kernel (fp64 straight
+// from global memory) for wider filters and for sources of 2^32 pixels or more.  The two fast kernels classify what they
+// stage (no nodata -> plain FMAs under a uniform weight sum; all nodata -> skipped; band-specific nodata -> exact
+// per-element weights) and list the pixels whose fp32 quotient is ill-conditioned; warp_exact_kernel recomputes those.
 #include <cuda.h>
 #include <math.h>
 #include <stdlib.h>
@@ -27,9 +28,6 @@ namespace {
 
 constexpr int WARPS = 8;        // warps per CTA
 constexpr int MAX_TAPS = 16;    // taps per axis: radius <= 8, i.e. scale >= 0.25 for cubic
-constexpr int GB = 128;         // bands per CTA (32 lanes x 4)
-constexpr int TILE_PX = 64;     // destination pixels per tile (<= 8 x 8)
-constexpr int BOX_CAP = 192;    // source pixels staged per tile and band group: 192 x 512 B = 96 KB, two CTAs per SM
 
 struct WarpParams {
     const float* src;
@@ -47,9 +45,8 @@ struct WarpParams {
     int kind;                   // 0 nearest, 1 bilinear, 2 cubic, 3 average
     int rx, ry;                 // radius in taps per axis
     double fx, fy;              // min(scale, 1) per axis
-    double* coords;             // hsr_warp_coords_f64 only
-    int tile_w, tile_h;         // destination tile of one CTA (tile_w * tile_h <= TILE_PX)
-    unsigned long long* redo_list;   // warp_quad_kernel -> warp_fixup_kernel: (pixel << 8 | band group) of ill-conditioned quotients
+    double* coords;             // source coordinates of every destination pixel (warp_coords_kernel)
+    unsigned long long* redo_list;   // quad / lane kernel -> warp_exact_kernel: (pixel << 8 | band group) of ill-conditioned quotients
     unsigned int* redo_count;
     unsigned int redo_cap;
 };
@@ -213,12 +210,7 @@ __global__ void __launch_bounds__(256) warp_point_kernel(const WarpParams P) {
     }
 }
 
-// One CTA = one TW x TH tile of the destination and one group of GB = 128 bands (lane l of a warp owns bands
-// 4l .. 4l+3 of the group).  (1) 64 threads transform the tile's pixel centres (fp64) and the CTA takes the bounding
-// box of all their taps in the source; (2) the 8 warps copy the box's spectra (512 B per pixel and group) into shared
-// memory ONCE — the only global reads of the tile; 16-byte loads when the records allow, scalar otherwise; (3) each warp
-// resamples 8 destination pixels from shared memory (conflict-free 16-byte loads, fp32 FMAs).  A box larger than the
-// staging buffer (extreme down-scaling or rotation) falls back to reading the taps from global memory, same arithmetic.
+// bands b .. b+3 of one spectrum, 4-byte loads unless the records are 16-byte aligned
 template <bool SRC_VEC>
 __device__ __forceinline__ float4 load_group_raw(const float* __restrict__ rec, int b, int bands, bool act) {
     // bands b .. b+3 of one spectrum (words beyond `bands`: record padding with SRC_VEC, 0 otherwise)
@@ -243,627 +235,19 @@ __device__ __forceinline__ float4 pad_fix(float4 v, int b, int bands) {
     return v;
 }
 
-template <bool SRC_VEC>
-__device__ __forceinline__ float4 load_group(const float* __restrict__ rec, int b, int bands, bool act) {
-    return pad_fix(load_group_raw<SRC_VEC>(rec, b, bands, act), b, bands);
-}
-
-template <bool SRC_VEC, bool DST_VEC>
-__global__ void __launch_bounds__(32 * WARPS, 2) warp_tile_kernel(const WarpParams P) {
-    extern __shared__ __align__(16) float4 box[];          // [BOX_CAP][32]
-    __shared__ double s_xy[TILE_PX][2];
-    __shared__ int s_box[4];                                // min ix, max ix, min iy, max iy over the tile's pixels
-    __shared__ unsigned char s_cls[BOX_CAP];                // per staged source pixel: 0 clean, 1 fill, 2 mixed
-    __shared__ double s_w1[WARPS][32];
-    __shared__ float s_w[WARPS][MAX_TAPS * MAX_TAPS];
-    const int tid = threadIdx.x, lane = tid & 31, wib = tid >> 5;
-    double* w1 = s_w1[wib];
-    float* tw = s_w[wib];
-    const int TW = P.tile_w, TH = P.tile_h, npix_tile = TW * TH;
-    const long long tiles_x = (P.Wd + TW - 1) / TW, tiles_y = (P.Hd + TH - 1) / TH, ntiles = tiles_x * tiles_y;
-    const int b = (int)blockIdx.y * GB + 4 * lane;          // my first band
-    const bool act = b < P.bands;
-    const int ntx = 2 * P.rx, nty = 2 * P.ry;
-    const float nd = P.nodata;
-    const bool has_nd = P.has_nodata != 0;
-    const unsigned int FULL = 0xffffffffu;
-    const float dnd = P.dst_nodata;
-
-    for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        const long long ty = tile / tiles_x, tx = tile - ty * tiles_x;
-        // ---- 1. transform the pixel centres, bounding box of the taps
-        if (tid < 4) s_box[tid] = (tid & 1) ? -2147483647 : 2147483647;
-        __syncthreads();
-        if (tid < npix_tile) {
-            const long long r = ty * TH + tid / TW, c = tx * TW + tid % TW;
-            double px = -1.0, py = -1.0;
-            if (r < P.Hd && c < P.Wd) {
-                if (P.coords) {     // transformed beforehand by warp_coords_kernel (all SMs busy instead of one warp per CTA)
-                    const double2 xy = __ldg(reinterpret_cast<const double2*>(P.coords) + (r * P.Wd + c));
-                    px = xy.x;
-                    py = xy.y;
-                } else {
-                    dst_to_src(P, (double)c + 0.5, (double)r + 0.5, px, py);
-                }
-            }
-            const bool inside = px >= 0.0 && px < (double)P.Ws && py >= 0.0 && py < (double)P.Hs;
-            s_xy[tid][0] = inside ? px : -1.0;
-            s_xy[tid][1] = inside ? py : -1.0;
-            if (inside) {
-                const int ix = (int)floor(px - 0.5), iy = (int)floor(py - 0.5);
-                atomicMin(&s_box[0], ix);
-                atomicMax(&s_box[1], ix);
-                atomicMin(&s_box[2], iy);
-                atomicMax(&s_box[3], iy);
-            }
-        }
-        __syncthreads();
-        long long bx0 = (long long)s_box[0] + 1 - P.rx, bx1 = (long long)s_box[1] + P.rx;
-        long long by0 = (long long)s_box[2] + 1 - P.ry, by1 = (long long)s_box[3] + P.ry;
-        const bool any_inside = s_box[1] >= s_box[0];
-        bx0 = bx0 < 0 ? 0 : bx0;
-        by0 = by0 < 0 ? 0 : by0;
-        bx1 = bx1 >= P.Ws ? P.Ws - 1 : bx1;
-        by1 = by1 >= P.Hs ? P.Hs - 1 : by1;
-        const int bw = any_inside ? (int)(bx1 - bx0 + 1) : 0, bh = any_inside ? (int)(by1 - by0 + 1) : 0;
-        const bool staged = any_inside && (long long)bw * bh <= BOX_CAP;
-        // ---- 2. stage the box: one warp per source pixel, 512 B of its spectrum; classify it once for all its uses:
-        //         0 = no band of the group is nodata, 1 = every band is (a fill pixel), 2 = some are
-        if (staged) {
-            constexpr int CB = 8;      // loads in flight per warp
-            const int nbox = bw * bh;
-            for (int p0 = wib; p0 < nbox; p0 += WARPS * CB) {
-                float4 v[CB];
-#pragma unroll
-                for (int u = 0; u < CB; ++u) {
-                    const int p = p0 + u * WARPS;
-                    v[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-                    if (p < nbox) {
-                        const long long yy = by0 + p / bw, xx = bx0 + p % bw;
-                        v[u] = load_group_raw<SRC_VEC>(P.src + (yy * P.Ws + xx) * P.src_pix_stride, b, P.bands, act);
-                    }
-                }
-#pragma unroll
-                for (int u = 0; u < CB; ++u) {
-                    const int p = p0 + u * WARPS;
-                    if (p >= nbox) break;
-                    const float4 x = pad_fix(v[u], b, P.bands);
-                    box[p * 32 + lane] = x;
-                    int cls = 0;
-                    if (has_nd) {
-                        const bool any = act && (x.x == nd || x.y == nd || x.z == nd || x.w == nd);
-                        const bool all = !act || (x.x == nd && x.y == nd && x.z == nd && x.w == nd);
-                        cls = !__any_sync(FULL, any) ? 0 : (__all_sync(FULL, all) ? 1 : 2);
-                    }
-                    if (lane == 0) s_cls[p] = (unsigned char)cls;
-                }
-            }
-        }
-        __syncthreads();
-        // (barrier) + does any staged pixel hold a nodata?  Tiles inside the swath do not: they take the lean loop below
-        const bool box_clean = __syncthreads_or(staged && tid < bw * bh && s_cls[tid] != 0) == 0;
-        // ---- 3. resample: warp w takes pixels w, w + 8, ... of the tile
-        for (int q = wib; q < npix_tile; q += WARPS) {
-            const long long r = ty * TH + q / TW, c = tx * TW + q % TW;
-            if (r >= P.Hd || c >= P.Wd) continue;
-            const double px = s_xy[q][0], py = s_xy[q][1];
-            float* outp = P.dst + (r * P.Wd + c) * P.dst_pix_stride + b;
-            float4 o = make_float4(dnd, dnd, dnd, dnd);
-            if (px >= 0.0) {
-                // separable weights: lane t < 16 computes column tap t, lane 16 + t row tap t (fp64), then the products
-                const double fxp = floor(px - 0.5), fyp = floor(py - 0.5);
-                const long long ix = (long long)fxp, iy = (long long)fyp;
-                {
-                    const bool isx = lane < 16;
-                    const int t = (isx ? lane : lane - 16) + 1 - (isx ? P.rx : P.ry);
-                    const double dd = isx ? px - 0.5 - fxp : py - 0.5 - fyp;
-                    __syncwarp();                       // everybody is done with the previous pixel's tables
-                    w1[lane] = tap_weight(P.kind, ((double)t - dd) * (isx ? P.fx : P.fy));
-                    __syncwarp();
-                    for (int t2 = lane; t2 < ntx * nty; t2 += 32) {
-                        const int j = t2 / ntx, k = t2 - j * ntx;
-                        tw[t2] = (float)(w1[16 + j] * w1[k]);
-                    }
-                    __syncwarp();
-                }
-                // taps inside the source: rows [jlo, jhi), columns [klo, khi) of the window whose first tap is (x0t, y0t)
-                const long long x0t = ix + 1 - P.rx, y0t = iy + 1 - P.ry;
-                int jlo = y0t < 0 ? (int)-y0t : 0, klo = x0t < 0 ? (int)-x0t : 0;
-                int jhi = y0t + nty > P.Hs ? (int)(P.Hs - y0t) : nty, khi = x0t + ntx > P.Ws ? (int)(P.Ws - x0t) : ntx;
-                // a tap of weight zero contributes nothing (not even its NaN): zero rows / columns at the ends of the
-                // window (the widened filter's support is rarely full) are trimmed, the others are skipped tap by tap
-                const unsigned int nzw = __ballot_sync(FULL, w1[lane] != 0.0);      // bits 0..15 columns, 16..31 rows
-                {
-                    const unsigned int cm = (nzw & 0xffffu) & (khi >= 32 ? 0xffffffffu : ((1u << khi) - 1u)) & ~((1u << klo) - 1u);
-                    const unsigned int rm = (nzw >> 16) & ((1u << jhi) - 1u) & ~((1u << jlo) - 1u);
-                    if (cm == 0u || rm == 0u) {
-                        jlo = jhi = 0;
-                    } else {
-                        klo = __ffs((int)cm) - 1;
-                        khi = 32 - __clz((int)cm);
-                        jlo = __ffs((int)rm) - 1;
-                        jhi = 32 - __clz((int)rm);
-                    }
-                }
-                const unsigned int span = ((1u << khi) - 1u) & ~((1u << klo) - 1u);
-                const bool dense_cols = ((nzw & 0xffffu) & span) == span && (((nzw >> 16) >> jlo) & ((1u << (jhi - jlo)) - 1u)) == ((1u << (jhi - jlo)) - 1u);
-                float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f, m0 = 0.f, m1 = 0.f, m2 = 0.f, m3 = 0.f, wu = 0.f;
-                if (staged && box_clean && dense_cols) {
-                    // lean loop: no nodata anywhere in the box, no zero weight inside the trimmed window
-                    const float4* bp = box + ((int)(y0t - by0) * bw + (int)(x0t - bx0)) * 32 + lane;
-                    for (int j = jlo; j < jhi; ++j) {
-                        const float4* rowb = bp + j * bw * 32;
-                        const float* twj = tw + j * ntx;
-#pragma unroll 2
-                        for (int k = klo; k < khi; ++k) {
-                            const float w = twj[k];
-                            const float4 v = rowb[k * 32];
-                            a0 = fmaf(w, v.x, a0);
-                            a1 = fmaf(w, v.y, a1);
-                            a2 = fmaf(w, v.z, a2);
-                            a3 = fmaf(w, v.w, a3);
-                            wu += w;
-                        }
-                    }
-                } else if (staged) {
-                    const int base = (int)(y0t - by0) * bw + (int)(x0t - bx0);
-                    for (int j = jlo; j < jhi; ++j) {
-                        const int rowi = base + j * bw;
-                        const float* twj = tw + j * ntx;
-#pragma unroll 2
-                        for (int k = klo; k < khi; ++k) {
-                            const int pi = rowi + k;
-                            const int cls = s_cls[pi];                  // three independent shared-memory loads, then branch
-                            const float w = twj[k];
-                            const float4 v = box[pi * 32 + lane];
-                            if (cls == 1 || w == 0.f) continue;         // a fill pixel (skipped by every band) or a zero weight
-                            if (cls == 0) {                             // plain FMAs under a warp-uniform weight sum
-                                a0 = fmaf(w, v.x, a0);
-                                a1 = fmaf(w, v.y, a1);
-                                a2 = fmaf(w, v.z, a2);
-                                a3 = fmaf(w, v.w, a3);
-                                wu += w;
-                            } else {                                    // band-specific nodata: exact per element
-                                const float w0 = v.x == nd ? 0.f : w, w1q = v.y == nd ? 0.f : w;
-                                const float w2 = v.z == nd ? 0.f : w, w3 = v.w == nd ? 0.f : w;
-                                a0 = fmaf(w0, v.x, a0);
-                                a1 = fmaf(w1q, v.y, a1);
-                                a2 = fmaf(w2, v.z, a2);
-                                a3 = fmaf(w3, v.w, a3);
-                                m0 += w0;
-                                m1 += w1q;
-                                m2 += w2;
-                                m3 += w3;
-                            }
-                        }
-                    }
-                } else {    // box too large for the staging buffer: the same taps straight from global memory
-                    for (int j = jlo; j < jhi; ++j) {
-                        const float* rowp = P.src + ((y0t + j) * P.Ws + x0t) * P.src_pix_stride;
-                        for (int k = klo; k < khi; ++k) {
-                            const float w = tw[j * ntx + k];
-                            if (w == 0.f) continue;
-                            const float4 v = load_group<SRC_VEC>(rowp + k * P.src_pix_stride, b, P.bands, act);
-                            const bool h = has_nd && act;
-                            const float w0 = (h && v.x == nd) ? 0.f : w, w1q = (h && v.y == nd) ? 0.f : w;
-                            const float w2 = (h && v.z == nd) ? 0.f : w, w3 = (h && v.w == nd) ? 0.f : w;
-                            a0 = fmaf(w0, v.x, a0);
-                            a1 = fmaf(w1q, v.y, a1);
-                            a2 = fmaf(w2, v.z, a2);
-                            a3 = fmaf(w3, v.w, a3);
-                            m0 += w0;
-                            m1 += w1q;
-                            m2 += w2;
-                            m3 += w3;
-                        }
-                    }
-                }
-                const float s0 = wu + m0, s1 = wu + m1, s2 = wu + m2, s3 = wu + m3;
-                o.x = s0 >= 1e-6f ? __fdiv_rn(a0, s0) : dnd;
-                o.y = s1 >= 1e-6f ? __fdiv_rn(a1, s1) : dnd;
-                o.z = s2 >= 1e-6f ? __fdiv_rn(a2, s2) : dnd;
-                o.w = s3 >= 1e-6f ? __fdiv_rn(a3, s3) : dnd;
-            }
-            if (act) {
-                if (DST_VEC) {
-                    __stcs(reinterpret_cast<float4*>(outp), o);
-                } else {
-                    __stcs(outp, o.x);
-                    if (b + 1 < P.bands) __stcs(outp + 1, o.y);
-                    if (b + 2 < P.bands) __stcs(outp + 2, o.z);
-                    if (b + 3 < P.bands) __stcs(outp + 3, o.w);
-                }
-            }
-        }
-        __syncthreads();        // the next tile overwrites s_xy / s_box / box
-    }
-}
-
-// ---------------------------------------------------------------------------- pipelined variant
-// The fast path (coordinates transformed beforehand, <= 64 taps): ONE persistent CTA per SM with 16 warps and TWO staging
-// buffers.  Work is a sequence of stages (tile, band group); while the warps resample stage s from buffer s & 1, the
-// cp.async copies of stage s + 1 land in the other buffer.  What depends on the tile only — bounding box, separable
-// weights, trimmed windows of its 32 pixels — is prepared once per tile (kept in shared memory for its band groups).
-constexpr int PWARPS = 16;
-constexpr int PTILE = 32;       // destination pixels per tile (8 x 4 at most)
-constexpr int PTAPS = 64;       // taps per pixel
-
-struct TileState {
-    int box[4];                 // scratch: min ix, max ix, min iy, max iy
-    int bx0, by0, bw, bh, staged;
-    double xy[PTILE][2];
-    float tw[PTILE][PTAPS];
-    float wsum[PTILE];          // sum of the weights of the window [jlo, jhi) x [0, ntx)
-    int meta[PTILE][8];         // inside, jlo, jhi, klo, khi, x0t, y0t, flags: 1 dense (no zero weight inside the trimmed
-                                // window), 2 whole rows usable (all ntx columns inside the source)
-};
-
-__device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(smem_u32(smem)), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async4(void* smem, const void* gmem) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(smem_u32(smem)), "l"(gmem) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
-
-// one row of N taps: acc += w[k] * v[k] for the lane's four bands; weights by 8-byte loads (rows of N = 4, 6, 8 floats
-// start on 8-byte boundaries), values by conflict-free 16-byte loads
-template <int N>
-__device__ __forceinline__ void row_fma(const float4* __restrict__ rowb, const float* __restrict__ twj, float& a0, float& a1,
-                                        float& a2, float& a3) {
-    float w[N];
-#pragma unroll
-    for (int k = 0; k < N; k += 2) {
-        const float2 t = *reinterpret_cast<const float2*>(twj + k);
-        w[k] = t.x;
-        w[k + 1] = t.y;
-    }
-    float4 v[N];
-#pragma unroll
-    for (int k = 0; k < N; ++k) v[k] = rowb[k * 32];
-#pragma unroll
-    for (int k = 0; k < N; ++k) {
-        a0 = fmaf(w[k], v[k].x, a0);
-        a1 = fmaf(w[k], v[k].y, a1);
-        a2 = fmaf(w[k], v[k].z, a2);
-        a3 = fmaf(w[k], v[k].w, a3);
-    }
-}
-
-template <bool SRC_VEC, bool DST_VEC>
-__global__ void __launch_bounds__(32 * PWARPS, 1) warp_pipe_kernel(const WarpParams P) {
-    extern __shared__ __align__(16) float4 dyn[];            // two boxes of [BOX_CAP][32] float4
-    __shared__ TileState s_tile[2];
-    __shared__ unsigned char s_cls[2][BOX_CAP];
-    __shared__ double s_w1[PWARPS][32];
-    const int tid = threadIdx.x, lane = tid & 31, wib = tid >> 5;
-    const int TW = P.tile_w, TH = P.tile_h, npix_tile = TW * TH;
-    const long long tiles_x = (P.Wd + TW - 1) / TW, tiles_y = (P.Hd + TH - 1) / TH, ntiles = tiles_x * tiles_y;
-    const int G = (P.bands + GB - 1) / GB;
-    const int ntx = 2 * P.rx, nty = 2 * P.ry;
-    const float nd = P.nodata, dnd = P.dst_nodata;
-    const bool has_nd = P.has_nodata != 0;
-    const unsigned int FULL = 0xffffffffu;
-    const int tw_shift = 31 - __clz(TW);
-    const long long my_tiles = blockIdx.x < ntiles ? (ntiles - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
-    const long long nstages = my_tiles * G;
-
-    // ---- per tile: coordinates -> box -> weights and windows of its pixels
-    auto prepare_tile = [&](long long it) {
-        TileState& T = s_tile[it & 1];
-        const long long tile = blockIdx.x + it * gridDim.x;
-        const long long ty = tile / tiles_x, tx = tile - ty * tiles_x;
-        if (tid < 4) T.box[tid] = (tid & 1) ? -2147483647 : 2147483647;
-        __syncthreads();
-        if (tid < npix_tile) {
-            const long long r = ty * TH + tid / TW, c = tx * TW + tid % TW;
-            double px = -1.0, py = -1.0;
-            if (r < P.Hd && c < P.Wd) {
-                const double2 xy = __ldg(reinterpret_cast<const double2*>(P.coords) + (r * P.Wd + c));
-                px = xy.x;
-                py = xy.y;
-            }
-            const bool inside = px >= 0.0 && px < (double)P.Ws && py >= 0.0 && py < (double)P.Hs;
-            T.xy[tid][0] = inside ? px : -1.0;
-            T.xy[tid][1] = inside ? py : -1.0;
-            if (inside) {
-                const int ix = (int)floor(px - 0.5), iy = (int)floor(py - 0.5);
-                atomicMin(&T.box[0], ix);
-                atomicMax(&T.box[1], ix);
-                atomicMin(&T.box[2], iy);
-                atomicMax(&T.box[3], iy);
-            }
-        }
-        __syncthreads();
-        long long bx0 = (long long)T.box[0] + 1 - P.rx, bx1 = (long long)T.box[1] + P.rx;
-        long long by0 = (long long)T.box[2] + 1 - P.ry, by1 = (long long)T.box[3] + P.ry;
-        const bool any_inside = T.box[1] >= T.box[0];
-        bx0 = bx0 < 0 ? 0 : bx0;
-        by0 = by0 < 0 ? 0 : by0;
-        bx1 = bx1 >= P.Ws ? P.Ws - 1 : bx1;
-        by1 = by1 >= P.Hs ? P.Hs - 1 : by1;
-        const int bw = any_inside ? (int)(bx1 - bx0 + 1) : 0, bh = any_inside ? (int)(by1 - by0 + 1) : 0;
-        if (tid == 0) {
-            T.bx0 = (int)bx0;
-            T.by0 = (int)by0;
-            T.bw = bw;
-            T.bh = bh;
-            T.staged = any_inside && (long long)bw * bh <= BOX_CAP;
-        }
-        double* w1 = s_w1[wib];
-        for (int q = wib; q < npix_tile; q += PWARPS) {
-            const double px = T.xy[q][0], py = T.xy[q][1];
-            int* M = T.meta[q];
-            if (!(px >= 0.0)) {
-                if (lane == 0) M[0] = 0;
-                continue;
-            }
-            const double fxp = floor(px - 0.5), fyp = floor(py - 0.5);
-            const long long ix = (long long)fxp, iy = (long long)fyp;
-            const bool isx = lane < 16;
-            const int t = (isx ? lane : lane - 16) + 1 - (isx ? P.rx : P.ry);
-            const double dd = isx ? px - 0.5 - fxp : py - 0.5 - fyp;
-            __syncwarp();
-            w1[lane] = tap_weight(P.kind, ((double)t - dd) * (isx ? P.fx : P.fy));
-            __syncwarp();
-            for (int t2 = lane; t2 < ntx * nty; t2 += 32) {
-                const int j = t2 / ntx, k = t2 - j * ntx;
-                T.tw[q][t2] = (float)(w1[16 + j] * w1[k]);
-            }
-            const long long x0t = ix + 1 - P.rx, y0t = iy + 1 - P.ry;
-            int jlo = y0t < 0 ? (int)-y0t : 0, klo = x0t < 0 ? (int)-x0t : 0;
-            int jhi = y0t + nty > P.Hs ? (int)(P.Hs - y0t) : nty, khi = x0t + ntx > P.Ws ? (int)(P.Ws - x0t) : ntx;
-            const unsigned int nzw = __ballot_sync(FULL, w1[lane] != 0.0);
-            const unsigned int cm = (nzw & 0xffffu) & ((1u << khi) - 1u) & ~((1u << klo) - 1u);
-            const unsigned int rm = (nzw >> 16) & ((1u << jhi) - 1u) & ~((1u << jlo) - 1u);
-            if (cm == 0u || rm == 0u) {
-                jlo = jhi = klo = khi = 0;
-            } else {
-                klo = __ffs((int)cm) - 1;
-                khi = 32 - __clz((int)cm);
-                jlo = __ffs((int)rm) - 1;
-                jhi = 32 - __clz((int)rm);
-            }
-            const unsigned int cspan = ((1u << khi) - 1u) & ~((1u << klo) - 1u), rspan = ((1u << jhi) - 1u) & ~((1u << jlo) - 1u);
-            // weight sum of the rows [jlo, jhi) over ALL ntx columns (the lean loop below runs whole rows: columns
-            // trimmed for a zero weight add exactly 0); fixed order: lanes stride the taps, then a shuffle tree
-            __syncwarp();
-            float ws = 0.f;
-            for (int t2 = jlo * ntx + lane; t2 < jhi * ntx; t2 += 32) ws += T.tw[q][t2];
-#pragma unroll
-            for (int o = 16; o > 0; o >>= 1) ws += __shfl_xor_sync(FULL, ws, o);
-            const bool whole = x0t >= 0 && x0t + ntx <= P.Ws;
-            if (lane == 0) {
-                M[0] = 1;
-                M[1] = jlo;
-                M[2] = jhi;
-                M[3] = klo;
-                M[4] = khi;
-                M[5] = (int)x0t;
-                M[6] = (int)y0t;
-                M[7] = (((cm & cspan) == cspan && (rm & rspan) == rspan) ? 1 : 0) | (whole && rm != 0u ? 2 : 0);
-                T.wsum[q] = ws;
-            }
-        }
-        __syncthreads();
-    };
-
-    // ---- copy of one stage's box into its buffer (asynchronous; one commit group per stage, possibly empty)
-    auto issue_copy = [&](long long s) {
-        const TileState& T = s_tile[(s / G) & 1];
-        const int b = (int)(s % G) * GB + 4 * lane;
-        float4* box = dyn + (size_t)(s & 1) * BOX_CAP * 32;
-        if (T.staged && b < P.bands) {
-            const int bw = T.bw, nbox = bw * T.bh;
-            // running source pointer: no multiplication, division or shared-memory re-read inside the loop (the
-            // cp.async statements are memory clobbers, so everything the loop needs lives in registers)
-            const long long stride = P.src_pix_stride;
-            const float* rec = P.src + ((long long)T.by0 * P.Ws + T.bx0) * stride + b + wib * stride;
-            const long long step = PWARPS * stride, wrap = P.Ws * stride - bw * stride;
-            const int nb = P.bands;
-            float4* dstp = box + wib * 32 + lane;
-            int col = wib;                              // pixel p = wib, wib + 16, ... walks the box row by row
-            for (int p = wib; p < nbox; p += PWARPS, col += PWARPS, rec += step, dstp += PWARPS * 32) {
-                while (col >= bw) {
-                    col -= bw;
-                    rec += wrap;
-                }
-                if (SRC_VEC) {
-                    cp_async16(dstp, rec);
-                } else {
-                    float* d = reinterpret_cast<float*>(dstp);
-                    cp_async4(d, rec);
-                    if (b + 1 < nb) cp_async4(d + 1, rec + 1);
-                    if (b + 2 < nb) cp_async4(d + 2, rec + 2);
-                    if (b + 3 < nb) cp_async4(d + 3, rec + 3);
-                }
-            }
-        }
-        cp_async_commit();
-    };
-
-    if (nstages > 0) {
-        prepare_tile(0);
-        issue_copy(0);
-    }
-    for (long long s = 0; s < nstages; ++s) {
-        const long long it = s / G;
-        const int g = (int)(s - it * G);
-        if (s + 1 < nstages) {
-            if (g == G - 1) prepare_tile(it + 1);      // the other TileState slot: nobody reads it any more
-            issue_copy(s + 1);
-            cp_async_wait<1>();
-        } else {
-            cp_async_wait<0>();
-        }
-        __syncthreads();
-        const TileState& T = s_tile[it & 1];
-        float4* box = dyn + (size_t)(s & 1) * BOX_CAP * 32;
-        unsigned char* cls = s_cls[s & 1];
-        const int b = g * GB + 4 * lane;
-        const bool act = b < P.bands;
-        const bool staged = T.staged != 0;
-        const int bw = T.bw, nbox = staged ? bw * T.bh : 0;
-        // ---- classify the staged pixels (0 clean, 1 fill, 2 band-specific nodata); pad words take band b's value
-        bool dirty = false;
-        if (act && b + 3 >= P.bands) {                  // the lane holding the last, partial vector of the spectrum
-            for (int p = wib; p < nbox; p += PWARPS) box[p * 32 + lane] = pad_fix(box[p * 32 + lane], b, P.bands);
-        }
-        bool allfill = nbox > 0;
-        {
-            // class 0: no nodata and every value finite (the lean loop may then multiply any of them by a zero weight);
-            // 1: every band is nodata (a fill pixel); 2: anything else
-            const float4* bp = box + wib * 32 + lane;
-            for (int p = wib; p < nbox; p += PWARPS, bp += PWARPS * 32) {
-                const float4 x = *bp;
-                const float z = fmaf(x.x, 0.f, fmaf(x.y, 0.f, fmaf(x.z, 0.f, x.w * 0.f)));      // NaN iff a value is not finite
-                const bool any = act && ((has_nd && (x.x == nd || x.y == nd || x.z == nd || x.w == nd)) || !(z == 0.f));
-                int c = 0;
-                if (__any_sync(FULL, any)) {
-                    const bool all = !act || (x.x == nd && x.y == nd && x.z == nd && x.w == nd);
-                    c = (has_nd && __all_sync(FULL, all)) ? 1 : 2;
-                    dirty = true;
-                }
-                allfill = allfill && c == 1;
-                if (lane == 0) cls[p] = (unsigned char)c;
-            }
-        }
-        const bool box_clean = __syncthreads_or(dirty) == 0;
-        // every staged pixel is fill (the tile lies outside the swath): nothing to resample (uniform: second reduction)
-        const bool box_fill = !box_clean && staged && __syncthreads_and(allfill) != 0;
-        // ---- resample
-        const long long tile = blockIdx.x + it * gridDim.x;
-        const long long ty = tile / tiles_x, tx = tile - ty * tiles_x;
-        for (int q = wib; q < npix_tile; q += PWARPS) {
-            const long long r = ty * TH + (q >> tw_shift), c = tx * TW + (q & (TW - 1));      // TW is a power of two
-            if (r >= P.Hd || c >= P.Wd) continue;
-            const int* M = T.meta[q];
-            float* outp = P.dst + (r * P.Wd + c) * P.dst_pix_stride + b;
-            float4 o = make_float4(dnd, dnd, dnd, dnd);
-            if (M[0]) {
-                const int jlo = M[1], jhi = M[2], klo = M[3], khi = M[4];
-                const float* tw = T.tw[q];
-                float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f, m0 = 0.f, m1 = 0.f, m2 = 0.f, m3 = 0.f, wu = 0.f;
-                if (box_fill) {
-                    // nothing valid under any tap: the weight sum stays 0 -> nodata
-                } else if (staged && box_clean && (M[7] & 2) && (ntx == 4 || ntx == 6 || ntx == 8)) {
-                    // lean loop: clean finite box, whole rows inside the source -> fully unrolled rows, weights by vector
-                    // loads, the weight sum precomputed per pixel (zero-weight columns contribute exactly 0)
-                    const float4* rowb = box + ((M[6] + jlo - T.by0) * bw + (M[5] - T.bx0)) * 32 + lane;
-                    const float* twj = tw + jlo * ntx;
-                    const int rstep = bw * 32;
-                    if (ntx == 6) {
-                        for (int j = jlo; j < jhi; ++j, rowb += rstep, twj += 6) row_fma<6>(rowb, twj, a0, a1, a2, a3);
-                    } else if (ntx == 4) {
-                        for (int j = jlo; j < jhi; ++j, rowb += rstep, twj += 4) row_fma<4>(rowb, twj, a0, a1, a2, a3);
-                    } else {
-                        for (int j = jlo; j < jhi; ++j, rowb += rstep, twj += 8) row_fma<8>(rowb, twj, a0, a1, a2, a3);
-                    }
-                    wu = T.wsum[q];
-                } else if (staged && box_clean && (M[7] & 1)) {
-                    const float4* bp = box + ((M[6] - T.by0) * bw + (M[5] - T.bx0)) * 32 + lane;
-                    for (int j = jlo; j < jhi; ++j) {
-                        const float4* rowb = bp + j * bw * 32;
-                        const float* twj = tw + j * ntx;
-#pragma unroll 2
-                        for (int k = klo; k < khi; ++k) {
-                            const float w = twj[k];
-                            const float4 v = rowb[k * 32];
-                            a0 = fmaf(w, v.x, a0);
-                            a1 = fmaf(w, v.y, a1);
-                            a2 = fmaf(w, v.z, a2);
-                            a3 = fmaf(w, v.w, a3);
-                            wu += w;
-                        }
-                    }
-                } else if (staged) {
-                    const int base = (M[6] - T.by0) * bw + (M[5] - T.bx0);
-                    for (int j = jlo; j < jhi; ++j) {
-                        const int rowi = base + j * bw;
-                        const float* twj = tw + j * ntx;
-#pragma unroll 2
-                        for (int k = klo; k < khi; ++k) {
-                            const int pi = rowi + k;
-                            const int cl = cls[pi];
-                            const float w = twj[k];
-                            const float4 v = box[pi * 32 + lane];
-                            if (cl == 1 || w == 0.f) continue;
-                            if (cl == 0) {
-                                a0 = fmaf(w, v.x, a0);
-                                a1 = fmaf(w, v.y, a1);
-                                a2 = fmaf(w, v.z, a2);
-                                a3 = fmaf(w, v.w, a3);
-                                wu += w;
-                            } else {
-                                const float w0 = v.x == nd ? 0.f : w, w1q = v.y == nd ? 0.f : w;
-                                const float w2 = v.z == nd ? 0.f : w, w3 = v.w == nd ? 0.f : w;
-                                a0 = fmaf(w0, v.x, a0);
-                                a1 = fmaf(w1q, v.y, a1);
-                                a2 = fmaf(w2, v.z, a2);
-                                a3 = fmaf(w3, v.w, a3);
-                                m0 += w0;
-                                m1 += w1q;
-                                m2 += w2;
-                                m3 += w3;
-                            }
-                        }
-                    }
-                } else {    // box too large for the staging buffer: the same taps straight from global memory
-                    for (int j = jlo; j < jhi; ++j) {
-                        const float* rowp = P.src + (((long long)M[6] + j) * P.Ws + M[5]) * P.src_pix_stride;
-                        for (int k = klo; k < khi; ++k) {
-                            const float w = tw[j * ntx + k];
-                            if (w == 0.f) continue;
-                            const float4 v = load_group<SRC_VEC>(rowp + k * P.src_pix_stride, b, P.bands, act);
-                            const bool h = has_nd && act;
-                            const float w0 = (h && v.x == nd) ? 0.f : w, w1q = (h && v.y == nd) ? 0.f : w;
-                            const float w2 = (h && v.z == nd) ? 0.f : w, w3 = (h && v.w == nd) ? 0.f : w;
-                            a0 = fmaf(w0, v.x, a0);
-                            a1 = fmaf(w1q, v.y, a1);
-                            a2 = fmaf(w2, v.z, a2);
-                            a3 = fmaf(w3, v.w, a3);
-                            m0 += w0;
-                            m1 += w1q;
-                            m2 += w2;
-                            m3 += w3;
-                        }
-                    }
-                }
-                const float s0 = wu + m0, s1 = wu + m1, s2 = wu + m2, s3 = wu + m3;
-                o.x = s0 >= 1e-6f ? __fdiv_rn(a0, s0) : dnd;
-                o.y = s1 >= 1e-6f ? __fdiv_rn(a1, s1) : dnd;
-                o.z = s2 >= 1e-6f ? __fdiv_rn(a2, s2) : dnd;
-                o.w = s3 >= 1e-6f ? __fdiv_rn(a3, s3) : dnd;
-            }
-            if (act) {
-                if (DST_VEC) {
-                    __stcs(reinterpret_cast<float4*>(outp), o);
-                } else {
-                    __stcs(outp, o.x);
-                    if (b + 1 < P.bands) __stcs(outp + 1, o.y);
-                    if (b + 2 < P.bands) __stcs(outp + 2, o.z);
-                    if (b + 3 < P.bands) __stcs(outp + 3, o.w);
-                }
-            }
-        }
-        __syncthreads();        // buffer s & 1 and (after the tile's last group) its TileState are free again
-    }
-}
-
 // ---------------------------------------------------------------------------- lane-per-pixel variant
 // Lanes across DESTINATION PIXELS instead of bands.  A CTA owns a 32 x LROWS tile of the destination and walks the
 // spectrum in groups of 32 bands (8 float4 "quads"); a thread owns one pixel of the tile for the whole tile: its window
 // origin, its separable weights (registers, fully unrolled NT x NT window) and its weight sum are computed ONCE and
-// serve every band of the pixel — in the band-per-lane kernels that per-pixel work is redone by a whole warp for every
-// pixel and band group, and it dominated them.  Per group the box of the tile's windows is staged in shared memory
-// TRANSPOSED ([quad][pixel], odd pitch): the coalesced global reads (lanes across the quads of two source pixels) become
-// conflict-free shared-memory writes, and the taps of 32 neighbouring destination pixels — 32 nearly consecutive source
-// pixels of one quad — are conflict-free 16-byte reads.  The box covers the windows UNCLIPPED (pixels outside the source
-// are staged as zeros and carry zero weight), so tap addresses are base + j * bw + k with k an immediate.  Groups whose
-// box holds no nodata and no non-finite value take a lean loop (5 instructions per tap and quad); the others select
-// weights and values per element.  Three CTAs per SM (single buffer each): staging of one overlaps resampling of another.
+// serve every band of the pixel — in the band-per-lane kernels this design replaced, that per-pixel work was redone by
+// a whole warp for every pixel and band group, and it dominated them.  Per group the box of the tile's windows is
+// staged in shared memory TRANSPOSED ([quad][pixel], odd pitch): the coalesced global reads (lanes across the quads of
+// two source pixels) become conflict-free shared-memory writes, and the taps of 32 neighbouring destination pixels — 32
+// nearly consecutive source pixels of one quad — are conflict-free 16-byte reads.  The box covers the windows UNCLIPPED
+// (pixels outside the source are staged as zeros and carry zero weight), so tap addresses are base + j * bw + k with k
+// an immediate.  Groups whose box holds no nodata and no non-finite value take a lean loop (5 instructions per tap and
+// quad); the others select weights and values per element.  Three CTAs per SM (single buffer each): staging of one
+// overlaps resampling of another.
 constexpr int LROWS = 8;            // destination tile: LCOLS x LROWS pixels, one per thread and quad half
 constexpr int LCOLS = 16;
 constexpr int LQ = 8;               // quads (float4) per band group: 32 bands
@@ -1026,7 +410,7 @@ __global__ void __launch_bounds__(256, 3) warp_lane_kernel(const WarpParams P, c
             };
             const float4 fillq = make_float4(dnd, dnd, dnd, dnd);
             // accumulated weights that cancel below 0.03 amplify the fp32 rounding of this kernel beyond the 1e-5 bar: such
-            // (pixel, group) pairs are listed and recomputed in fp64 by warp_fixup_kernel (as for warp_quad_kernel)
+            // (pixel, group) pairs are listed and recomputed in fp64 by warp_exact_kernel (as for warp_quad_kernel)
             bool ill = false;
             if (!inside || allfill) {
                 for (int qq = 0; qq < LQ / 2; ++qq) store_quad((q0 + qhalf * (LQ / 2) + qq) * 4, fillq);
@@ -1115,7 +499,7 @@ __global__ void __launch_bounds__(256, 3) warp_lane_kernel(const WarpParams P, c
                     ill = ill || (mm < 0.03f && (m0 != 0.f || m1 != 0.f || m2 != 0.f || m3 != 0.f));
                 }
             }
-            if (ill && P.redo_list != nullptr && r < P.Hd && c < P.Wd) {
+            if (ill && r < P.Hd && c < P.Wd) {
                 const unsigned int pos = atomicAdd(P.redo_count, 1u);
                 if (pos < P.redo_cap) P.redo_list[pos] = ((unsigned long long)(r * P.Wd + c) << 8) | (unsigned int)g;
             }
@@ -1213,7 +597,7 @@ struct ExactArgs {
 };
 
 // `ill`: some band's accumulated weight is small (|m| < 0.03): its quotient amplifies the last bit of the fp32 weight
-// factors used here by 1 / m — the caller lists the pixel for warp_fixup_kernel, which forms the weights as the oracle does.
+// factors used here by 1 / m — the caller lists the pixel for warp_exact_kernel, which forms the weights as the oracle does.
 __device__ __noinline__ float4 warp_exact_pixel(const ExactArgs A, bool& ill) {
     double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0, m0 = 0.0, m1 = 0.0, m2 = 0.0, m3 = 0.0;
     for (int j = 0; j < A.nrows; ++j) {
@@ -1250,55 +634,66 @@ __device__ __noinline__ float4 warp_exact_pixel(const ExactArgs A, bool& ill) {
     return o;
 }
 
-// Fix-up pass of the fast loops: the (pixel, band group) pairs whose weight sum came out small (taps lost to fill pixels or to
-// the source's border: the quotient of two nearly cancelled fp32 sums is not accurate to 1e-5 below a weight sum of ~0.03)
-// are listed by warp_quad_kernel and recomputed here in fp64 — GDAL accumulates in double — straight from global memory,
-// 8 lanes (quads) per entry.  A ring a fraction of a pixel wide around the swath: a few thousand entries per granule.
-__global__ void __launch_bounds__(256) warp_fixup_kernel(const WarpParams P) {
-    const unsigned int count = *P.redo_count < P.redo_cap ? *P.redo_count : P.redo_cap;
-    const int q = threadIdx.x & 7;
+// The exact pass: one lane per (destination pixel, quad of 4 bands), fp64 accumulation (GDAL accumulates in double) straight
+// from global memory; any radius up to MAX_TAPS / 2, any record alignment, 64-bit indices.  Two modes:
+//   * the fix-up (dense = false): the (pixel, band group) entries the quad and lane kernels listed because their weight sum
+//     came out small (taps lost to fill pixels or to the source's border: the quotient of two nearly cancelled fp32 sums is
+//     not accurate to 1e-5 below a weight sum of ~0.03), 8 lanes per entry.  A ring a fraction of a pixel wide around
+//     the swath: a few thousand entries per granule;
+//   * dense: every (pixel, quad) of the destination — filters wider than the fast kernels hold (radius > 4) and sources of
+//     2^32 pixels or more.
+__global__ void __launch_bounds__(256) warp_exact_kernel(const WarpParams P, const bool dense) {
     const int nvec = (P.bands + 3) >> 2;
+    const long long n = dense ? P.Hd * P.Wd * nvec : (long long)LQ * (*P.redo_count < P.redo_cap ? *P.redo_count : P.redo_cap);
     const bool src_vec = (P.src_pix_stride & 3) == 0 && (reinterpret_cast<uintptr_t>(P.src) & 15) == 0;
-    for (unsigned int e = blockIdx.x * 32u + (threadIdx.x >> 3); e < count; e += gridDim.x * 32u) {
-        const unsigned long long ent = P.redo_list[e];
-        const long long pix = (long long)(ent >> 8);
-        const int g = (int)(ent & 0xffu);
-        const int qi = g * LQ + q;
-        if (qi >= nvec) continue;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        long long pix;
+        int qi;
+        if (dense) {
+            pix = i / nvec;
+            qi = (int)(i - pix * nvec);
+        } else {
+            const unsigned long long ent = P.redo_list[i / LQ];
+            pix = (long long)(ent >> 8);
+            qi = (int)(ent & 0xffu) * LQ + (int)(i % LQ);
+            if (qi >= nvec) continue;
+        }
         const int b = qi * 4;
         const double2 xy = __ldg(reinterpret_cast<const double2*>(P.coords) + pix);
         const double px = xy.x, py = xy.y;
-        const double fxp = floor(px - 0.5), fyp = floor(py - 0.5);
-        const long long x0 = (long long)fxp + 1 - P.rx, y0 = (long long)fyp + 1 - P.ry;
-        const double ddx = px - 0.5 - fxp, ddy = py - 0.5 - fyp;
-        double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0, m0 = 0.0, m1 = 0.0, m2 = 0.0, m3 = 0.0;
-        for (int j = 0; j < 2 * P.ry; ++j) {
-            const long long yy = y0 + j;
-            if (yy < 0 || yy >= P.Hs) continue;
-            const double wy = tap_weight(P.kind, ((double)(j + 1 - P.ry) - ddy) * P.fy);
-            if (wy == 0.0) continue;
-            for (int k = 0; k < 2 * P.rx; ++k) {
-                const long long xx = x0 + k;
-                if (xx < 0 || xx >= P.Ws) continue;
-                // ONE rounding to fp32, of the product of the fp64 factors: the convention of oracle/warp.py.  (Rounding the
-                // factors separately, as the fast loops do, moves a quotient whose weights cancel to 1e-4 by 1e-3.)
-                const double w = (double)(float)(wy * tap_weight(P.kind, ((double)(k + 1 - P.rx) - ddx) * P.fx));
-                if (w == 0.0) continue;
-                const float* rec = P.src + (yy * P.Ws + xx) * P.src_pix_stride;
-                const float4 v = pad_fix(src_vec ? load_group_raw<true>(rec, b, P.bands, true) : load_group_raw<false>(rec, b, P.bands, true),
-                                         b, P.bands);
-                const bool hn = P.has_nodata != 0;
-                if (!(hn && v.x == P.nodata)) { a0 = fma(w, (double)v.x, a0); m0 += w; }
-                if (!(hn && v.y == P.nodata)) { a1 = fma(w, (double)v.y, a1); m1 += w; }
-                if (!(hn && v.z == P.nodata)) { a2 = fma(w, (double)v.z, a2); m2 += w; }
-                if (!(hn && v.w == P.nodata)) { a3 = fma(w, (double)v.w, a3); m3 += w; }
+        float4 o = make_float4(P.dst_nodata, P.dst_nodata, P.dst_nodata, P.dst_nodata);
+        if (px >= 0.0 && px < (double)P.Ws && py >= 0.0 && py < (double)P.Hs) {     // listed entries always are
+            const double fxp = floor(px - 0.5), fyp = floor(py - 0.5);
+            const long long x0 = (long long)fxp + 1 - P.rx, y0 = (long long)fyp + 1 - P.ry;
+            const double ddx = px - 0.5 - fxp, ddy = py - 0.5 - fyp;
+            double a0 = 0.0, a1 = 0.0, a2 = 0.0, a3 = 0.0, m0 = 0.0, m1 = 0.0, m2 = 0.0, m3 = 0.0;
+            for (int j = 0; j < 2 * P.ry; ++j) {
+                const long long yy = y0 + j;
+                if (yy < 0 || yy >= P.Hs) continue;
+                const double wy = tap_weight(P.kind, ((double)(j + 1 - P.ry) - ddy) * P.fy);
+                if (wy == 0.0) continue;
+                for (int k = 0; k < 2 * P.rx; ++k) {
+                    const long long xx = x0 + k;
+                    if (xx < 0 || xx >= P.Ws) continue;
+                    // ONE rounding to fp32, of the product of the fp64 factors: the convention of oracle/warp.py.  (Rounding
+                    // the factors separately, as the fast loops do, moves a quotient whose weights cancel to 1e-4 by 1e-3.)
+                    const double w = (double)(float)(wy * tap_weight(P.kind, ((double)(k + 1 - P.rx) - ddx) * P.fx));
+                    if (w == 0.0) continue;
+                    const float* rec = P.src + (yy * P.Ws + xx) * P.src_pix_stride;
+                    const float4 v = pad_fix(src_vec ? load_group_raw<true>(rec, b, P.bands, true) : load_group_raw<false>(rec, b, P.bands, true),
+                                             b, P.bands);
+                    const bool hn = P.has_nodata != 0;
+                    if (!(hn && v.x == P.nodata)) { a0 = fma(w, (double)v.x, a0); m0 += w; }
+                    if (!(hn && v.y == P.nodata)) { a1 = fma(w, (double)v.y, a1); m1 += w; }
+                    if (!(hn && v.z == P.nodata)) { a2 = fma(w, (double)v.z, a2); m2 += w; }
+                    if (!(hn && v.w == P.nodata)) { a3 = fma(w, (double)v.w, a3); m3 += w; }
+                }
             }
+            if (m0 >= 1e-6) o.x = (float)(a0 / m0);
+            if (m1 >= 1e-6) o.y = (float)(a1 / m1);
+            if (m2 >= 1e-6) o.z = (float)(a2 / m2);
+            if (m3 >= 1e-6) o.w = (float)(a3 / m3);
         }
-        float4 o;
-        o.x = m0 >= 1e-6 ? (float)(a0 / m0) : P.dst_nodata;
-        o.y = m1 >= 1e-6 ? (float)(a1 / m1) : P.dst_nodata;
-        o.z = m2 >= 1e-6 ? (float)(a2 / m2) : P.dst_nodata;
-        o.w = m3 >= 1e-6 ? (float)(a3 / m3) : P.dst_nodata;
         float* op = P.dst + pix * P.dst_pix_stride + b;
         if (((reinterpret_cast<uintptr_t>(op) & 15) == 0) && b + 3 < P.dst_pix_stride) {
             *reinterpret_cast<float4*>(op) = o;
@@ -1617,7 +1012,7 @@ __global__ void __launch_bounds__(256, 2) warp_quad_kernel(const __grid_constant
                     store_px(p, warp_exact_pixel(A, ill));
                     return ill;
                 };
-                auto list_px = [&](int p) {                  // leave (pixel p, this band group) to warp_fixup_kernel
+                auto list_px = [&](int p) {                  // leave (pixel p, this band group) to warp_exact_kernel
                     if (q != 0 || !((exb >> p) & 1u) || P.redo_list == nullptr) return;
                     const unsigned int pos = atomicAdd(P.redo_count, 1u);
                     if (pos < P.redo_cap)
@@ -1756,7 +1151,7 @@ __global__ void __launch_bounds__(256, 2) warp_quad_kernel(const __grid_constant
 // hsr_warp_planes_f32: K <= 16 planar images (the pseudo-S2 planes of the SRF pass) resampled with the taps of
 // hsr_warp_f32, validity per SOURCE PIXEL (src_valid) instead of per band and value.  One thread per destination pixel
 // of a 32 x 8 tile; the K accumulators are fp64 registers (K is a template parameter, every loop over it unrolled), so
-// the quotient is formed as warp_fixup_kernel forms it and there is no fix-up pass.  Tap weights: the fp32 rounding of
+// the quotient is formed as warp_exact_kernel forms it and there is no fix-up pass.  Tap weights: the fp32 rounding of
 // the fp64 product wy * wx (oracle/warp.py); zero weights, taps outside the source and invalid source pixels skipped.
 constexpr int PL_COLS = 32, PL_ROWS = 8;
 
@@ -1917,7 +1312,77 @@ static int encode_src_map(CUtensorMap* map, const float* src, long long Hs, long
     return rc == CUDA_SUCCESS ? HSR_OK : HSR_EINVAL;
 }
 
-// coordinates of every destination pixel (16 B each) + the fix-up list of the fast kernel (count word + entries)
+// warp_quad_kernel, if its two TMA buffers fit an SM next to the instantiation's static shared memory (`launched`;
+// otherwise the caller takes the lane-per-pixel kernel).  TMA box = the tile's windows estimated from the scales (+ 1 of
+// slack per axis for rotation / rounding; a tile that needs more reads its taps from global memory)
+static int launch_warp_quad(const WarpParams& P, const hsr_warp_geo_t* geo, bool& launched, cudaStream_t stream) {
+    launched = false;
+    const double xs = geo->xscale > 0.0 ? geo->xscale : 1.0, ys = geo->yscale > 0.0 ? geo->yscale : 1.0;
+    // source pixels per destination pixel, from the transformer itself at the grid's centre and corners (the
+    // filter scales the caller passes need not describe the geometry)
+    const long long Hd = P.Hd, Wd = P.Wd;
+    double stepx = 1.0 / xs, stepy = 1.0 / ys;
+    {
+        const double cs[3] = {0.5, Wd * 0.5, Wd - 0.5}, rs[3] = {0.5, Hd * 0.5, Hd - 0.5};
+        for (int i = 0; i < 3; ++i)
+            for (int j = 0; j < 3; ++j) {
+                double x0, y0, x1, y1, x2, y2;
+                dst_to_src(P, cs[i], rs[j], x0, y0);
+                dst_to_src(P, cs[i] + 1.0, rs[j], x1, y1);
+                dst_to_src(P, cs[i], rs[j] + 1.0, x2, y2);
+                // a tile's window origins span (QCOLS - 1) column steps and (QROWS - 1) row steps, in x AND in y
+                const double sx = (fabs(x1 - x0) * (QCOLS - 1) + fabs(x2 - x0) * (QROWS - 1)) / (QCOLS - 1);
+                const double sy = (fabs(y2 - y0) * (QROWS - 1) + fabs(y1 - y0) * (QCOLS - 1)) / (QROWS - 1);
+                if (sx == sx && sx > stepx) stepx = sx;
+                if (sy == sy && sy > stepy) stepy = sy;
+            }
+    }
+    QuadGeo G{};
+    // span of the window origins over the tile + the window + 1 of slack for rounding; kept tight: two CTAs of
+    // 2 buffers each must fit an SM's 227 KB
+    G.BW = (int)ceil((QCOLS - 1) * stepx) + 2 * P.rx + 1;
+    G.BH = (int)ceil((QROWS - 1) * stepy) + 2 * P.ry + 1;
+    const size_t qsmem_bytes = (size_t)2 * G.BW * G.BH * 128;
+    CUtensorMap tmap;
+    if (!(G.BW <= 256 && G.BH <= 256 && qsmem_bytes + 8192 <= (size_t)device_max_smem_optin() &&
+          encode_src_map(&tmap, P.src, P.Hs, P.Ws, P.bands, P.src_pix_stride, G.BW, G.BH) == HSR_OK))
+        return HSR_OK;
+    const long long qtiles = ((Wd + QCOLS - 1) / QCOLS) * ((Hd + QROWS - 1) / QROWS);
+    long long qblocks = (long long)device_sm_count() * 2;
+    if (qblocks > qtiles) qblocks = qtiles;
+// (the static shared memory of an instantiation — weight tables, class table — grows with the tap counts: the two
+//  buffers must fit next to it, or the call takes the lane-per-pixel kernel; found by the fuzz soak, <8, 8>)
+#define HSR_LAUNCH_QUAD(NX, NY)                                                                                           \
+    do {                                                                                                                  \
+        static int set__[HSR_MAX_DEVICES];                                                                                \
+        static size_t static__ = 0;                                                                                       \
+        if (static__ == 0) {                                                                                              \
+            cudaFuncAttributes fa__;                                                                                      \
+            HSR_CUDA(cudaFuncGetAttributes(&fa__, warp_quad_kernel<NX, NY, true>));                                       \
+            static__ = fa__.sharedSizeBytes + 1;                                                                          \
+        }                                                                                                                 \
+        if (qsmem_bytes + static__ > (size_t)device_max_smem_optin()) return HSR_OK;                                      \
+        HSR_CUDA(ensure_dynamic_smem(warp_quad_kernel<NX, NY, true>, (int)qsmem_bytes, set__));                           \
+        warp_quad_kernel<NX, NY, true><<<(unsigned int)qblocks, 256, qsmem_bytes, stream>>>(tmap, P, G);                  \
+    } while (0)
+#define HSR_QUAD_Y(NX)                                  \
+    do {                                                \
+        if (P.ry == 1) HSR_LAUNCH_QUAD(NX, 2);          \
+        else if (P.ry == 2) HSR_LAUNCH_QUAD(NX, 4);     \
+        else if (P.ry == 3) HSR_LAUNCH_QUAD(NX, 6);     \
+        else HSR_LAUNCH_QUAD(NX, 8);                    \
+    } while (0)
+    if (P.rx == 1) HSR_QUAD_Y(2);
+    else if (P.rx == 2) HSR_QUAD_Y(4);
+    else if (P.rx == 3) HSR_QUAD_Y(6);
+    else HSR_QUAD_Y(8);
+#undef HSR_QUAD_Y
+#undef HSR_LAUNCH_QUAD
+    launched = true;
+    return HSR_OK;
+}
+
+// coordinates of every destination pixel (16 B each) + the fix-up list of the fast kernels (count word + entries)
 static size_t warp_list_cap(long long Hd, long long Wd) {
     const long long n = Hd * Wd;
     return (size_t)(n < (1LL << 18) ? (n < 1024 ? 1024 : n) : (1LL << 18));
@@ -1955,115 +1420,31 @@ int warp_impl(const float* src, long long Hs, long long Ws, int bands, long long
         HSR_CUDA(cudaGetLastError());
         return HSR_OK;
     }
-    // destination tile: the largest of 8x4, 4x4, 4x2, 2x2, 1x1 whose tap footprint fits the staging buffer
-    // (estimated from the scales plus two pixels of slack for rotation; the kernel checks the real box per tile)
-    const double xs = geo->xscale > 0.0 ? geo->xscale : 1.0, ys = geo->yscale > 0.0 ? geo->yscale : 1.0;
-    const int cand[5][2] = {{8, 4}, {4, 4}, {4, 2}, {2, 2}, {1, 1}};
-    P.tile_w = P.tile_h = 1;
-    for (int i = 0; i < 5; ++i) {
-        const double fw = cand[i][0] / xs + 2 * P.rx + 2, fh = cand[i][1] / ys + 2 * P.ry + 2;
-        if (fw * fh <= BOX_CAP) {
-            P.tile_w = cand[i][0];
-            P.tile_h = cand[i][1];
-            break;
-        }
-    }
-    const long long ntiles = ((Hd + P.tile_h - 1) / P.tile_h) * ((Wd + P.tile_w - 1) / P.tile_w);
-    if (workspace) {    // source coordinates of every destination pixel, once, instead of per tile and band group
-        HSR_REQUIRE(workspace_bytes >= warp_workspace(Hd, Wd), HSR_EINVAL, "workspace too small (%zu < %zu bytes)",
-                    workspace_bytes, warp_workspace(Hd, Wd));
-        HSR_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, HSR_EALIGN, "workspace not 16-byte aligned");
-        P.coords = static_cast<double*>(workspace);
-        unsigned char* tail = static_cast<unsigned char*>(workspace) + (size_t)Hd * (size_t)Wd * 16;
-        P.redo_count = reinterpret_cast<unsigned int*>(tail);
-        P.redo_list = reinterpret_cast<unsigned long long*>(tail + 16);
-        P.redo_cap = (unsigned int)warp_list_cap(Hd, Wd);
-        long long cb = (Hd * Wd + 32 * WARPS - 1) / (32 * WARPS);
-        const long long ccap = (long long)device_sm_count() * 8;
-        warp_coords_kernel<<<(unsigned int)(cb < ccap ? cb : ccap), 32 * WARPS, 0, stream>>>(P);
-        HSR_CUDA(cudaGetLastError());
-    }
-    const int groups = (bands + GB - 1) / GB;
+    HSR_REQUIRE(workspace, HSR_EINVAL, "null workspace: kernels 1 (bilinear) and 2 (cubic) need hsr_warp_workspace_bytes(Hd, Wd)");
+    HSR_REQUIRE(workspace_bytes >= warp_workspace(Hd, Wd), HSR_EINVAL, "workspace too small (%zu < %zu bytes)",
+                workspace_bytes, warp_workspace(Hd, Wd));
+    HSR_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 15) == 0, HSR_EALIGN, "workspace not 16-byte aligned");
+    // source coordinates of every destination pixel, once, instead of per tile and band group
+    P.coords = static_cast<double*>(workspace);
+    unsigned char* tail = static_cast<unsigned char*>(workspace) + (size_t)Hd * (size_t)Wd * 16;
+    P.redo_count = reinterpret_cast<unsigned int*>(tail);
+    P.redo_list = reinterpret_cast<unsigned long long*>(tail + 16);
+    P.redo_cap = (unsigned int)warp_list_cap(Hd, Wd);
+    long long cb = (Hd * Wd + 32 * WARPS - 1) / (32 * WARPS);
+    const long long ccap = (long long)device_sm_count() * 8;
+    warp_coords_kernel<<<(unsigned int)(cb < ccap ? cb : ccap), 32 * WARPS, 0, stream>>>(P);
+    HSR_CUDA(cudaGetLastError());
+    HSR_CUDA(cudaMemsetAsync(P.redo_count, 0, 16, stream));
     const bool src_vec = (src_pix_stride & 3) == 0 && (reinterpret_cast<uintptr_t>(src) & 15) == 0;
     const bool dst_vec = (dst_pix_stride & 3) == 0 && (reinterpret_cast<uintptr_t>(dst) & 15) == 0;
-    const bool fast = P.coords && 4 * P.rx * P.ry <= PTAPS && P.tile_w * P.tile_h <= PTILE && Ws < 2147483647LL &&
-                      Hs < 2147483647LL;
-    if (P.coords && P.rx <= 4 && P.ry <= 4 && Hs * Ws < 4294967295LL && Hs < 2147483000LL && Ws < 2147483000LL) {
-        if (src_vec && dst_vec) {
-            // 2 x 2 block kernel, TMA-staged.  TMA box = the tile's windows estimated from the scales (+ 1 of slack per
-            // axis for rotation / rounding; a tile that needs more reads its taps from global memory)
-            const double xs = geo->xscale > 0.0 ? geo->xscale : 1.0, ys = geo->yscale > 0.0 ? geo->yscale : 1.0;
-            // source pixels per destination pixel, from the transformer itself at the grid's centre and corners (the
-            // filter scales the caller passes need not describe the geometry)
-            double stepx = 1.0 / xs, stepy = 1.0 / ys;
-            {
-                const double cs[3] = {0.5, Wd * 0.5, Wd - 0.5}, rs[3] = {0.5, Hd * 0.5, Hd - 0.5};
-                for (int i = 0; i < 3; ++i)
-                    for (int j = 0; j < 3; ++j) {
-                        double x0, y0, x1, y1, x2, y2;
-                        dst_to_src(P, cs[i], rs[j], x0, y0);
-                        dst_to_src(P, cs[i] + 1.0, rs[j], x1, y1);
-                        dst_to_src(P, cs[i], rs[j] + 1.0, x2, y2);
-                        // a tile's window origins span (QCOLS - 1) column steps and (QROWS - 1) row steps, in x AND in y
-                        const double sx = (fabs(x1 - x0) * (QCOLS - 1) + fabs(x2 - x0) * (QROWS - 1)) / (QCOLS - 1);
-                        const double sy = (fabs(y2 - y0) * (QROWS - 1) + fabs(y1 - y0) * (QCOLS - 1)) / (QROWS - 1);
-                        if (sx == sx && sx > stepx) stepx = sx;
-                        if (sy == sy && sy > stepy) stepy = sy;
-                    }
-            }
-            QuadGeo G{};
-            // span of the window origins over the tile + the window + 1 of slack for rounding; kept tight: two CTAs of
-            // 2 buffers each must fit an SM's 227 KB
-            G.BW = (int)ceil((QCOLS - 1) * stepx) + 2 * P.rx + 1;
-            G.BH = (int)ceil((QROWS - 1) * stepy) + 2 * P.ry + 1;
-            const size_t qsmem_bytes = (size_t)2 * G.BW * G.BH * 128;
-            CUtensorMap tmap;
-            if (G.BW <= 256 && G.BH <= 256 && qsmem_bytes + 8192 <= (size_t)device_max_smem_optin() &&
-                encode_src_map(&tmap, src, Hs, Ws, bands, src_pix_stride, G.BW, G.BH) == HSR_OK) {
-                const long long qtiles = ((Wd + QCOLS - 1) / QCOLS) * ((Hd + QROWS - 1) / QROWS);
-                long long qblocks = (long long)device_sm_count() * 2;
-                if (qblocks > qtiles) qblocks = qtiles;
-// (the static shared memory of an instantiation — weight tables, class table — grows with the tap counts: the two
-//  buffers must fit next to it, or the call takes the lane-per-pixel kernel below; found by the fuzz soak, <8, 8>)
-#define HSR_LAUNCH_QUAD(NX, NY)                                                                                           \
-    do {                                                                                                                  \
-        static int set__[HSR_MAX_DEVICES];                                                                                \
-        static size_t static__ = 0;                                                                                       \
-        if (static__ == 0) {                                                                                              \
-            cudaFuncAttributes fa__;                                                                                      \
-            HSR_CUDA(cudaFuncGetAttributes(&fa__, warp_quad_kernel<NX, NY, true>));                                       \
-            static__ = fa__.sharedSizeBytes + 1;                                                                          \
-        }                                                                                                                 \
-        if (qsmem_bytes + static__ > (size_t)device_max_smem_optin()) {                                                   \
-            quad_ok = false;                                                                                              \
-            break;                                                                                                        \
-        }                                                                                                                 \
-        HSR_CUDA(ensure_dynamic_smem(warp_quad_kernel<NX, NY, true>, (int)qsmem_bytes, set__));                           \
-        warp_quad_kernel<NX, NY, true><<<(unsigned int)qblocks, 256, qsmem_bytes, stream>>>(tmap, P, G);                  \
-    } while (0)
-#define HSR_QUAD_Y(NX)                                  \
-    do {                                                \
-        if (P.ry == 1) HSR_LAUNCH_QUAD(NX, 2);          \
-        else if (P.ry == 2) HSR_LAUNCH_QUAD(NX, 4);     \
-        else if (P.ry == 3) HSR_LAUNCH_QUAD(NX, 6);     \
-        else HSR_LAUNCH_QUAD(NX, 8);                    \
-    } while (0)
-                bool quad_ok = true;
-                HSR_CUDA(cudaMemsetAsync(P.redo_count, 0, 16, stream));
-                if (P.rx == 1) HSR_QUAD_Y(2);
-                else if (P.rx == 2) HSR_QUAD_Y(4);
-                else if (P.rx == 3) HSR_QUAD_Y(6);
-                else HSR_QUAD_Y(8);
-#undef HSR_QUAD_Y
-#undef HSR_LAUNCH_QUAD
-                if (quad_ok) {
-                    HSR_CUDA(cudaGetLastError());
-                    warp_fixup_kernel<<<(unsigned int)device_sm_count(), 256, 0, stream>>>(P);
-                    HSR_CUDA(cudaGetLastError());
-                    return HSR_OK;
-                }
-            }
-        }
+    // the quad and lane kernels hold windows of up to 8 x 8 taps and index the source's pixels in 32 bits
+    const bool narrow = P.rx <= 4 && P.ry <= 4 && Hs * Ws < 4294967295LL;
+    bool quad = false;
+    if (narrow && src_vec && dst_vec) {     // 2 x 2 block kernel, TMA-staged; declines when its buffers do not fit an SM
+        rc = launch_warp_quad(P, geo, quad, stream);
+        if (rc != HSR_OK) return rc;
+    }
+    if (!quad && narrow) {
         // lane-per-pixel kernel: register window of NT x NT taps, NT = 2 * max radius rounded up to 2, 4, 6, 8
         const int rmax = P.rx > P.ry ? P.rx : P.ry;
         const long long ltiles = ((Wd + LCOLS - 1) / LCOLS) * ((Hd + LROWS - 1) / LROWS);
@@ -2081,50 +1462,21 @@ int warp_impl(const float* src, long long Hs, long long Ws, int bands, long long
             warp_lane_kernel<NTV, false><<<(unsigned int)blocks, 256, smem, stream>>>(P, sv);                             \
         }                                                                                                                 \
     } while (0)
-        HSR_CUDA(cudaMemsetAsync(P.redo_count, 0, 16, stream));
         if (rmax <= 1) HSR_LAUNCH_LANE(2);
         else if (rmax == 2) HSR_LAUNCH_LANE(4);
         else if (rmax == 3) HSR_LAUNCH_LANE(6);
         else HSR_LAUNCH_LANE(8);
 #undef HSR_LAUNCH_LANE
-        HSR_CUDA(cudaGetLastError());
-        warp_fixup_kernel<<<(unsigned int)device_sm_count(), 256, 0, stream>>>(P);
-        HSR_CUDA(cudaGetLastError());
-        return HSR_OK;
+    } else if (!quad) {
+        // the exact pass over every (pixel, quad): wider filters, sources of 2^32 pixels or more
+        static int resident[HSR_MAX_DEVICES];
+        long long blocks = (Hd * Wd * ((bands + 3) / 4) + 255) / 256;
+        const long long cap = resident_blocks_cached(warp_exact_kernel, 256, resident);
+        warp_exact_kernel<<<(unsigned int)(blocks < cap ? blocks : cap), 256, 0, stream>>>(P, true);
     }
-    if (fast) {   // radii beyond 4 (NT > 8): the band-per-lane pipeline
-        // pipelined: one persistent CTA per SM, two staging buffers
-        const size_t smem = (size_t)2 * BOX_CAP * 32 * sizeof(float4);
-        long long blocks = device_sm_count();
-        if (blocks > ntiles) blocks = ntiles;
-#define HSR_LAUNCH_PIPE(SV, DV)                                                                                      \
-    do {                                                                                                             \
-        { static int set__[HSR_MAX_DEVICES]; HSR_CUDA(ensure_dynamic_smem(warp_pipe_kernel<SV, DV>, (int)smem, set__)); } \
-        warp_pipe_kernel<SV, DV><<<(unsigned int)blocks, 32 * PWARPS, smem, stream>>>(P);                            \
-    } while (0)
-        if (src_vec && dst_vec) HSR_LAUNCH_PIPE(true, true);
-        else if (src_vec) HSR_LAUNCH_PIPE(true, false);
-        else if (dst_vec) HSR_LAUNCH_PIPE(false, true);
-        else HSR_LAUNCH_PIPE(false, false);
-#undef HSR_LAUNCH_PIPE
-        HSR_CUDA(cudaGetLastError());
-        return HSR_OK;
-    }
-    long long blocks = ntiles;
-    const long long cap = (long long)device_sm_count() * 2 * 4;
-    if (blocks > cap) blocks = cap;
-    const size_t smem = (size_t)BOX_CAP * 32 * sizeof(float4);
-    const dim3 grid((unsigned int)blocks, (unsigned int)groups);
-#define HSR_LAUNCH_WARP(SV, DV)                                                                                      \
-    do {                                                                                                             \
-        { static int set__[HSR_MAX_DEVICES]; HSR_CUDA(ensure_dynamic_smem(warp_tile_kernel<SV, DV>, (int)smem, set__)); } \
-        warp_tile_kernel<SV, DV><<<grid, 32 * WARPS, smem, stream>>>(P);                                             \
-    } while (0)
-    if (src_vec && dst_vec) HSR_LAUNCH_WARP(true, true);
-    else if (src_vec) HSR_LAUNCH_WARP(true, false);
-    else if (dst_vec) HSR_LAUNCH_WARP(false, true);
-    else HSR_LAUNCH_WARP(false, false);
-#undef HSR_LAUNCH_WARP
+    HSR_CUDA(cudaGetLastError());
+    // the fix-up: the entries the quad or lane kernel listed (the list is empty after the exact pass)
+    warp_exact_kernel<<<(unsigned int)device_sm_count(), 256, 0, stream>>>(P, false);
     HSR_CUDA(cudaGetLastError());
     return HSR_OK;
 }

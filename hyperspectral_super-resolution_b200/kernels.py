@@ -1114,8 +1114,7 @@ def padded_bands(bands: int) -> int:
 
 
 def warp(src: torch.Tensor, src_gt, dst_gt, dst_shape, *, utm_zone: int = 0, south: bool = False, scales=None,
-         kernel: str = "cubic", nodata=None, dst_nodata=None, out: Optional[torch.Tensor] = None,
-         workspace: bool = True) -> torch.Tensor:
+         kernel: str = "cubic", nodata=None, dst_nodata=None, out: Optional[torch.Tensor] = None) -> torch.Tensor:
     """Resample the band-interleaved cube ``src`` [Hs, Ws, B] f32 onto the grid ``dst_gt`` / ``dst_shape`` = (Hd, Wd):
     [Hd, Wd, B] f32 (``hsr_warp_f32``; gdalwarp of emit_proj.py:876-940).  ``src`` may be a view of a padded buffer
     (``src.stride(1) >= B``); ``out`` likewise — when it is not given it is allocated with records padded to a
@@ -1139,7 +1138,7 @@ def warp(src: torch.Tensor, src_gt, dst_gt, dst_shape, *, utm_zone: int = 0, sou
             _cuda(out, "out", torch.float32)
             if tuple(out.shape) != (Hd, Wd, B) or out.stride(2) != 1 or out.stride(0) != Wd * out.stride(1):
                 raise ValueError("out must be a [Hd, Wd, B] view with unit band stride and dense rows")
-        wsb = int(_lib.lib().hsr_warp_workspace_bytes(Hd, Wd)) if workspace and code in (1, 2) else 0   # point kernels need none
+        wsb = int(_lib.lib().hsr_warp_workspace_bytes(Hd, Wd)) if code in (1, 2) else 0   # point kernels need none
         ws = torch.empty(wsb // 8, dtype=torch.float64, device=s.device) if wsb else None
         _lib.check(_lib.lib().hsr_warp_f32(s.data_ptr(), Hs, Ws, B, int(s.stride(1)), ctypes.addressof(geo), code,
                                            int(nodata is not None), 0.0 if nodata is None else float(nodata), float(fill),

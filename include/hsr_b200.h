@@ -34,7 +34,7 @@
 extern "C" {
 #endif
 
-#define HSR_ABI_VERSION 6
+#define HSR_ABI_VERSION 7
 
 enum {
     HSR_OK = 0,
@@ -539,8 +539,7 @@ HSR_API int hsr_affine_apply_f32(const float* rgb, const double* W, const uint8_
  * src [Hs, Ws, bands] f32 with src_pix_stride, dst [Hd, Wd, bands] f32 with dst_pix_stride (elements).  Records
  * padded to a multiple of 4 floats on 16-byte aligned bases take the vector path (pad words of dst are undefined).
  * workspace: hsr_warp_workspace_bytes(Hd, Wd) bytes of 16-byte aligned device memory for the source coordinates of
- * the destination pixels (transformed once by a separate launch); NULL = each tile transforms its own pixels (same
- * results, slower: the fp64 transformer is a long dependent chain that one warp per tile cannot hide).
+ * the destination pixels (transformed once by a separate launch); required by kernels 1 and 2 (NULL: HSR_EINVAL).
  */
 typedef struct hsr_warp_geo {
     double src_gt[6];

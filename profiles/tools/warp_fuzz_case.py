@@ -1,4 +1,4 @@
-"""Re-run one geometry of tests/test_gpu_fuzz.py::test_warp_random_geometries and show the worst element.
+"""Re-run one geometry of tests/test_gpu_fuzz.py::test_warp_random_geometries_with_coordinate_workspace and show the worst element.
    python profiles/tools/warp_fuzz_case.py SEED [SEED ...]"""
 import math
 import os
@@ -49,14 +49,13 @@ def case(seed):
     else:
         s = torch.from_numpy(src).cuda()
     out = None if rng.random() < 0.5 else torch.empty((Hd, Wd, bands), dtype=torch.float32, device="cuda")
-    ws = bool(rng.random() < 0.75)
-    got = kernels.warp(s, sgt, dgt, (Hd, Wd), scales=scales, kernel=kernel, nodata=nodata, out=out, workspace=ws).cpu().numpy()
+    got = kernels.warp(s, sgt, dgt, (Hd, Wd), scales=scales, kernel=kernel, nodata=nodata, out=out).cpu().numpy()
     ok = np.isfinite(want)
     err = np.where(ok, np.abs(got.astype(np.float64) - want), 0.0)
     bar = 1e-5 * np.maximum(np.abs(want), 1.0) * 4 + 1e-6
     bad = ok & (err > bar)
     print(f"seed {seed}: bands {bands} src {Hs}x{Ws} dst {Hd}x{Wd} mode {int(mode)} nodata {nodata} kernel {kernel} scales "
-          f"{scales[0]:.3f} {scales[1]:.3f} workspace {ws} records {'padded' if s.stride(1) != bands else 'dense'}: {int(bad.sum())} elements over the bar")
+          f"{scales[0]:.3f} {scales[1]:.3f} records {'padded' if s.stride(1) != bands else 'dense'}: {int(bad.sum())} elements over the bar")
     for r, c, b in list(zip(*np.nonzero(bad)))[:6]:
         sx, sy = owarp.dst_to_src(c, r, dgt, sgt, 0, False, False)
         ix, iy = int(math.floor(sx - 0.5)), int(math.floor(sy - 0.5))

@@ -34,9 +34,9 @@ def test_binding_table_covers_header_one_to_one():
     assert sorted(_lib.SIGNATURES) == _declared_symbols()
 
 
-def test_version_and_workspace_are_callable_without_a_gpu():
+def test_abi_v7_version_and_workspace_are_callable_without_a_gpu():
     lib = _lib.lib()
-    assert lib.hsr_version() == 6
+    assert lib.hsr_version() == 7
     ws = lib.hsr_workspace_bytes(_lib.HSR_OP_POLY_MOMENTS, 1685 * 1667, 12, 2)
     assert ws > 0 and ws % (12 * 8 * 8) == 0
     assert lib.hsr_workspace_bytes(99, 10, 1, 2) == 0

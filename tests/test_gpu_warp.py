@@ -3,6 +3,8 @@ step of nc_to_envi, EMIT_data/emit_proj.py:876-940) against oracle/warp.py on sm
 size-independent properties at granule size.  Bars: source coordinates 1e-8 px (fp64 on both sides); resampled
 values 1e-5 relative + 1e-6 absolute (fp32 accumulation of <= 64 fp32-weighted taps against the oracle's fp64);
 nodata / NaN patterns identical.  Parity with GDAL / PROJ themselves is unpinned (oracle/warp.py header)."""
+import ctypes
+
 import numpy as np
 import pytest
 import torch
@@ -66,7 +68,7 @@ def test_coords_match_oracle_transformer():
 
 
 @pytest.mark.parametrize("bands,padded", [(285, True), (285, False), (37, False), (3, False), (8, True)])
-def test_utm_cubic_warp_vs_oracle(bands, padded):
+def test_utm_cubic_warp_vs_oracle_with_coordinate_workspace(bands, padded):
     """The nc_to_envi geometry (lon / lat -> UTM 60 m, x-scale ~0.83 so the cubic filter is widened to 6 taps), with
     GLT-style fill pixels (every band nodata), band-specific nodata, NaN and Inf samples; vector and scalar paths."""
     rng = np.random.default_rng(bands)
@@ -92,8 +94,7 @@ def test_utm_cubic_warp_vs_oracle(bands, padded):
     got = kernels.warp(s, src_gt, dst_gt, (Hd, Wd), utm_zone=11, scales=scales, nodata=ND)
     if not padded:                                                 # force the scalar path on the output side too
         out = torch.empty((Hd, Wd, bands), dtype=torch.float32, device="cuda")
-        got = kernels.warp(s, src_gt, dst_gt, (Hd, Wd), utm_zone=11, scales=scales, nodata=ND, out=out,
-                           workspace=False)                        # ... and let the tiles transform their own pixels
+        got = kernels.warp(s, src_gt, dst_gt, (Hd, Wd), utm_zone=11, scales=scales, nodata=ND, out=out)
     assert_warp_close(got, want)
     assert (want == ND).any() and (want != ND).any() and np.isnan(want).any()
 
@@ -115,6 +116,18 @@ def test_same_crs_bilinear_and_downsampling_vs_oracle():
         got = hwarp.warp_to_grid(src, sgt, dgt, shape, kernel=kernel, nodata=ND, scales=scales)       # numpy in -> numpy out
         assert isinstance(got, np.ndarray)
         assert_warp_close(got, want)
+    # filters wider than the quad and lane kernels hold (the exact pass): x scale 0.4 (cubic, radii 5 x 2) and a 6x
+    # bilinear reduction (radius 6), on padded records (vector path) and on dense ones with a dense output (scalar path)
+    sub = src[..., :11]
+    for kernel, dgt, shape in (("cubic", (500003.0, 25.0, 0.0, 3999998.0, 0.0, -10.0), (28, 13)),
+                               ("bilinear", (500007.0, 60.0, 0.0, 3999996.0, 0.0, -60.0), (5, 6))):
+        scales = hwarp.warp_scales(dgt, sgt, shape)
+        want = owarp.warp(sub, sgt, dgt, shape[0], shape[1], utm=False, nodata=ND, kernel=kernel, scales=scales)
+        buf = torch.full((30, 34, kernels.padded_bands(11)), 7.0, dtype=torch.float32, device="cuda")
+        buf[..., :11] = dev(sub)
+        dense_out = torch.empty((shape[0], shape[1], 11), dtype=torch.float32, device="cuda")
+        for s, out in ((buf[..., :11], None), (dev(sub), dense_out)):
+            assert_warp_close(kernels.warp(s, sgt, dgt, shape, scales=scales, kernel=kernel, nodata=ND, out=out), want)
     # no nodata value given: every tap counts, the destination outside the source is 0
     want = owarp.warp(src, sgt, (499900.0, 10.0, 0.0, 4000000.0, 0.0, -10.0), 8, 20, utm=False, nodata=None)
     got = hwarp.warp_to_grid(src, sgt, (499900.0, 10.0, 0.0, 4000000.0, 0.0, -10.0), (8, 20), nodata=None)
@@ -178,6 +191,12 @@ def test_warp_to_s2_grid_plane_and_errors():
         kernels.warp(torch.zeros(4, 4, 3, device="cuda"), src_gt, dst_gt, (2, 2), scales=(0.1, 1.0))
     with pytest.raises(_lib.HsrError):                                                   # singular geotransform
         kernels.warp(torch.zeros(4, 4, 3, device="cuda"), (0, 0, 0, 0, 0, 0), dst_gt, (2, 2))
+    s, d = torch.zeros(4, 4, 3, device="cuda"), torch.empty(2, 2, 3, device="cuda")
+    geo = kernels._warp_geo(src_gt, dst_gt, 11, False, None)
+    with pytest.raises(_lib.HsrError, match="workspace") as err:                          # cubic needs the coordinate workspace
+        _lib.check(_lib.lib().hsr_warp_f32(s.data_ptr(), 4, 4, 3, 3, ctypes.addressof(geo), 2, 1, ND, ND, 2, 2,
+                                           d.data_ptr(), 3, None, 0, None))
+    assert err.value.code == -1                                                          # HSR_EINVAL
 
 
 def test_full_granule_warp_properties():
