@@ -274,11 +274,16 @@ class S2Target:
     kernel: str = "cubic"
     _coords: dict = field(default_factory=dict, repr=False, compare=False)
 
-    def coords(self, device=None) -> torch.Tensor:
-        """[Hd, Wd, 2] f64 source pixel coordinates of the target's pixel centres on ``device`` (cached)."""
+    def coords(self, device=None, rows=None) -> torch.Tensor:
+        """[Hd, Wd, 2] f64 source pixel coordinates of the target's pixel centres on ``device`` (cached).  ``rows`` =
+        (r0, r1): only target rows [r0, r1), bit-identical to those rows of the whole grid and not cached (a rank of a
+        mosaic transforms its own band; the whole target would be 16 bytes per pixel on every rank)."""
         dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
         if dev.type == "cuda" and dev.index is None:
             dev = torch.device("cuda", torch.cuda.current_device())
+        if rows is not None:
+            return kernels.warp_coords(self.src_gt, self.dst_gt, self.shape, utm_zone=self.zone, south=self.south,
+                                       device=dev, rows=rows)
         c = self._coords.get(dev)
         if c is None:
             c = kernels.warp_coords(self.src_gt, self.dst_gt, self.shape, utm_zone=self.zone, south=self.south,

@@ -102,6 +102,10 @@ SIGNATURES = {
     "hsr_warp_coords_f64": (_int, [_p, _i64, _i64, _p, _p]),
     "hsr_warp_planes_f32": (_int, [_p, _i64, _i64, _int, _i64, _p, _p, _p, _int, _p, _int, _f32, _i64, _i64, _p, _i64,
                                    _p, _p, _p]),
+    "hsr_warp_coords_rows_f64": (_int, [_p, _i64, _i64, _i64, _p, _p]),
+    "hsr_warp_src_row_range": (_int, [_p, _i64, _i64, _i64, _i64, _p, _int, _p, _p]),
+    "hsr_warp_planes_window_f32": (_int, [_p, _i64, _i64, _int, _i64, _p, _i64, _i64, _p, _p, _int, _p, _int, _f32,
+                                          _i64, _i64, _p, _i64, _p, _p, _p, _p]),
     "hsr_peer_block_bytes": (_c.c_size_t, []),
     "hsr_peer_alloc": (_int, [_p]),
     "hsr_peer_free": (_int, [_p]),

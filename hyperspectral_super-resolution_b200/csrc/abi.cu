@@ -84,9 +84,15 @@ int warp_impl(const float*, long long, long long, int, long long, const hsr_warp
               long long, long long, float*, long long, void*, size_t, cudaStream_t);
 size_t warp_workspace(long long, long long);
 int warp_coords_impl(const hsr_warp_geo_t*, long long, long long, double*, cudaStream_t);
+int warp_coords_rows_impl(const hsr_warp_geo_t*, long long, long long, long long, double*, cudaStream_t);
+int warp_src_row_range_impl(const double*, long long, long long, long long, long long, const hsr_warp_geo_t*, int,
+                            unsigned long long*, cudaStream_t);
 int warp_planes_impl(const float*, long long, long long, int, long long, const uint8_t*, const double*,
                      const hsr_warp_geo_t*, int, const float*, int, float, long long, long long, float*, long long,
                      uint8_t*, uint8_t*, cudaStream_t);
+int warp_planes_window_impl(const float*, long long, long long, int, long long, const uint8_t*, long long, long long,
+                            const double*, const hsr_warp_geo_t*, int, const float*, int, float, long long, long long,
+                            float*, long long, uint8_t*, uint8_t*, unsigned long long*, cudaStream_t);
 int affine_fit_impl(const double*, const double*, long long, int, double*, cudaStream_t);
 int affine_apply_impl(const float*, const double*, const uint8_t*, long long, int, float, float, float*, cudaStream_t);
 int stretch64_impl(const float*, long long, long long, const double*, const uint8_t*, long long, int, int, double*,
@@ -352,6 +358,26 @@ int hsr_warp_planes_f32(const float* src, int64_t Hs, int64_t Ws, int K, int64_t
                         int64_t dst_plane_stride, uint8_t* dst_valid, uint8_t* fit_mask, void* stream) {
     return hsr::warp_planes_impl(src, Hs, Ws, K, src_plane_stride, src_valid, coords, geo, kernel, fill_out, gate_k,
                                  gate_gt, Hd, Wd, dst, dst_plane_stride, dst_valid, fit_mask, (cudaStream_t)stream);
+}
+
+int hsr_warp_coords_rows_f64(const hsr_warp_geo_t* geo, int64_t row0, int64_t rows, int64_t Wd, double* coords,
+                             void* stream) {
+    return hsr::warp_coords_rows_impl(geo, row0, rows, Wd, coords, (cudaStream_t)stream);
+}
+
+int hsr_warp_src_row_range(const double* coords, int64_t rows, int64_t Wd, int64_t Hs, int64_t Ws,
+                           const hsr_warp_geo_t* geo, int kernel, unsigned long long* range, void* stream) {
+    return hsr::warp_src_row_range_impl(coords, rows, Wd, Hs, Ws, geo, kernel, range, (cudaStream_t)stream);
+}
+
+int hsr_warp_planes_window_f32(const float* src, int64_t Hs, int64_t Ws, int K, int64_t src_plane_stride,
+                               const uint8_t* src_valid, int64_t src_row0, int64_t src_rows, const double* coords,
+                               const hsr_warp_geo_t* geo, int kernel, const float* fill_out, int gate_k, float gate_gt,
+                               int64_t Hd, int64_t Wd, float* dst, int64_t dst_plane_stride, uint8_t* dst_valid,
+                               uint8_t* fit_mask, unsigned long long* outside, void* stream) {
+    return hsr::warp_planes_window_impl(src, Hs, Ws, K, src_plane_stride, src_valid, src_row0, src_rows, coords, geo,
+                                        kernel, fill_out, gate_k, gate_gt, Hd, Wd, dst, dst_plane_stride, dst_valid,
+                                        fit_mask, outside, (cudaStream_t)stream);
 }
 
 int hsr_affine_fit_f64(const double* X, const double* Ybar, int64_t ns, int C, double* W, void* stream) {

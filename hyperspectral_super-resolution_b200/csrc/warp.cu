@@ -101,12 +101,14 @@ __device__ __forceinline__ double tap_weight(int kind, double x) {
     return w;
 }
 
-__global__ void __launch_bounds__(32 * WARPS) warp_coords_kernel(const WarpParams P) {
+// P.Hd rows of coordinates starting at destination row row0: the transform sees the absolute row, so a band of rows
+// is bit-identical to those rows of the whole grid
+__global__ void __launch_bounds__(32 * WARPS) warp_coords_kernel(const WarpParams P, long long row0) {
     const long long n = P.Hd * P.Wd;
     for (long long o = blockIdx.x * (long long)blockDim.x + threadIdx.x; o < n; o += (long long)gridDim.x * blockDim.x) {
         const long long r = o / P.Wd, c = o - r * P.Wd;
         double px, py;
-        dst_to_src(P, (double)c + 0.5, (double)r + 0.5, px, py);
+        dst_to_src(P, (double)c + 0.5, (double)(r + row0) + 0.5, px, py);
         P.coords[2 * o] = px;
         P.coords[2 * o + 1] = py;
     }
@@ -1153,12 +1155,18 @@ __global__ void __launch_bounds__(256, 2) warp_quad_kernel(const __grid_constant
 // of a 32 x 8 tile; the K accumulators are fp64 registers (K is a template parameter, every loop over it unrolled), so
 // the quotient is formed as warp_exact_kernel forms it and there is no fix-up pass.  Tap weights: the fp32 rounding of
 // the fp64 product wy * wx (oracle/warp.py); zero weights, taps outside the source and invalid source pixels skipped.
+// The source may be a window of rows [src_row0, src_row0 + src_rows) of the logical Hs x Ws source (a row slab of the
+// target reads only the rows its filter reaches): every test and weight still uses the logical Hs, so the window only
+// decides where a tap's row is read from.  A non-zero-weight tap in a row outside the window is skipped and its
+// destination pixel counted in *outside (the caller sized the window wrongly).
 constexpr int PL_COLS = 32, PL_ROWS = 8;
 
 struct PlaneParams {
-    const float* src;
+    const float* src;               // window rows [src_row0, src_row0 + src_rows), row stride Ws
     const uint8_t* src_valid;
     long long Hs, Ws, src_plane_stride;
+    long long src_row0, src_rows;
+    unsigned long long* outside;    // nullable
     const double* coords;
     long long Hd, Wd;
     int kind, rx, ry;
@@ -1187,6 +1195,7 @@ __global__ void __launch_bounds__(PL_COLS * PL_ROWS) warp_planes_kernel(const Pl
 #pragma unroll
         for (int k = 0; k < K; ++k) acc[k] = 0.0;
         double ws = 0.0;
+        bool missed = false;
         const bool inside = px >= 0.0 && px < (double)P.Ws && py >= 0.0 && py < (double)P.Hs;
         if (inside) {
             const double fxp = floor(px - 0.5), fyp = floor(py - 0.5);
@@ -1197,11 +1206,24 @@ __global__ void __launch_bounds__(PL_COLS * PL_ROWS) warp_planes_kernel(const Pl
                 if (yy < 0 || yy >= P.Hs) continue;
                 const double wy = tap_weight(P.kind, ((double)(j + 1 - P.ry) - ddy) * P.fy);
                 if (wy == 0.0) continue;
+                const long long wr = yy - P.src_row0;
+                // a row the window does not hold (wr < 0 wraps): any tap of weight != 0 in it is a miss
+                if ((unsigned long long)wr >= (unsigned long long)P.src_rows) {
+                    for (int i = 0; i < 2 * P.rx; ++i) {
+                        const long long xx = x0 + i;
+                        if (xx >= 0 && xx < P.Ws &&
+                            (float)(wy * tap_weight(P.kind, ((double)(i + 1 - P.rx) - ddx) * P.fx)) != 0.0f) {
+                            missed = true;
+                            break;
+                        }
+                    }
+                    continue;
+                }
                 for (int i = 0; i < 2 * P.rx; ++i) {
                     const long long xx = x0 + i;
                     if (xx < 0 || xx >= P.Ws) continue;
                     const double w = (double)(float)(wy * tap_weight(P.kind, ((double)(i + 1 - P.rx) - ddx) * P.fx));
-                    const long long s = yy * P.Ws + xx;
+                    const long long s = wr * P.Ws + xx;
                     if (w == 0.0 || !__ldg(P.src_valid + s)) continue;
                     ws += w;
                     const float* sp = P.src + s;
@@ -1221,6 +1243,33 @@ __global__ void __launch_bounds__(PL_COLS * PL_ROWS) warp_planes_kernel(const Pl
         }
         if (P.dst_valid) P.dst_valid[o] = covered ? 1 : 0;
         if (P.fit_mask) P.fit_mask[o] = fit ? 1 : 0;
+        if (missed && P.outside) atomicAdd(P.outside, 1ull);
+    }
+}
+
+// Source rows a band of destination coordinates reads through the filter: over the pixels whose centre is inside the
+// Hs x Ws source, range[0] = min(floor(py - 0.5) + 1 - ry) and range[1] = max(floor(py - 0.5) + 1 + ry), both clipped
+// to [0, Hs) — the rows warp_planes_kernel's tap loop visits (zero weights included, so it is never too small).
+__global__ void __launch_bounds__(256) warp_src_row_range_kernel(const double* __restrict__ coords, long long n,
+                                                                 long long Hs, long long Ws, int ry,
+                                                                 unsigned long long* __restrict__ range) {
+    unsigned long long lo = ~0ull, hi = 0ull;
+    for (long long o = blockIdx.x * (long long)blockDim.x + threadIdx.x; o < n; o += (long long)gridDim.x * blockDim.x) {
+        const double2 xy = __ldg(reinterpret_cast<const double2*>(coords) + o);
+        if (!(xy.x >= 0.0 && xy.x < (double)Ws && xy.y >= 0.0 && xy.y < (double)Hs)) continue;
+        const long long y0 = (long long)floor(xy.y - 0.5) + 1 - ry;
+        const long long a = y0 < 0 ? 0 : y0, b = y0 + 2 * ry > Hs ? Hs : y0 + 2 * ry;
+        lo = (unsigned long long)a < lo ? (unsigned long long)a : lo;
+        hi = (unsigned long long)b > hi ? (unsigned long long)b : hi;
+    }
+    for (int d = 16; d > 0; d >>= 1) {
+        const unsigned long long l2 = __shfl_xor_sync(0xffffffffu, lo, d), h2 = __shfl_xor_sync(0xffffffffu, hi, d);
+        lo = l2 < lo ? l2 : lo;
+        hi = h2 > hi ? h2 : hi;
+    }
+    if ((threadIdx.x & 31) == 0 && hi != 0ull) {
+        atomicMin(range + 0, lo);
+        atomicMax(range + 1, hi);
     }
 }
 
@@ -1432,7 +1481,7 @@ int warp_impl(const float* src, long long Hs, long long Ws, int bands, long long
     P.redo_cap = (unsigned int)warp_list_cap(Hd, Wd);
     long long cb = (Hd * Wd + 32 * WARPS - 1) / (32 * WARPS);
     const long long ccap = (long long)device_sm_count() * 8;
-    warp_coords_kernel<<<(unsigned int)(cb < ccap ? cb : ccap), 32 * WARPS, 0, stream>>>(P);
+    warp_coords_kernel<<<(unsigned int)(cb < ccap ? cb : ccap), 32 * WARPS, 0, stream>>>(P, 0);
     HSR_CUDA(cudaGetLastError());
     HSR_CUDA(cudaMemsetAsync(P.redo_count, 0, 16, stream));
     const bool src_vec = (src_pix_stride & 3) == 0 && (reinterpret_cast<uintptr_t>(src) & 15) == 0;
@@ -1481,54 +1530,90 @@ int warp_impl(const float* src, long long Hs, long long Ws, int bands, long long
     return HSR_OK;
 }
 
-int warp_coords_impl(const hsr_warp_geo_t* geo, long long Hd, long long Wd, double* coords, cudaStream_t stream) {
+int warp_coords_rows_impl(const hsr_warp_geo_t* geo, long long row0, long long rows, long long Wd, double* coords,
+                          cudaStream_t stream) {
     HSR_REQUIRE(coords, HSR_EINVAL, "null coords pointer");
-    HSR_REQUIRE(Hd >= 0 && Wd >= 0, HSR_EINVAL, "bad shape");
+    HSR_REQUIRE(row0 >= 0 && rows >= 0 && Wd >= 0, HSR_EINVAL, "bad shape");
     WarpParams P{};
-    int rc = fill_params(P, geo, 1, 1, Hd, Wd, 2);
+    int rc = fill_params(P, geo, 1, 1, rows, Wd, 2);
     if (rc != HSR_OK) return rc;
-    if (Hd == 0 || Wd == 0) return HSR_OK;
+    if (rows == 0 || Wd == 0) return HSR_OK;
     P.coords = coords;
-    long long blocks = (Hd * Wd + 32 * WARPS - 1) / (32 * WARPS);
+    long long blocks = (rows * Wd + 32 * WARPS - 1) / (32 * WARPS);
     const long long cap = (long long)device_sm_count() * 8;
     if (blocks > cap) blocks = cap;
-    warp_coords_kernel<<<(unsigned int)blocks, 32 * WARPS, 0, stream>>>(P);
+    warp_coords_kernel<<<(unsigned int)blocks, 32 * WARPS, 0, stream>>>(P, row0);
     HSR_CUDA(cudaGetLastError());
     return HSR_OK;
 }
 
-int warp_planes_impl(const float* src, long long Hs, long long Ws, int K, long long src_plane_stride,
-                     const uint8_t* src_valid, const double* coords, const hsr_warp_geo_t* geo, int kernel,
-                     const float* fill_out, int gate_k, float gate_gt, long long Hd, long long Wd, float* dst,
-                     long long dst_plane_stride, uint8_t* dst_valid, uint8_t* fit_mask, cudaStream_t stream) {
-    HSR_REQUIRE(src && dst && src_valid && fill_out, HSR_EINVAL, "null src / dst / src_valid / fill_out pointer");
-    HSR_REQUIRE(coords, HSR_EINVAL, "null coords pointer: pass hsr_warp_coords_f64's output");
+int warp_coords_impl(const hsr_warp_geo_t* geo, long long Hd, long long Wd, double* coords, cudaStream_t stream) {
+    return warp_coords_rows_impl(geo, 0, Hd, Wd, coords, stream);
+}
+
+// filter of the plane warp: kernel 1 / 2, radius ceil(r / scale) per axis below scale 1 (the rule of fill_params)
+static int plane_filter(const hsr_warp_geo_t* geo, int kernel, PlaneParams& P) {
     HSR_REQUIRE(geo, HSR_EINVAL, "null geo pointer");
-    HSR_REQUIRE(K >= 1 && K <= HSR_MAX_SRF_BANDS, HSR_EINVAL, "K = %d outside [1, %d]", K, HSR_MAX_SRF_BANDS);
     HSR_REQUIRE(kernel == 1 || kernel == 2, HSR_EINVAL, "kernel must be 1 (bilinear) or 2 (cubic), got %d", kernel);
-    HSR_REQUIRE(Hs > 0 && Ws > 0 && Hd >= 0 && Wd >= 0, HSR_EINVAL, "bad shape");
-    HSR_REQUIRE(Hs * Ws < (1LL << 40) && Hd * Wd < (1LL << 40), HSR_EINVAL, "grid too large (limit 2^40 pixels)");
-    HSR_REQUIRE((K == 1 || src_plane_stride >= Hs * Ws) && (K == 1 || dst_plane_stride >= Hd * Wd) &&
-                    src_plane_stride >= 0 && dst_plane_stride >= 0,
-                HSR_EINVAL, "plane stride below the plane size");
-    HSR_REQUIRE((reinterpret_cast<uintptr_t>(coords) & 15) == 0, HSR_EALIGN, "coords not 16-byte aligned");
-    HSR_REQUIRE(gate_k < K, HSR_EINVAL, "gate_k = %d >= K = %d", gate_k, K);
-    PlaneParams P{};
     const int r0 = kernel == 2 ? 2 : 1;
     const double xs = geo->xscale > 0.0 ? geo->xscale : 1.0, ys = geo->yscale > 0.0 ? geo->yscale : 1.0;
     const double rxd = xs < 1.0 ? ceil(r0 / xs) : (double)r0, ryd = ys < 1.0 ? ceil(r0 / ys) : (double)r0;
     HSR_REQUIRE(rxd <= MAX_TAPS / 2 && ryd <= MAX_TAPS / 2, HSR_EINVAL,
                 "scale (%g, %g) needs a filter radius beyond %d taps", xs, ys, MAX_TAPS / 2);
-    if (Hd == 0 || Wd == 0) return HSR_OK;
-    P.src = src;
-    P.src_valid = src_valid;
-    P.Hs = Hs, P.Ws = Ws, P.src_plane_stride = src_plane_stride;
-    P.coords = coords;
-    P.Hd = Hd, P.Wd = Wd;
     P.kind = kernel;
     P.rx = (int)rxd, P.ry = (int)ryd;
     P.fx = xs < 1.0 ? xs : 1.0;
     P.fy = ys < 1.0 ? ys : 1.0;
+    return HSR_OK;
+}
+
+int warp_src_row_range_impl(const double* coords, long long rows, long long Wd, long long Hs, long long Ws,
+                            const hsr_warp_geo_t* geo, int kernel, unsigned long long* range, cudaStream_t stream) {
+    HSR_REQUIRE(coords && range, HSR_EINVAL, "null coords / range pointer");
+    HSR_REQUIRE(rows >= 0 && Wd >= 0 && Hs > 0 && Ws > 0, HSR_EINVAL, "bad shape");
+    HSR_REQUIRE((reinterpret_cast<uintptr_t>(coords) & 15) == 0, HSR_EALIGN, "coords not 16-byte aligned");
+    PlaneParams P{};
+    const int rc = plane_filter(geo, kernel, P);
+    if (rc != HSR_OK) return rc;
+    const long long n = rows * Wd;
+    if (n == 0) return HSR_OK;
+    long long blocks = (n + 1023) / 1024;
+    const long long cap = (long long)device_sm_count() * 8;
+    if (blocks > cap) blocks = cap;
+    warp_src_row_range_kernel<<<(unsigned int)blocks, 256, 0, stream>>>(coords, n, Hs, Ws, P.ry, range);
+    HSR_CUDA(cudaGetLastError());
+    return HSR_OK;
+}
+
+int warp_planes_window_impl(const float* src, long long Hs, long long Ws, int K, long long src_plane_stride,
+                            const uint8_t* src_valid, long long src_row0, long long src_rows, const double* coords,
+                            const hsr_warp_geo_t* geo, int kernel, const float* fill_out, int gate_k, float gate_gt,
+                            long long Hd, long long Wd, float* dst, long long dst_plane_stride, uint8_t* dst_valid,
+                            uint8_t* fit_mask, unsigned long long* outside, cudaStream_t stream) {
+    HSR_REQUIRE(dst && fill_out, HSR_EINVAL, "null dst / fill_out pointer");
+    HSR_REQUIRE(src_rows == 0 || (src && src_valid), HSR_EINVAL, "null src / src_valid pointer");
+    HSR_REQUIRE(coords, HSR_EINVAL, "null coords pointer: pass hsr_warp_coords_f64's output");
+    HSR_REQUIRE(K >= 1 && K <= HSR_MAX_SRF_BANDS, HSR_EINVAL, "K = %d outside [1, %d]", K, HSR_MAX_SRF_BANDS);
+    HSR_REQUIRE(Hs > 0 && Ws > 0 && Hd >= 0 && Wd >= 0, HSR_EINVAL, "bad shape");
+    HSR_REQUIRE(src_row0 >= 0 && src_rows >= 0 && src_row0 + src_rows <= Hs, HSR_EINVAL,
+                "source window [%lld, %lld) outside the source's %lld rows", src_row0, src_row0 + src_rows, Hs);
+    HSR_REQUIRE(Hs * Ws < (1LL << 40) && Hd * Wd < (1LL << 40), HSR_EINVAL, "grid too large (limit 2^40 pixels)");
+    HSR_REQUIRE((K == 1 || src_plane_stride >= src_rows * Ws) && (K == 1 || dst_plane_stride >= Hd * Wd) &&
+                    src_plane_stride >= 0 && dst_plane_stride >= 0,
+                HSR_EINVAL, "plane stride below the plane size");
+    HSR_REQUIRE((reinterpret_cast<uintptr_t>(coords) & 15) == 0, HSR_EALIGN, "coords not 16-byte aligned");
+    HSR_REQUIRE(gate_k < K, HSR_EINVAL, "gate_k = %d >= K = %d", gate_k, K);
+    PlaneParams P{};
+    const int rc = plane_filter(geo, kernel, P);
+    if (rc != HSR_OK) return rc;
+    if (Hd == 0 || Wd == 0) return HSR_OK;
+    P.src = src;
+    P.src_valid = src_valid;
+    P.Hs = Hs, P.Ws = Ws, P.src_plane_stride = src_plane_stride;
+    P.src_row0 = src_row0, P.src_rows = src_rows;
+    P.outside = outside;
+    P.coords = coords;
+    P.Hd = Hd, P.Wd = Wd;
     P.fill_out = fill_out;
     P.gate_k = gate_k;
     P.gate_gt = gate_gt;
@@ -1548,6 +1633,14 @@ int warp_planes_impl(const float* src, long long Hs, long long Ws, int K, long l
     launch[K - 1](grid, stream, P);
     HSR_CUDA(cudaGetLastError());
     return HSR_OK;
+}
+
+int warp_planes_impl(const float* src, long long Hs, long long Ws, int K, long long src_plane_stride,
+                     const uint8_t* src_valid, const double* coords, const hsr_warp_geo_t* geo, int kernel,
+                     const float* fill_out, int gate_k, float gate_gt, long long Hd, long long Wd, float* dst,
+                     long long dst_plane_stride, uint8_t* dst_valid, uint8_t* fit_mask, cudaStream_t stream) {
+    return warp_planes_window_impl(src, Hs, Ws, K, src_plane_stride, src_valid, 0, Hs, coords, geo, kernel, fill_out,
+                                   gate_k, gate_gt, Hd, Wd, dst, dst_plane_stride, dst_valid, fit_mask, nullptr, stream);
 }
 
 }  // namespace hsr

@@ -1147,50 +1147,104 @@ def warp(src: torch.Tensor, src_gt, dst_gt, dst_shape, *, utm_zone: int = 0, sou
     return out
 
 
-def warp_coords(src_gt, dst_gt, dst_shape, *, utm_zone: int = 0, south: bool = False, device=None) -> torch.Tensor:
-    """[Hd, Wd, 2] f64: source pixel coordinates (x, y) of every destination pixel centre (``hsr_warp_coords_f64``)."""
+def warp_coords(src_gt, dst_gt, dst_shape, *, utm_zone: int = 0, south: bool = False, device=None,
+                rows=None) -> torch.Tensor:
+    """[Hd, Wd, 2] f64: source pixel coordinates (x, y) of every destination pixel centre (``hsr_warp_coords_f64``).
+    ``rows`` = (r0, r1): only destination rows [r0, r1), [r1 - r0, Wd, 2], bit-identical to those rows of the whole
+    grid (``hsr_warp_coords_rows_f64``)."""
     Hd, Wd = int(dst_shape[0]), int(dst_shape[1])
     dev = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device())
     geo = _warp_geo(src_gt, dst_gt, utm_zone, south, None)
+    if rows is not None:
+        r0, r1 = int(rows[0]), int(rows[1])
+        if not 0 <= r0 <= r1 <= Hd:
+            raise ValueError(f"rows must satisfy 0 <= r0 <= r1 <= {Hd}, got {tuple(rows)}")
     with torch.cuda.device(dev):
-        out = torch.empty((Hd, Wd, 2), dtype=torch.float64, device=dev)
-        _lib.check(_lib.lib().hsr_warp_coords_f64(ctypes.addressof(geo), Hd, Wd, out.data_ptr(), _stream()))
+        if rows is None:
+            out = torch.empty((Hd, Wd, 2), dtype=torch.float64, device=dev)
+            _lib.check(_lib.lib().hsr_warp_coords_f64(ctypes.addressof(geo), Hd, Wd, out.data_ptr(), _stream()))
+        else:
+            out = torch.empty((r1 - r0, Wd, 2), dtype=torch.float64, device=dev)
+            if out.numel():                   # an empty tensor has no storage to point at
+                _lib.check(_lib.lib().hsr_warp_coords_rows_f64(ctypes.addressof(geo), r0, r1 - r0, Wd, out.data_ptr(),
+                                                               _stream()))
     return out
 
 
 PLANE_WARP_KERNELS = {"bilinear": 1, "cubic": 2}
 
 
+def _plane_kernel(kernel: str) -> int:
+    code = PLANE_WARP_KERNELS.get(kernel)
+    if code is None:
+        raise ValueError(f"kernel must be one of {sorted(PLANE_WARP_KERNELS)} for a plane warp, got {kernel!r}")
+    return code
+
+
+def _coords_arg(coords) -> torch.Tensor:
+    co = _cuda(coords, "coords", torch.float64)
+    if co.dim() != 3 or co.shape[2] != 2 or not co.is_contiguous():
+        raise ValueError(f"coords must be a contiguous [Hd, Wd, 2] tensor, got shape {tuple(co.shape)}")
+    return co
+
+
+def _scales_geo(scales):
+    geo = _lib.WarpGeo()
+    geo.xscale, geo.yscale = float(scales[0]), float(scales[1])
+    return geo
+
+
+def warp_src_row_range(coords: torch.Tensor, src_shape, scales, *, kernel: str) -> torch.Tensor:
+    """int64[2] on the device: [first, last + 1) source row that :func:`warp_planes` reads through its filter for the
+    pixels of ``coords`` [rows, Wd, 2] f64 (a band of :func:`warp_coords`) on a source of ``src_shape`` = (Hs, Ws);
+    ``range[1] == 0`` when no pixel centre is inside the source (``hsr_warp_src_row_range``).  Conservative: zero
+    weights and invalid source pixels are counted, so a window of these rows is never too small."""
+    code = _plane_kernel(kernel)
+    co = _coords_arg(coords)
+    Hs, Ws = int(src_shape[0]), int(src_shape[1])
+    geo = _scales_geo(scales)
+    with torch.cuda.device_of(co):
+        rng = torch.tensor([-1, 0], dtype=torch.int64, device=co.device)       # u64 max, 0
+        _lib.check(_lib.lib().hsr_warp_src_row_range(co.data_ptr(), int(co.shape[0]), int(co.shape[1]), Hs, Ws,
+                                                     ctypes.addressof(geo), code, rng.data_ptr(), _stream()))
+    return rng
+
+
 def warp_planes(planes: torch.Tensor, src_valid: torch.Tensor, coords: torch.Tensor, scales, *, kernel: str,
                 fill_out: torch.Tensor, gate_k: int = 0, gate_gt: float = 0.0, out: Optional[torch.Tensor] = None,
-                valid_out: Optional[torch.Tensor] = None, fit_mask_out: Optional[torch.Tensor] = None):
+                valid_out: Optional[torch.Tensor] = None, fit_mask_out: Optional[torch.Tensor] = None,
+                src_row0: int = 0, src_rows_total: Optional[int] = None, outside: Optional[torch.Tensor] = None):
     """Warp K planar images ``planes`` [K, Hs, Ws] f32 (any plane stride, as ``alloc_planes`` pads them) onto the grid
     of ``coords`` [Hd, Wd, 2] f64 (:func:`warp_coords`) with the taps of :func:`warp` (``hsr_warp_planes_f32``).
     ``src_valid`` [Hs, Ws] bool/u8: source pixels whose taps may be used (the GLT valid mask); ``scales`` = (xscale,
     yscale) of ``EMIT_data.warp.warp_scales``; ``fill_out`` [K] f32: written where the destination is not covered.
     Returns ``(planes [K, Hd, Wd] f32, dst_valid [Hd, Wd] bool, fit_mask [Hd, Wd] bool)``, the fit mask being
-    ``dst_valid & isfinite(planes).all(0) & (planes[gate_k] > gate_gt)`` (gate_k < 0: no gate)."""
-    code = PLANE_WARP_KERNELS.get(kernel)
-    if code is None:
-        raise ValueError(f"kernel must be one of {sorted(PLANE_WARP_KERNELS)} for a plane warp, got {kernel!r}")
+    ``dst_valid & isfinite(planes).all(0) & (planes[gate_k] > gate_gt)`` (gate_k < 0: no gate).
+    ``src_row0`` / ``src_rows_total``: ``planes`` and ``src_valid`` hold only source rows [src_row0, src_row0 + Hs) of
+    a source of ``src_rows_total`` rows (``hsr_warp_planes_window_f32``; :func:`warp_src_row_range` sizes the window).
+    Where the window holds every row a pixel's taps reach, the result is bit-identical to the warp of the whole source;
+    the pixels that needed a row outside it are added to ``outside`` (int64[1] on the device), which must stay 0."""
+    code = _plane_kernel(kernel)
     p = _cuda(planes, "planes", torch.float32)
     if p.dim() != 3:
         raise ValueError(f"planes must be [K, Hs, Ws], got shape {tuple(p.shape)}")
     K, Hs, Ws = (int(d) for d in p.shape)
+    windowed = src_rows_total is not None or src_row0 != 0 or outside is not None
     ps = _plane_stride(p, K, Hs * Ws, "planes")
     sv = src_valid.view(torch.uint8) if src_valid.dtype == torch.bool else src_valid
     sv = _cuda(sv, "src_valid", torch.uint8).contiguous()
     if sv.numel() != Hs * Ws:
         raise ValueError(f"src_valid must have one entry per source pixel ({Hs} x {Ws}), got shape {tuple(sv.shape)}")
-    co = _cuda(coords, "coords", torch.float64)
-    if co.dim() != 3 or co.shape[2] != 2 or not co.is_contiguous():
-        raise ValueError(f"coords must be a contiguous [Hd, Wd, 2] tensor, got shape {tuple(co.shape)}")
+    co = _coords_arg(coords)
     Hd, Wd = int(co.shape[0]), int(co.shape[1])
     fo = _cuda(fill_out, "fill_out", torch.float32).contiguous()
     if fo.numel() != K:
         raise ValueError(f"fill_out must have K = {K} entries, got {fo.numel()}")
-    geo = _lib.WarpGeo()
-    geo.xscale, geo.yscale = float(scales[0]), float(scales[1])
+    if outside is not None:
+        _cuda(outside, "outside", torch.int64)
+        if outside.numel() != 1:
+            raise ValueError("outside must be an int64[1] device tensor")
+    geo = _scales_geo(scales)
     with torch.cuda.device_of(p):
         if out is None:
             out = alloc_planes(K, (Hd, Wd), p.device)
@@ -1201,8 +1255,15 @@ def warp_planes(planes: torch.Tensor, src_valid: torch.Tensor, coords: torch.Ten
                  else torch.empty(Hd * Wd, dtype=torch.uint8, device=p.device))
         fm = (_mask_out(fit_mask_out, Hd * Wd) if fit_mask_out is not None
               else torch.empty(Hd * Wd, dtype=torch.uint8, device=p.device))
-        _lib.check(_lib.lib().hsr_warp_planes_f32(p.data_ptr(), Hs, Ws, K, ps, sv.data_ptr(), co.data_ptr(),
-                                                  ctypes.addressof(geo), code, fo.data_ptr(), int(gate_k),
-                                                  float(gate_gt), Hd, Wd, out.data_ptr(), ops, valid.data_ptr(),
-                                                  fm.data_ptr(), _stream()))
+        if windowed:
+            total = int(src_rows_total) if src_rows_total is not None else int(src_row0) + Hs
+            _lib.check(_lib.lib().hsr_warp_planes_window_f32(
+                p.data_ptr(), total, Ws, K, ps, sv.data_ptr(), int(src_row0), Hs, co.data_ptr(), ctypes.addressof(geo),
+                code, fo.data_ptr(), int(gate_k), float(gate_gt), Hd, Wd, out.data_ptr(), ops, valid.data_ptr(),
+                fm.data_ptr(), _ptr(outside), _stream()))
+        else:
+            _lib.check(_lib.lib().hsr_warp_planes_f32(p.data_ptr(), Hs, Ws, K, ps, sv.data_ptr(), co.data_ptr(),
+                                                      ctypes.addressof(geo), code, fo.data_ptr(), int(gate_k),
+                                                      float(gate_gt), Hd, Wd, out.data_ptr(), ops, valid.data_ptr(),
+                                                      fm.data_ptr(), _stream()))
     return out, valid.view(torch.bool).view(Hd, Wd), fm.view(torch.bool).view(Hd, Wd)

@@ -12,7 +12,9 @@ from HBM once:
     poly_solve_apply (K, deg+1) coefficients and the colour-matched planes, clipped to [0, 1]
 
 ``synthesize_on_s2_grid`` runs the same pass on the Sentinel-2 UTM grid, where the reference fits: glt_srf, then a warp
-of the K planes onto the S2 grid (``warp_planes``), then the same fit and solve / apply.
+of the K planes onto the S2 grid (``warp_planes``), then the same fit and solve / apply.  ``synthesize_sharded`` takes
+granules with an S2 target too, and ``synthesize_slab_on_s2_grid`` runs one band of target rows of a mosaic, staging only
+the ortho and raw rows that band reads.
 """
 from __future__ import annotations
 
@@ -51,6 +53,7 @@ class PairResult:
     y_limits: Optional[torch.Tensor] = None  # ... and of the S2 reference
     raw_rows: Optional[tuple] = None         # synthesize_slab: the [row0, row1) raw rows that were staged
     grid: Optional[S2Target] = None          # synthesize_on_s2_grid: the S2 grid of bands / matched / valid / fit_mask
+    ortho_rows: Optional[tuple] = None       # synthesize_slab_on_s2_grid: the [row0, row1) ortho rows that were staged
 
 
 class PairSynthesizer:
@@ -142,6 +145,14 @@ class PairSynthesizer:
         return kernels.masked_percentiles_union(units, self.stretch, reduce=reduce or _no_reduce, K=self.K, pair=True,
                                                 device=self.device)
 
+    def _check_global(self, exchange, allreduce) -> bool:
+        """Whether a call's fit is global across ranks (``exchange=`` / ``allreduce=True`` with more than one
+        process); raises for a stretch whose limits would be per granule."""
+        global_fit = (exchange is not None and exchange.world > 1) or (allreduce and hdist.world()[1] > 1)
+        if global_fit:
+            self._no_global_stretch("exchange= / allreduce=True")
+        return global_fit
+
     def _global_reduce(self, group):
         """The SUM all-reduce of the percentile histograms of a global fit (None for one process)."""
         if self.stretch is None or hdist.group_size(group) == 1:
@@ -169,9 +180,7 @@ class PairSynthesizer:
         Three launches (+ the moment finalize): glt_srf, fit_moments, poly_solve_apply.
         Global fit across ranks: ``exchange`` (a ``dist.PeerExchange``: moments travel over NVLink peer memory
         inside the finalize / solve kernels) or ``allreduce=True`` (one NCCL all-reduce between the two)."""
-        global_fit = (exchange is not None and exchange.world > 1) or (allreduce and hdist.world()[1] > 1)
-        if global_fit:
-            self._no_global_stretch("exchange= / allreduce=True")
+        global_fit = self._check_global(exchange, allreduce)
         fm = torch.empty(glt_x.shape, dtype=torch.bool, device=raw.device)
         bands, valid, diag, ortho = self.bands_from_raw(raw, glt_x, glt_y, transpose_raw_yx=transpose_raw_yx,
                                                         materialize_ortho=materialize_ortho, bands_out=bands_out,
@@ -200,7 +209,7 @@ class PairSynthesizer:
     # ------------------------------------------------------------------ one granule on the Sentinel-2 grid
     def synthesize_on_s2_grid(self, raw: torch.Tensor, glt_x: torch.Tensor, glt_y: torch.Tensor, s2_ref: torch.Tensor,
                               target: S2Target, *, transpose_raw_yx: bool = False, bands_out=None,
-                              matched_out=None) -> PairResult:
+                              matched_out=None, group=None, allreduce: bool = False, exchange=None) -> PairResult:
         """The pair on the Sentinel-2 UTM grid ``target`` (:func:`hsr_b200.EMIT_data.warp.s2_target`), where the
         reference fits: ``s2_ref`` [K, Hd, Wd] f32 is the S2 stack on that grid.  Instead of warping the B-band ortho
         cube and integrating the SRF over it (nc_to_envi's gdalwarp, then synth.py:9-45), the K pseudo-S2 planes of
@@ -209,17 +218,31 @@ class PairSynthesizer:
         Stages: glt_srf, the target's cached coordinates, warp_planes, then the fit and solve / apply of
         :meth:`synthesize` (stretch, ``y_finite``, gate band and clip as there, on the S2-grid planes).
         ``bands``, ``matched``, ``valid`` and ``fit_mask`` of the result are on the target grid, ``diag`` is the GLT
-        diagnostics of the source pass and ``grid`` is ``target``.  Deviation from the reference: a GLT-valid raw
-        spectrum holding the nodata value in some or all of its bands is used as data (DESIGN section 7)."""
-        Hd, Wd = target.shape
+        diagnostics of the source pass and ``grid`` is ``target``.  ``group`` / ``allreduce`` / ``exchange``: a global
+        fit across ranks, one granule per rank, as in :meth:`synthesize` (with ``stretch_scope="fit"`` the limits are
+        those of every rank's pixels).  Deviation from the reference: a GLT-valid raw spectrum holding the nodata value
+        in some or all of its bands is used as data (DESIGN section 7)."""
+        self._check_s2_ref(s2_ref, target.shape)
+        global_fit = self._check_global(exchange, allreduce)
+        bands, dvalid, fm, diag = self._planes_on_grid(raw, glt_x, glt_y, target, transpose_raw_yx, bands_out)
+        ex = exchange.next() if exchange is not None and exchange.world > 1 else None
+        reduce = self._global_reduce(group) if global_fit else None
+        return self._fit_apply(bands, s2_ref, dvalid, fm, diag, matched_out=matched_out, ex=ex, reduce=reduce,
+                               allreduce=allreduce, group=group, grid=target)
+
+    def _check_s2_ref(self, s2_ref, shape) -> None:
+        Hd, Wd = shape
         if tuple(s2_ref.shape) != (self.K, Hd, Wd):
             raise ValueError(f"s2_ref must be [K={self.K}, {Hd}, {Wd}] on the target grid, got {tuple(s2_ref.shape)}")
+
+    def _planes_on_grid(self, raw, glt_x, glt_y, target: S2Target, transpose_raw_yx=False, bands_out=None):
+        """glt_srf, then the plane warp onto ``target``: (bands, dst_valid, fit_mask, diag)."""
         src, valid, diag, _ = self.bands_from_raw(raw, glt_x, glt_y, transpose_raw_yx=transpose_raw_yx)
-        fm = torch.empty((Hd, Wd), dtype=torch.bool, device=src.device)
+        fm = torch.empty(target.shape, dtype=torch.bool, device=src.device)
         bands, dvalid, fm = kernels.warp_planes(src, valid, target.coords(src.device), target.scales,
                                                 kernel=target.kernel, fill_out=self.fill_out, gate_k=self.gate_k,
                                                 gate_gt=0.0, out=bands_out, fit_mask_out=fm)
-        return self._fit_apply(bands, s2_ref, dvalid, fm, diag, matched_out=matched_out, grid=target)
+        return bands, dvalid, fm, diag
 
     # ------------------------------------------------------------------ a row slab of a mosaic
     def synthesize_slab(self, raw, glt_x: torch.Tensor, glt_y: torch.Tensor, s2_ref: torch.Tensor, *,
@@ -233,25 +256,11 @@ class PairSynthesizer:
         reference planes.  ``stage``: optional preallocated CUDA buffer the window is copied into (flat f32, at least
         rows * Wr * B elements).  Other keywords as :meth:`synthesize` (``exchange=`` / ``allreduce=`` make the fit
         global over the slabs).  The result's ``raw_rows`` holds the staged [row0, row1) range."""
-        import numpy as np
-
-        if isinstance(raw, np.ndarray):
-            raw = torch.from_numpy(raw)
+        raw = _as_tensor(raw)
         d0, d1 = int(raw.shape[0]), int(raw.shape[1])
         Hr, Wr = (d1, d0) if transpose_raw_yx else (d0, d1)
         with torch.cuda.device(self.device):
-            lo, hi = kernels.glt_row_range(glt_x, glt_y, Hr, Wr, transpose_raw_yx=transpose_raw_yx).tolist()
-            if hi == 0:                       # no valid entry in this slab: any one row will do
-                lo, hi = 0, 1
-            win = raw[lo:hi]
-            if not win.is_cuda:
-                n = win.numel()
-                buf = stage if stage is not None else torch.empty(n, dtype=torch.float32, device=self.device)
-                if buf.numel() < n:
-                    raise ValueError(f"stage holds {buf.numel()} floats, the slab's raw window needs {n}")
-                dst = buf.view(-1)[:n].view(win.shape)
-                dst.copy_(win, non_blocking=win.is_pinned())
-                win = dst
+            lo, hi, win = self._stage_raw(raw, glt_x, glt_y, Hr, Wr, transpose_raw_yx, stage)
             res = self.synthesize(win, glt_x, glt_y, s2_ref, transpose_raw_yx=transpose_raw_yx, raw_row0=lo,
                                   raw_rows_total=d0, **kw)
             outside = int(res.diag[3])
@@ -259,6 +268,88 @@ class PairSynthesizer:
                 raise RuntimeError(f"{outside} valid GLT entries fell outside the staged raw rows [{lo}, {hi})")
         res.diag = res.diag[:3]
         res.raw_rows = (lo, hi)
+        return res
+
+    def _stage_raw(self, raw, glt_x, glt_y, Hr, Wr, transpose_raw_yx, stage):
+        """(lo, hi, window on the device): the raw rows [lo, hi) the GLT rows reference, copied into ``stage`` (or a
+        new device buffer) when ``raw`` is in host memory."""
+        lo, hi = kernels.glt_row_range(glt_x, glt_y, Hr, Wr, transpose_raw_yx=transpose_raw_yx).tolist()
+        if hi == 0:                       # no valid entry in this slab: any one row will do
+            lo, hi = 0, 1
+        win = raw[lo:hi]
+        if not win.is_cuda:
+            n = win.numel()
+            buf = stage if stage is not None else torch.empty(n, dtype=torch.float32, device=self.device)
+            if buf.numel() < n:
+                raise ValueError(f"stage holds {buf.numel()} floats, the slab's raw window needs {n}")
+            dst = buf.view(-1)[:n].view(win.shape)
+            dst.copy_(win, non_blocking=win.is_pinned())
+            win = dst
+        return lo, hi, win
+
+    # ------------------------------------------------------------------ a row band of a mosaic on the Sentinel-2 grid
+    def synthesize_slab_on_s2_grid(self, raw, glt_x: torch.Tensor, glt_y: torch.Tensor, s2_ref: torch.Tensor,
+                                   target: S2Target, rows, *, transpose_raw_yx: bool = False,
+                                   stage: Optional[torch.Tensor] = None, group=None, allreduce: bool = False,
+                                   exchange=None) -> PairResult:
+        """One band ``rows`` = (t0, t1) of the target rows of a mosaic on the Sentinel-2 grid ``target``
+        (``dist.shard_rows(target.shape[0], ...)`` deals the bands), staging only what the band reads: the
+        coordinates of its rows, the ortho rows [o0, o1) its filter reaches (``kernels.warp_src_row_range``), the raw
+        rows the GLT rows [o0, o1) reference (``kernels.glt_row_range``), then glt_srf on those GLT rows through a raw
+        view, the plane warp over the ortho window and the fit / solve / apply of :meth:`synthesize_on_s2_grid`.
+
+        raw: the whole raw mosaic [Hr, Wr, B] f32 — a (pinned) host tensor / numpy array or a CUDA tensor; glt_x /
+        glt_y: the whole GLT [Ho, Wo] on the device; s2_ref: [K, t1 - t0, Wd], the band's rows of the reference.
+        ``stage``: as in :meth:`synthesize_slab`.  ``group`` / ``allreduce`` / ``exchange``: a global fit over the bands
+        of every rank (with ``stretch_scope="fit"``, limits over every band).  Stitched along rows, the bands' planes
+        and masks are bit-identical to one :meth:`synthesize_on_s2_grid` call: the windowed warp reads the same source
+        values with the same weights.  A band that reads no source row (no pixel centre inside the ortho grid) stages
+        nothing and yields fill, and still takes part in the exchange / all-reduce / percentile reduce.
+
+        The result's ``raw_rows`` and ``ortho_rows`` hold the staged [row0, row1) ranges.  ``diag`` is the GLT
+        diagnostics of the staged ortho rows; neighbouring bands overlap by the filter footprint, so the bands' diag
+        do NOT sum to the granule's.  Raises ``RuntimeError`` when a GLT entry or a filter tap fell outside the staged
+        rows (after the fit, so that no rank is left waiting in the exchange)."""
+        Hd, Wd = target.shape
+        t0, t1 = int(rows[0]), int(rows[1])
+        if not 0 <= t0 < t1 <= Hd:
+            raise ValueError(f"rows must satisfy 0 <= t0 < t1 <= {Hd}, got {tuple(rows)}")
+        self._check_s2_ref(s2_ref, (t1 - t0, Wd))
+        global_fit = self._check_global(exchange, allreduce)
+        raw = _as_tensor(raw)
+        d0, d1 = int(raw.shape[0]), int(raw.shape[1])
+        Hr, Wr = (d1, d0) if transpose_raw_yx else (d0, d1)
+        Ho, Wo = glt_x.shape
+        with torch.cuda.device(self.device):
+            coords = target.coords(self.device, rows=(t0, t1))
+            o0, o1 = kernels.warp_src_row_range(coords, (Ho, Wo), target.scales, kernel=target.kernel).tolist()
+            if o1 == 0:                       # no pixel centre inside the ortho grid: nothing to stage
+                o0 = o1 = lo = hi = 0
+                src = torch.empty((self.K, 0, Wo), dtype=torch.float32, device=self.device)
+                valid = torch.empty((0, Wo), dtype=torch.bool, device=self.device)
+                diag = torch.zeros(4, dtype=torch.int64, device=self.device)
+            else:
+                gx, gy = glt_x[o0:o1], glt_y[o0:o1]
+                lo, hi, win = self._stage_raw(raw, gx, gy, Hr, Wr, transpose_raw_yx, stage)
+                src, valid, diag, _ = self.bands_from_raw(win, gx, gy, transpose_raw_yx=transpose_raw_yx, raw_row0=lo,
+                                                          raw_rows_total=d0)
+            outside = torch.zeros(1, dtype=torch.int64, device=self.device)
+            fm = torch.empty((t1 - t0, Wd), dtype=torch.bool, device=self.device)
+            bands, dvalid, fm = kernels.warp_planes(src, valid, coords, target.scales, kernel=target.kernel,
+                                                    fill_out=self.fill_out, gate_k=self.gate_k, gate_gt=0.0,
+                                                    fit_mask_out=fm, src_row0=o0, src_rows_total=Ho, outside=outside)
+            ex = exchange.next() if exchange is not None and exchange.world > 1 else None
+            reduce = self._global_reduce(group) if global_fit else None
+            res = self._fit_apply(bands, s2_ref, dvalid, fm, diag, ex=ex, reduce=reduce, allreduce=allreduce,
+                                  group=group, grid=target)
+            raw_missed, tap_missed = torch.cat([res.diag[3:], outside]).tolist()
+            if raw_missed:
+                raise RuntimeError(f"{raw_missed} valid GLT entries fell outside the staged raw rows [{lo}, {hi})")
+            if tap_missed:
+                raise RuntimeError(f"{tap_missed} target pixels needed ortho rows outside the staged rows [{o0}, {o1})")
+        res.diag = res.diag[:3]
+        res.raw_rows = (lo, hi)
+        res.ortho_rows = (o0, o1)
         return res
 
     # ------------------------------------------------------------------ a batch of equal tiles
@@ -284,7 +375,9 @@ class PairSynthesizer:
 
     # ------------------------------------------------------------------ many granules, one global fit
     def synthesize_sharded(self, granules: Sequence[dict], *, group=None, exchange=None) -> List[PairResult]:
-        """Granules owned by THIS rank (dicts with raw, glt_x, glt_y, s2_ref) — BASELINE configs[3]; the fit is
+        """Granules owned by THIS rank (dicts with raw, glt_x, glt_y, s2_ref, optionally "target": an ``S2Target``, for
+        a granule synthesised on that Sentinel-2 grid as :meth:`synthesize_on_s2_grid` does, s2_ref then being on the
+        target grid and the result's ``grid`` the target) — BASELINE configs[3]; the fit is
         GLOBAL: the local moments are summed in a fixed order (``kernels.moments_sum``), summed across ranks once —
         over NVLink peer memory when ``exchange`` (a ``dist.PeerExchange``) is given, else one all-reduce (NCCL /
         gloo) — and solved redundantly.  A rank that was dealt no granule still takes part in the exchange.
@@ -293,24 +386,30 @@ class PairSynthesizer:
         self._no_global_stretch("synthesize_sharded")
         stage = []
         for g in granules:
-            fm = torch.empty(g["glt_x"].shape, dtype=torch.bool, device=self.device)
-            bands, valid, diag, _ = self.bands_from_raw(g["raw"], g["glt_x"], g["glt_y"],
-                                                        transpose_raw_yx=g.get("transpose_raw_yx", False),
-                                                        fit_mask_out=fm)
+            target = g.get("target")
+            if target is not None:
+                self._check_s2_ref(g["s2_ref"], target.shape)
+                bands, valid, fm, diag = self._planes_on_grid(g["raw"], g["glt_x"], g["glt_y"], target,
+                                                              g.get("transpose_raw_yx", False))
+            else:
+                fm = torch.empty(g["glt_x"].shape, dtype=torch.bool, device=self.device)
+                bands, valid, diag, _ = self.bands_from_raw(g["raw"], g["glt_x"], g["glt_y"],
+                                                            transpose_raw_yx=g.get("transpose_raw_yx", False),
+                                                            fit_mask_out=fm)
             if self.stretch is not None:
                 fm = self.stretch_mask(bands, g["s2_ref"], valid, fm)
-            stage.append((bands, valid, diag, fm, g["s2_ref"]))
+            stage.append((bands, valid, diag, fm, g["s2_ref"], target))
         xl = yl = None
         if self.stretch is not None:
             xl, yl = self.stretch_limits([(s[0], s[4], s[3]) for s in stage], self._global_reduce(group))
         moms = []
-        for i, (bands, valid, diag, fm, s2_ref) in enumerate(stage):
+        for i, (bands, valid, diag, fm, s2_ref, target) in enumerate(stage):
             if self.stretch is not None:
                 mom, _ = kernels.fit_moments(bands, s2_ref, fm, self.deg, mask_given=True, x_stretch=xl, y_stretch=yl)
             else:
                 mom, fm, _, _ = self.fit(bands, s2_ref, valid, fm)
             moms.append(mom.view(self.K, -1))
-            stage[i] = (bands, valid, diag, fm)
+            stage[i] = (bands, valid, diag, fm, target)
         ex = exchange.next() if exchange is not None and exchange.world > 1 else None
         like = torch.empty((self.K, 3 * self.deg + 2), dtype=torch.float64, device=self.device)
         with torch.cuda.device(self.device):
@@ -325,7 +424,7 @@ class PairSynthesizer:
             x0 = torch.zeros((self.K, 1), dtype=torch.float32, device=self.device)
             m0 = torch.zeros(1, dtype=torch.uint8, device=self.device)
             kernels.poly_solve_apply(x0, mom, m0, self.deg, min_count=self.min_count, lo=lo, hi=hi, exchange=ex)
-        for i, (bands, valid, diag, fm) in enumerate(stage):
+        for i, (bands, valid, diag, fm, target) in enumerate(stage):
             if i == 0 and ex is not None:
                 gmom = torch.empty_like(mom)
                 coeffs, matched = kernels.poly_solve_apply(bands, mom, fm, self.deg, min_count=self.min_count, lo=lo,
@@ -335,8 +434,15 @@ class PairSynthesizer:
                 coeffs, matched = kernels.poly_solve_apply(bands, mom, fm, self.deg, min_count=self.min_count, lo=lo,
                                                            hi=hi, x_stretch=xl)
             out.append(PairResult(bands, matched, coeffs.view(self.K, self.deg + 1), valid, fm.view(valid.shape), diag,
-                                  mom, None, self.band_names, xl, yl))
+                                  mom, None, self.band_names, xl, yl, grid=target))
         return out
+
+
+def _as_tensor(raw):
+    """A numpy raw mosaic as a (host) tensor; tensors pass through."""
+    import numpy as np
+
+    return torch.from_numpy(raw) if isinstance(raw, np.ndarray) else raw
 
 
 class HostGranuleStream:

@@ -586,6 +586,47 @@ HSR_API int hsr_warp_planes_f32(const float* src, int64_t Hs, int64_t Ws, int K,
                                 int64_t dst_plane_stride, uint8_t* dst_valid, uint8_t* fit_mask, void* stream);
 
 /*
+ * Row slabs of the Sentinel-2 grid (a mosaic target dealt to ranks by rows).  Call order for one band of target rows
+ * [row0, row0 + rows): hsr_warp_coords_rows_f64 -> hsr_warp_src_row_range (source = ortho rows [o0, o1)) ->
+ * hsr_glt_row_range on GLT rows [o0, o1) (raw rows to stage) -> hsr_glt_srf_f32 with an hsr_raw_view_t ->
+ * hsr_warp_planes_window_f32 with src_row0 = o0, src_rows = o1 - o0.
+ *
+ * hsr_warp_coords_rows_f64: coords[r - row0] for destination rows r in [row0, row0 + rows), coords [rows, Wd, 2] f64.
+ * The transform takes the absolute row (r + 0.5), so the band is bit-identical to those rows of hsr_warp_coords_f64.
+ */
+HSR_API int hsr_warp_coords_rows_f64(const hsr_warp_geo_t* geo, int64_t row0, int64_t rows, int64_t Wd, double* coords,
+                                     void* stream);
+/*
+ * hsr_warp_src_row_range: the source rows that hsr_warp_planes_f32 reads for the destination pixels of coords
+ * [rows, Wd, 2] (16-byte aligned).  Over every pixel whose centre is inside the Hs x Ws source: range[0] =
+ * min(floor(py - 0.5) + 1 - ry), range[1] = max(floor(py - 0.5) + 1 + ry), both clipped to [0, Hs), with ry the
+ * plane warp's row radius for `kernel` (1 / 2) and geo->yscale (only xscale / yscale are read).  Conservative: taps
+ * of zero weight and invalid source pixels are included.  ACCUMULATED with min / max like hsr_glt_row_range: the
+ * caller initialises range to {UINT64_MAX, 0}; an untouched range means no centre is inside the source.
+ */
+HSR_API int hsr_warp_src_row_range(const double* coords, int64_t rows, int64_t Wd, int64_t Hs, int64_t Ws,
+                                   const hsr_warp_geo_t* geo, int kernel, unsigned long long* range /*[2] u64*/,
+                                   void* stream);
+/*
+ * hsr_warp_planes_window_f32: hsr_warp_planes_f32 over a window of source rows.  src / src_valid hold only rows
+ * [src_row0, src_row0 + src_rows) of the logical Hs x Ws source (plane stride >= src_rows * Ws unless K == 1); Hs
+ * stays the logical height, so the "centre outside the source" test, the tap bounds, the weights and the fp64 sums are
+ * those of the unwindowed call, and where the window holds every row a pixel's non-zero-weight taps reach, its output
+ * is bit-identical to hsr_warp_planes_f32 on the whole source.  A non-zero-weight tap in a row outside the window is
+ * skipped and its destination pixel counted in *outside (nullable, u64, ACCUMULATED): the caller must treat a non-zero
+ * count as an error (it sized the window wrongly), as it does diag[3] of a raw view.  src_rows = 0 is allowed (src /
+ * src_valid may then be NULL): nothing is read and every pixel gets fill_out, dst_valid = 0 and fit_mask = 0.
+ * hsr_warp_planes_f32 is this call with src_row0 = 0, src_rows = Hs and no counter.
+ * HSR_EINVAL: as hsr_warp_planes_f32, and a window outside [0, Hs).
+ */
+HSR_API int hsr_warp_planes_window_f32(const float* src, int64_t Hs, int64_t Ws, int K, int64_t src_plane_stride,
+                                       const uint8_t* src_valid, int64_t src_row0, int64_t src_rows,
+                                       const double* coords, const hsr_warp_geo_t* geo, int kernel,
+                                       const float* fill_out, int gate_k, float gate_gt, int64_t Hd, int64_t Wd,
+                                       float* dst, int64_t dst_plane_stride, uint8_t* dst_valid, uint8_t* fit_mask,
+                                       unsigned long long* outside, void* stream);
+
+/*
  * Peer blocks for hsr_exchange_t.  hsr_peer_alloc creates (cudaMalloc + zero) this rank's block — the one
  * persistent allocation the library makes, the analogue of a communicator; hsr_ipc_export / hsr_ipc_import wrap
  * cudaIpcGetMemHandle / cudaIpcOpenMemHandle (lazy peer access) so that the processes of one node can map each
