@@ -90,6 +90,8 @@ SIGNATURES = {
                                         _p, _i64, _i64, _p, _p, _p]),
     "hsr_block_average_f32": (_int, [_p, _int, _int, _i64, _i64, _i64, _int, _int, _c.c_double, _int, _f32, _p, _i64, _p]),
     "hsr_bilinear_upsample_f32": (_int, [_p, _int, _i64, _i64, _i64, _int, _int, _f32, _p, _i64, _p]),
+    "hsr_bilinear_fine_mask_u8": (_int, [_p, _int, _i64, _i64, _i64, _int, _p, _p]),
+    "hsr_bilinear_apply_f32": (_int, [_p, _int, _i64, _i64, _i64, _int, _p, _int, _p, _f32, _f32, _p, _i64, _p, _p]),
     "hsr_stretch_f64": (_int, [_p, _i64, _i64, _p, _p, _i64, _int, _int, _p, _i64, _i64, _p]),
     "hsr_notnan_mask_u8": (_int, [_p, _p, _i64, _p, _p]),
     "hsr_run_ends_u8": (_int, [_p, _i64, _p, _p]),
@@ -134,6 +136,7 @@ SIGNATURES = {
     "hsr_union_select_begin": (_int, [_p, _int, _int, _p, _p, _p]),
     "hsr_union_select_count": (_int, [_p, _i64, _p, _i64, _p, _i64, _int, _int, _int, _p, _p, _p]),
     "hsr_union_select_step": (_int, [_int, _int, _int, _p, _p, _p, _p, _p]),
+    "hsr_union_select_count_bilinear": (_int, [_p, _i64, _i64, _i64, _int, _p, _int, _int, _int, _p, _p, _p]),
 }
 
 _lock = threading.Lock()

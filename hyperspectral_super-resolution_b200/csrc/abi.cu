@@ -80,6 +80,9 @@ int block_average_impl(const void*, int, int, long long, long long, long long, i
                        long long, cudaStream_t);
 int bilinear_upsample_impl(const float*, int, long long, long long, long long, int, int, float, float*, long long,
                            cudaStream_t);
+int bilinear_fine_mask_impl(const float*, int, long long, long long, long long, int, uint8_t*, cudaStream_t);
+int bilinear_apply_impl(const float*, int, long long, long long, long long, int, const double*, int, const double*, float,
+                        float, float*, long long, uint8_t*, cudaStream_t);
 int warp_impl(const float*, long long, long long, int, long long, const hsr_warp_geo_t*, int, int, float, float,
               long long, long long, float*, long long, void*, size_t, cudaStream_t);
 size_t warp_workspace(long long, long long);
@@ -125,6 +128,8 @@ long long union_hist_doubles(int Q, int S);
 int union_begin_impl(const double*, int, int, void*, double*, cudaStream_t);
 int union_count_impl(const float*, long long, const float*, long long, const uint8_t*, long long, int, int, int, void*,
                      double*, cudaStream_t);
+int union_count_bilinear_impl(const float*, long long, long long, long long, int, const uint8_t*, int, int, int, void*,
+                              double*, cudaStream_t);
 int union_step_impl(int, int, int, void*, double*, double*, int*, cudaStream_t);
 
 size_t compact_workspace(long long n);
@@ -279,6 +284,13 @@ int hsr_union_select_count(const float* x, int64_t x_k_stride, const float* y, i
     return hsr::union_count_impl(x, x_k_stride, y, y_k_stride, mask, n, K, Q, pass, state, hist, (cudaStream_t)stream);
 }
 
+int hsr_union_select_count_bilinear(const float* src, int64_t src_plane_stride, int64_t Hs, int64_t Ws, int factor,
+                                    const uint8_t* mask, int K, int Q, int pass, void* state, double* hist,
+                                    void* stream) {
+    return hsr::union_count_bilinear_impl(src, src_plane_stride, Hs, Ws, factor, mask, K, Q, pass, state, hist,
+                                          (cudaStream_t)stream);
+}
+
 int hsr_union_select_step(int Q, int S, int pass, void* state, double* hist, double* out, int* more, void* stream) {
     return hsr::union_step_impl(Q, S, pass, state, hist, out, more, (cudaStream_t)stream);
 }
@@ -337,6 +349,18 @@ int hsr_bilinear_upsample_f32(const float* src, int C, int64_t Hs, int64_t Ws, i
                               int has_nodata, float nodata, float* dst, int64_t dst_plane_stride, void* stream) {
     return hsr::bilinear_upsample_impl(src, C, Hs, Ws, src_plane_stride, factor, has_nodata, nodata, dst, dst_plane_stride,
                                        (cudaStream_t)stream);
+}
+
+int hsr_bilinear_fine_mask_u8(const float* src, int K, int64_t Hs, int64_t Ws, int64_t src_plane_stride, int factor,
+                              uint8_t* mask, void* stream) {
+    return hsr::bilinear_fine_mask_impl(src, K, Hs, Ws, src_plane_stride, factor, mask, (cudaStream_t)stream);
+}
+
+int hsr_bilinear_apply_f32(const float* src, int K, int64_t Hs, int64_t Ws, int64_t src_plane_stride, int factor,
+                           const double* coeffs, int deg, const double* x_stretch, float lo, float hi, float* dst,
+                           int64_t dst_plane_stride, uint8_t* mask_out, void* stream) {
+    return hsr::bilinear_apply_impl(src, K, Hs, Ws, src_plane_stride, factor, coeffs, deg, x_stretch, lo, hi, dst,
+                                    dst_plane_stride, mask_out, (cudaStream_t)stream);
 }
 
 int hsr_warp_f32(const float* src, int64_t Hs, int64_t Ws, int bands, int64_t src_pix_stride, const hsr_warp_geo_t* geo,

@@ -159,6 +159,50 @@ __device__ __forceinline__ bool close32(float x, float y, float tol) {
     return fabsf(__fsub_rn(x, y)) <= tol || x == y;
 }
 
+// ---------------------------------------------------------------- bilinear x factor onto an aligned finer grid
+// The 2 x 2 fp64 interpolation of hsr_bilinear_upsample_f32 (s2_emit/poly_regression.py:150-156), split so that a
+// kernel mapping several planes at one fine pixel forms the pixel's taps once.  The destination pixel centre
+// ((x + 0.5) / factor - 0.5 in source pixel coordinates) is interpolated from its 2 x 2 source neighbours; neighbours
+// outside the source, equal to nodata or NaN are skipped and the weights renormalised, none usable -> 0.  Every kernel
+// that resamples this way goes through these two helpers, so their fine values carry the same bits.
+struct BilinearTap {
+    long long y0, x0;
+    double wy1, wx1;
+};
+
+__device__ __forceinline__ BilinearTap bilinear_up_tap(long long y, long long x, int factor) {
+    const double sy = ((double)y + 0.5) / factor - 0.5, sx = ((double)x + 0.5) / factor - 0.5;
+    const double fy = floor(sy), fx = floor(sx);
+    return {(long long)fy, (long long)fx, sy - fy, sx - fx};
+}
+
+__device__ __forceinline__ float bilinear_up_value(const float* __restrict__ sp, long long Hs, long long Ws,
+                                                   const BilinearTap& t, int has_nodata, float nodata) {
+    double acc = 0.0, wsum = 0.0;
+#pragma unroll
+    for (int dy = 0; dy < 2; ++dy) {
+        const long long yy = t.y0 + dy;
+        const double wy = dy ? t.wy1 : 1.0 - t.wy1;
+        if (yy < 0 || yy >= Hs) continue;
+#pragma unroll
+        for (int dx = 0; dx < 2; ++dx) {
+            const long long xx = t.x0 + dx;
+            const double w = wy * (dx ? t.wx1 : 1.0 - t.wx1);
+            if (xx < 0 || xx >= Ws || w == 0.0) continue;
+            const float v = __ldg(sp + yy * Ws + xx);
+            if ((has_nodata && v == nodata) || v != v) continue;
+            acc += w * (double)v;
+            wsum += w;
+        }
+    }
+    return wsum > 0.0 ? (float)(acc / wsum) : 0.f;
+}
+
+// fine (y, x) of flat index i of a plane Wd wide, then of i + 1 (no division)
+__device__ __forceinline__ void next_pixel(long long& y, long long& x, long long Wd) {
+    if (++x == Wd) x = 0, ++y;
+}
+
 // tiles_helpers/utils.py:357-371: valid = isfinite(v) & (v != nodata); clip(int32(rint(v * scale)), 0, hi), nd otherwise.
 // rint by the 1.5 * 2^23 trick (round-to-nearest-even of the clamped product; exact for 0 <= t <= 65534); a product
 // beyond int32 converts to INT_MIN on x86 (numpy's astype) and is therefore clipped to 0.

@@ -733,6 +733,93 @@ void launch_apply(const float* x, long long xks, long long xns, const double* co
                                                      ons);
 }
 
+// Colour-matched planes on the factor-times finer aligned grid (s2_emit/poly_regression.py:150-162) in one pass: for
+// every fine pixel the K fine values are interpolated from the coarse planes (bilinear_up_value, the bits of
+// hsr_bilinear_upsample_f32), mask10 = all_k finite, then per plane the percentile stretch (stretch1, as
+// solve_apply_kernel), Horner under mask10 and the clip (horner_clip).  One thread per 4 fine pixels of the flat index
+// (16-byte stores when the planes allow it); the 4 x K fine values wait in a thread-private slice of dynamic shared
+// memory [K * 4][256] between the mask and the apply, so no register array is indexed by the run-time K.
+struct FineApplyParams {
+    const float* src;
+    long long sps, Hs, Ws;
+    int factor, K, vec, vecm;
+    const double* coeffs;  // [K, DEG+1]
+    const double* xst;     // nullable [K][2] (lo, hi)
+    float lo, hi;
+    float* dst;
+    long long dps;
+    uint8_t* mask;         // nullable [n]
+};
+
+constexpr int FINE_THREADS = 256;
+
+template <int DEG, bool STRETCH>
+__global__ void __launch_bounds__(FINE_THREADS) bilinear_apply_kernel(const FineApplyParams P) {
+    extern __shared__ float fv[];                 // [K * 4][FINE_THREADS]
+    __shared__ double cs[HSR_MAX_SRF_BANDS][DEG + 1];
+    __shared__ double sl[HSR_MAX_SRF_BANDS][3];   // lo, den, rcp of the stretch
+    const int tid = threadIdx.x, K = P.K;
+    for (int e = tid; e < K * (DEG + 1); e += FINE_THREADS) cs[e / (DEG + 1)][e % (DEG + 1)] = P.coeffs[e];
+    if (STRETCH && tid < K) {
+        const double lo = P.xst[2 * tid];
+        const double den = P.xst[2 * tid + 1] - lo + 1e-12;
+        sl[tid][0] = lo, sl[tid][1] = den, sl[tid][2] = 1.0 / den;
+    }
+    __syncthreads();
+    const long long Wd = P.Ws * P.factor, n = P.Hs * P.factor * Wd, n4 = (n + 3) >> 2;
+    for (long long q = blockIdx.x * (long long)FINE_THREADS + tid; q < n4; q += (long long)gridDim.x * FINE_THREADS) {
+        const long long i = q << 2;
+        long long y = i / Wd, x = i - y * Wd;
+        BilinearTap t[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            t[j] = bilinear_up_tap(y, x, P.factor);
+            next_pixel(y, x, Wd);
+        }
+        const unsigned int inside = i + 4 <= n ? 0xfu : (1u << (n - i)) - 1u;
+        unsigned int m = inside;
+        for (int k = 0; k < K; ++k) {
+            const float* sp = P.src + (long long)k * P.sps;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                float v = 0.f;
+                if ((inside >> j) & 1u) v = bilinear_up_value(sp, P.Hs, P.Ws, t[j], 0, 0.f);
+                if (!finite_f32(v)) m &= ~(1u << j);
+                fv[(k * 4 + j) * FINE_THREADS + tid] = v;
+            }
+        }
+        for (int k = 0; k < K; ++k) {
+            double c[DEG + 1];
+#pragma unroll
+            for (int d = 0; d <= DEG; ++d) c[d] = cs[k][d];
+            float r[4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                float v = fv[(k * 4 + j) * FINE_THREADS + tid];
+                if (STRETCH) v = stretch1(v, sl[k][0], sl[k][1], sl[k][2]);
+                r[j] = horner_clip<DEG>(v, c, ((m >> j) & 1u) != 0u, P.lo, P.hi);
+            }
+            float* dp = P.dst + (long long)k * P.dps;
+            if (P.vec && inside == 0xfu) {
+                __stcs(reinterpret_cast<float4*>(dp + i), make_float4(r[0], r[1], r[2], r[3]));
+            } else {
+#pragma unroll
+                for (int j = 0; j < 4; ++j)
+                    if ((inside >> j) & 1u) dp[i + j] = r[j];
+            }
+        }
+        if (P.mask) {
+            if (P.vecm && inside == 0xfu) {
+                *reinterpret_cast<uchar4*>(P.mask + i) =
+                    make_uchar4(m & 1u, (m >> 1) & 1u, (m >> 2) & 1u, (m >> 3) & 1u);
+            } else {
+                for (int j = 0; j < 4; ++j)
+                    if ((inside >> j) & 1u) P.mask[i + j] = (m >> j) & 1u;
+            }
+        }
+    }
+}
+
 }  // namespace
 
 size_t poly_moments_workspace(long long n, int K, int deg) {
@@ -895,6 +982,43 @@ int poly_solve_apply_impl(const float* x, long long xks, long long xgs, const do
         solve_apply_kernel<D, true><<<grid, 256, 0, stream>>>(P); \
     else                                                          \
         solve_apply_kernel<D, false><<<grid, 256, 0, stream>>>(P)
+    HSR_DEG_SWITCH(deg, CALL)
+#undef CALL
+    HSR_CUDA(cudaGetLastError());
+    return HSR_OK;
+}
+
+int bilinear_apply_impl(const float* src, int K, long long Hs, long long Ws, long long src_plane_stride, int factor,
+                        const double* coeffs, int deg, const double* x_stretch, float lo, float hi, float* dst,
+                        long long dst_plane_stride, uint8_t* mask_out, cudaStream_t stream) {
+    HSR_REQUIRE(src && coeffs && dst, HSR_EINVAL, "null src / coeffs / dst pointer");
+    HSR_REQUIRE(K >= 1 && K <= HSR_MAX_SRF_BANDS && Hs >= 0 && Ws >= 0 && factor >= 1, HSR_EINVAL,
+                "bad K = %d (1..%d), shape or factor", K, HSR_MAX_SRF_BANDS);
+    HSR_REQUIRE(deg >= 1 && deg <= MAXDEG, HSR_ERANGE, "deg = %d outside [1, %d]", deg, MAXDEG);
+    const long long n = Hs * Ws * factor * factor;
+    HSR_REQUIRE(src_plane_stride >= Hs * Ws && dst_plane_stride >= n, HSR_EINVAL, "plane stride too small");
+    HSR_REQUIRE(((reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst)) & 3) == 0, HSR_EALIGN,
+                "src / dst not 4-byte aligned");
+    if (n == 0) return HSR_OK;
+    FineApplyParams P{};
+    P.src = src, P.sps = K > 1 ? src_plane_stride : Hs * Ws, P.Hs = Hs, P.Ws = Ws, P.factor = factor, P.K = K;
+    P.coeffs = coeffs, P.xst = x_stretch, P.lo = lo, P.hi = hi, P.dst = dst, P.dps = K > 1 ? dst_plane_stride : n;
+    P.mask = mask_out;
+    P.vec = ((reinterpret_cast<uintptr_t>(dst) | (uintptr_t)(P.dps * 4)) & 15) == 0 ? 1 : 0;
+    P.vecm = (reinterpret_cast<uintptr_t>(mask_out) & 3) == 0 ? 1 : 0;
+    const int smem = K * 4 * FINE_THREADS * (int)sizeof(float);
+    const long long n4 = (n + 3) / 4;
+    const long long want = (n4 + FINE_THREADS - 1) / FINE_THREADS;
+#define CALL(D)                                                                                                      \
+    {                                                                                                                \
+        auto kern = x_stretch ? bilinear_apply_kernel<D, true> : bilinear_apply_kernel<D, false>;                    \
+        static int smem_set[2][HSR_MAX_DEVICES];                                                                     \
+        HSR_CUDA(ensure_dynamic_smem(kern, smem, smem_set[x_stretch ? 1 : 0]));                                      \
+        int per_sm = 0;                                                                                              \
+        HSR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, FINE_THREADS, smem));                  \
+        const long long cap = (long long)device_sm_count() * (per_sm > 0 ? per_sm : 1);                             \
+        kern<<<(unsigned int)(want < cap ? want : cap), FINE_THREADS, smem, stream>>>(P);                            \
+    }
     HSR_DEG_SWITCH(deg, CALL)
 #undef CALL
     HSR_CUDA(cudaGetLastError());

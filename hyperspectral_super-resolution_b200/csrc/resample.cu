@@ -81,7 +81,7 @@ namespace {
 // Resampling.bilinear, cell 73; s2_emit/poly_regression.py:150-156): the destination pixel centre
 // ((x + 0.5) / factor - 0.5 in source pixel coordinates) is interpolated from its 2 x 2 source neighbours; neighbours
 // outside the source, equal to nodata or NaN are skipped and the weights renormalised (GDAL's 4-sample bilinear
-// kernel), none usable -> 0.  fp64 weights, fp32 result.
+// kernel), none usable -> 0.  fp64 weights, fp32 result (bilinear_up_tap / bilinear_up_value of hsr_common.cuh).
 __global__ void __launch_bounds__(256) bilinear_up_kernel(const float* __restrict__ src, long long src_plane_stride,
                                                           long long Hs, long long Ws, int factor, int has_nodata,
                                                           float nodata, float* __restrict__ dst,
@@ -92,28 +92,7 @@ __global__ void __launch_bounds__(256) bilinear_up_kernel(const float* __restric
     const long long Hd = Hs * factor, Wd = Ws * factor, n = Hd * Wd;
     for (long long o = blockIdx.x * (long long)blockDim.x + threadIdx.x; o < n; o += (long long)gridDim.x * blockDim.x) {
         const long long y = o / Wd, x = o - y * Wd;
-        const double sy = ((double)y + 0.5) / factor - 0.5, sx = ((double)x + 0.5) / factor - 0.5;
-        const double fy = floor(sy), fx = floor(sx);
-        const long long y0 = (long long)fy, x0 = (long long)fx;
-        const double wy1 = sy - fy, wx1 = sx - fx;
-        double acc = 0.0, wsum = 0.0;
-#pragma unroll
-        for (int dy = 0; dy < 2; ++dy) {
-            const long long yy = y0 + dy;
-            const double wy = dy ? wy1 : 1.0 - wy1;
-            if (yy < 0 || yy >= Hs) continue;
-#pragma unroll
-            for (int dx = 0; dx < 2; ++dx) {
-                const long long xx = x0 + dx;
-                const double w = wy * (dx ? wx1 : 1.0 - wx1);
-                if (xx < 0 || xx >= Ws || w == 0.0) continue;
-                const float v = __ldg(sp + yy * Ws + xx);
-                if ((has_nodata && v == nodata) || v != v) continue;
-                acc += w * (double)v;
-                wsum += w;
-            }
-        }
-        dp[o] = wsum > 0.0 ? (float)(acc / wsum) : 0.f;
+        dp[o] = bilinear_up_value(sp, Hs, Ws, bilinear_up_tap(y, x, factor), has_nodata, nodata);
     }
 }
 
@@ -132,6 +111,62 @@ int bilinear_upsample_impl(const float* src, int C, long long Hs, long long Ws, 
     dim3 grid((unsigned int)(blocks < cap ? blocks : cap), (unsigned int)C);
     bilinear_up_kernel<<<grid, 256, 0, stream>>>(src, src_plane_stride, Hs, Ws, factor, has_nodata, nodata, dst,
                                                  dst_plane_stride);
+    HSR_CUDA(cudaGetLastError());
+    return HSR_OK;
+}
+
+namespace {
+
+// mask10 of s2_emit/poly_regression.py:159: mask[i] = all_k isfinite(bilinear x factor of plane k at fine pixel i),
+// computed from the source planes without writing the fine planes.  One thread per 4 fine pixels of the flat index.
+__global__ void __launch_bounds__(256) bilinear_fine_mask_kernel(const float* __restrict__ src, int K,
+                                                                 long long src_plane_stride, long long Hs,
+                                                                 long long Ws, int factor, uint8_t* __restrict__ mask,
+                                                                 int vecm) {
+    const long long Wd = Ws * factor, n = Hs * factor * Wd, n4 = (n + 3) >> 2;
+    for (long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x; q < n4; q += (long long)gridDim.x * blockDim.x) {
+        const long long i = q << 2;
+        long long y = i / Wd, x = i - y * Wd;
+        BilinearTap t[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            t[j] = bilinear_up_tap(y, x, factor);
+            next_pixel(y, x, Wd);
+        }
+        unsigned int m = 0u;
+#pragma unroll
+        for (int j = 0; j < 4; ++j) m |= (i + j < n ? 1u : 0u) << j;
+        for (int k = 0; k < K; ++k) {
+            const float* sp = src + (long long)k * src_plane_stride;
+#pragma unroll
+            for (int j = 0; j < 4; ++j)
+                if (((m >> j) & 1u) && !finite_f32(bilinear_up_value(sp, Hs, Ws, t[j], 0, 0.f))) m &= ~(1u << j);
+        }
+        if (vecm && i + 4 <= n) {
+            *reinterpret_cast<uchar4*>(mask + i) = make_uchar4(m & 1u, (m >> 1) & 1u, (m >> 2) & 1u, (m >> 3) & 1u);
+        } else {
+            for (int j = 0; j < 4; ++j)
+                if (i + j < n) mask[i + j] = (m >> j) & 1u;
+        }
+    }
+}
+
+}  // namespace
+
+int bilinear_fine_mask_impl(const float* src, int K, long long Hs, long long Ws, long long src_plane_stride, int factor,
+                            uint8_t* mask, cudaStream_t stream) {
+    HSR_REQUIRE(src && mask, HSR_EINVAL, "null src / mask pointer");
+    HSR_REQUIRE(K >= 1 && K <= HSR_MAX_SRF_BANDS && Hs >= 0 && Ws >= 0 && factor >= 1, HSR_EINVAL,
+                "bad K = %d (1..%d), shape or factor", K, HSR_MAX_SRF_BANDS);
+    HSR_REQUIRE(src_plane_stride >= Hs * Ws, HSR_EINVAL, "plane stride too small");
+    HSR_REQUIRE((reinterpret_cast<uintptr_t>(src) & 3) == 0, HSR_EALIGN, "src not 4-byte aligned");
+    if (Hs == 0 || Ws == 0) return HSR_OK;
+    const long long n4 = (Hs * Ws * factor * factor + 3) / 4;
+    long long blocks = (n4 + 255) / 256;
+    const long long cap = (long long)device_sm_count() * 8;
+    const int vecm = (reinterpret_cast<uintptr_t>(mask) & 3) == 0 ? 1 : 0;
+    bilinear_fine_mask_kernel<<<(unsigned int)(blocks < cap ? blocks : cap), 256, 0, stream>>>(
+        src, K, K > 1 ? src_plane_stride : Hs * Ws, Hs, Ws, factor, mask, vecm);
     HSR_CUDA(cudaGetLastError());
     return HSR_OK;
 }

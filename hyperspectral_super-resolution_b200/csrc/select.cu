@@ -612,13 +612,18 @@ struct UnionCountParams {
     UnionSeries* ser;
     unsigned long long* hu;
     double* hf;
+    long long Hs, Ws;       // UNI_SRC_BILINEAR: x[0] holds K coarse planes [Hs, Ws] (plane stride xks[0]); sample i of
+    int factor;             // series k is fine pixel i of bilinear x factor of plane k (n = Hs * Ws * factor^2)
 };
+
+constexpr int UNI_SRC_PLANES = 0;     // the samples are stored planes
+constexpr int UNI_SRC_BILINEAR = 1;   // the samples are computed from coarse planes (bilinear_up_value)
 
 // One streaming pass over one unit's planes: blockIdx.y = series.  Image data in [0, 1] has a handful of distinct top
 // bytes, so a shared-memory atomic per sample would serialise on a few bins: the lanes of a warp that add to the same bin
 // are grouped with __match_any_sync and their leader adds them with one atomic.
-// NR: histograms per series of this pass (1 in pass 0, 2Q after it).
-template <int NR>
+// NR: histograms per series of this pass (1 in pass 0, 2Q after it); SRC: where the samples come from.
+template <int NR, int SRC = UNI_SRC_PLANES>
 __global__ void __launch_bounds__(UNI_THREADS) union_count_kernel(const UnionCountParams P) {
     __shared__ unsigned int h[NR][256];
     __shared__ unsigned int pre_s[NR];
@@ -653,7 +658,39 @@ __global__ void __launch_bounds__(UNI_THREADS) union_count_kernel(const UnionCou
             if (hit && lane == __ffs(peers) - 1) atomicAdd(&h[r][digit], (unsigned int)__popc(peers));
         }
     };
-    if (live) {
+    if (SRC == UNI_SRC_BILINEAR && live) {
+        // 4 consecutive fine pixels per lane; the fine value is only formed where the mask wants the sample
+        const long long n = P.n, n4 = (n + 3) >> 2, Wd = P.Ws * P.factor;
+        const long long gtid = (long long)blockIdx.x * UNI_THREADS + tid;
+        const long long nthreads = (long long)gridDim.x * UNI_THREADS;
+        const bool vm = (reinterpret_cast<uintptr_t>(P.mask) & 3) == 0;
+        for (long long q0 = gtid - lane; q0 < n4; q0 += nthreads) {
+            const long long q = q0 + lane, i = q << 2;
+            unsigned int m = 0u;
+            if (q < n4) {
+                if (P.mask == nullptr) {
+                    m = i + 4 <= n ? 0xfu : (1u << (n - i)) - 1u;
+                } else if (vm && i + 4 <= n) {
+                    const unsigned int w = __ldg(reinterpret_cast<const unsigned int*>(P.mask + i));
+                    m = ((w & 0xffu) ? 1u : 0u) | ((w & 0xff00u) ? 2u : 0u) | ((w & 0xff0000u) ? 4u : 0u) |
+                        ((w & 0xff000000u) ? 8u : 0u);
+                } else {
+                    for (int j = 0; j < 4; ++j)
+                        if (i + j < n && P.mask[i + j]) m |= 1u << j;
+                }
+            }
+            if (__ballot_sync(0xffffffffu, m != 0u) == 0u) continue;   // 128 unmasked samples: skipped whole
+            long long y = i / Wd, x = i - y * Wd;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+                const bool use = (m >> j) & 1u;
+                const float v = use ? bilinear_up_value(xs, P.Hs, P.Ws, bilinear_up_tap(y, x, P.factor), 0, 0.f) : 0.f;
+                add(v, use);
+                next_pixel(y, x, Wd);
+            }
+        }
+    }
+    if (SRC == UNI_SRC_PLANES && live) {
         const long long n = P.n;
         const long long gtid = (long long)blockIdx.x * UNI_THREADS + tid;
         const long long nthreads = (long long)gridDim.x * UNI_THREADS;
@@ -1110,6 +1147,40 @@ int union_count_impl(const float* x, long long xks, const float* y, long long yk
     if (pass == 0) union_count_kernel<1><<<grid, UNI_THREADS, 0, stream>>>(P);
     else if (Q == 1) union_count_kernel<2><<<grid, UNI_THREADS, 0, stream>>>(P);
     else union_count_kernel<2 * SEL_QMAX><<<grid, UNI_THREADS, 0, stream>>>(P);
+    HSR_CUDA(cudaGetLastError());
+    return HSR_OK;
+}
+
+int union_count_bilinear_impl(const float* src, long long src_plane_stride, long long Hs, long long Ws, int factor,
+                              const uint8_t* mask, int K, int Q, int pass, void* state, double* hist,
+                              cudaStream_t stream) {
+    HSR_REQUIRE(state && hist, HSR_EINVAL, "null state / hist pointer");
+    HSR_REQUIRE(Hs >= 0 && Ws >= 0 && factor >= 1 && src_plane_stride >= Hs * Ws, HSR_EINVAL,
+                "bad shape, factor = %d or plane stride", factor);
+    // n < 2^32 per unit, as for stored planes (checked before the product can overflow)
+    HSR_REQUIRE((double)Hs * (double)Ws * (double)factor * (double)factor < 4294967296.0, HSR_ERANGE,
+                "factor^2 * Hs * Ws = %.0f fine samples: a unit holds fewer than 2^32",
+                (double)Hs * (double)Ws * (double)factor * (double)factor);
+    const long long n = Hs * Ws * factor * factor;
+    HSR_REQUIRE(K >= 1 && union_args_ok(Q, K), HSR_ERANGE, "bad K = %d or Q = %d", K, Q);
+    HSR_REQUIRE(pass >= 0 && pass <= 3, HSR_ERANGE, "pass = %d outside [0, 3]", pass);
+    HSR_REQUIRE((reinterpret_cast<uintptr_t>(src) & 3) == 0, HSR_EALIGN, "src not 4-byte aligned");
+    HSR_REQUIRE((reinterpret_cast<uintptr_t>(state) & 255) == 0, HSR_EALIGN, "state not 256-byte aligned");
+    if (n == 0) return HSR_OK;
+    HSR_REQUIRE(src, HSR_EINVAL, "null src pointer");
+    const UnionState us = union_state(state, K);
+    UnionCountParams P{};
+    P.x[0] = src, P.xks[0] = K > 1 ? src_plane_stride : Hs * Ws;
+    P.mask = mask, P.n = n, P.K = K, P.S = K, P.Q = Q, P.pass = pass;
+    P.ser = us.ser, P.hu = us.hu, P.hf = hist;
+    P.Hs = Hs, P.Ws = Ws, P.factor = factor;
+    long long per = (n + (long long)UNI_THREADS * 4 - 1) / ((long long)UNI_THREADS * 4);
+    long long cap = (long long)device_sm_count() * 8 / K;
+    if (cap < 1) cap = 1;
+    const dim3 grid((unsigned int)(per < cap ? per : cap), (unsigned int)K);
+    if (pass == 0) union_count_kernel<1, UNI_SRC_BILINEAR><<<grid, UNI_THREADS, 0, stream>>>(P);
+    else if (Q == 1) union_count_kernel<2, UNI_SRC_BILINEAR><<<grid, UNI_THREADS, 0, stream>>>(P);
+    else union_count_kernel<2 * SEL_QMAX, UNI_SRC_BILINEAR><<<grid, UNI_THREADS, 0, stream>>>(P);
     HSR_CUDA(cudaGetLastError());
     return HSR_OK;
 }

@@ -665,7 +665,7 @@ def masked_percentiles(x: torch.Tensor, mask: Optional[torch.Tensor], q, *, grou
 
 
 def masked_percentiles_union(units, q, *, reduce=None, K: Optional[int] = None, pair: Optional[bool] = None,
-                             device=None, _state_out: Optional[list] = None):
+                             device=None, factor: int = 1, _state_out: Optional[list] = None):
     """``out[k, 0, j] = np.percentile(concatenation over units of x[k][mask], q[j])`` — the exact percentiles of the
     UNION of several units (granules, slabs) and, through ``reduce``, of every process's units: a radix select by four
     8-bit passes whose per-pass histograms are summed over the units and then across processes (hsr_union_select_*).
@@ -677,7 +677,12 @@ def masked_percentiles_union(units, q, *, reduce=None, K: Optional[int] = None, 
     in place across processes, called once per pass; default ``dist.allreduce_moments`` on the default group (a no-op
     for one process).  Every process must make the call.  Returns [K, 1, Q] f64 (a pair for ``(x, y, mask)`` units;
     NaN where the union has no sample or a NaN among them).  ``_state_out``: diagnostics (tests) — receives the
-    per-series select state after the last pass."""
+    per-series select state after the last pass.
+
+    ``factor > 1``: the samples of every unit's x planes [K, Hs, Ws] are those of ``bilinear_upsample(x, factor)``
+    (same bits), formed on the fly from the coarse planes in each pass and never written
+    (hsr_union_select_count_bilinear); the mask then has the fine shape [Hs*factor, Ws*factor], units are ``(x, mask)``
+    and ``pair`` must be False."""
     from . import dist as hdist
 
     units = [tuple(u) for u in units]
@@ -691,6 +696,9 @@ def masked_percentiles_union(units, q, *, reduce=None, K: Optional[int] = None, 
     elif K is None or pair is None or device is None:
         raise ValueError("an empty unit list needs K=, pair= and device=")
     K, pair, device = int(K), bool(pair), torch.device(device)
+    f = _factor(factor)
+    if f > 1 and pair:
+        raise ValueError("factor > 1 takes (x, mask) units only (pair=False)")
     qf = _percentile_fractions(q)
     Q, S = int(qf.size), K * (2 if pair else 1)
     prepared = []
@@ -698,8 +706,12 @@ def masked_percentiles_union(units, q, *, reduce=None, K: Optional[int] = None, 
         x, y, mask = (u[0], u[1], u[2]) if pair else (u[0], None, u[1])
         if int(x.shape[0]) != K or x.device != device:
             raise ValueError(f"every unit must hold K = {K} planes on {device}")
-        n = x.numel() // max(K, 1)
-        xv, xks, _ = _grouped(x, "x", K, 1, n)
+        if f > 1:
+            xv, _, Hs, Ws, xks = _coarse_planes(x, "x")
+            n = Hs * Ws * f * f
+        else:
+            n = x.numel() // max(K, 1)
+            xv, xks, _ = _grouped(x, "x", K, 1, n)
         yv, yks = None, 0
         if y is not None:
             if int(y.shape[0]) != K or y.numel() != x.numel():
@@ -710,7 +722,7 @@ def masked_percentiles_union(units, q, *, reduce=None, K: Optional[int] = None, 
             m = mask.view(torch.uint8) if mask.dtype == torch.bool else mask
             m = _cuda(m, "mask", torch.uint8).contiguous()
             if m.numel() != n:
-                raise ValueError("mask must have one entry per sample")
+                raise ValueError("mask must have one entry per sample" + (" of the fine grid" if f > 1 else ""))
         prepared.append((xv, xks, yv, yks, m, n))
     reduce = reduce if reduce is not None else hdist.allreduce_moments
     lib = _lib.lib()
@@ -723,6 +735,10 @@ def masked_percentiles_union(units, q, *, reduce=None, K: Optional[int] = None, 
         more, p = ctypes.c_int(1), 0
         while more.value:
             for xv, xks, yv, yks, m, n in prepared:
+                if f > 1:
+                    _lib.check(lib.hsr_union_select_count_bilinear(xv.data_ptr(), xks, xv.shape[1], xv.shape[2], f, _ptr(m),
+                                                                   K, Q, p, sp, hist.data_ptr(), _stream()))
+                    continue
                 _lib.check(lib.hsr_union_select_count(xv.data_ptr(), xks, _ptr(yv), yks, _ptr(m), n, K, Q, p, sp,
                                                       hist.data_ptr(), _stream()))
             reduce(hist)
@@ -1091,6 +1107,77 @@ def bilinear_upsample(src: torch.Tensor, factor: int, *, nodata=None, out: Optio
                                                         int(nodata is not None), 0.0 if nodata is None else float(nodata),
                                                         out.data_ptr(), max(ps, Hs * f * Ws * f), _stream()))
     return out
+
+
+def _coarse_planes(src: torch.Tensor, name: str = "src"):
+    """(planes, K, Hs, Ws, plane stride) of [K, Hs, Ws] f32 CUDA planes whose every plane is dense."""
+    s = _cuda(src, name, torch.float32)
+    if s.dim() != 3:
+        raise ValueError(f"{name} must be [K, Hs, Ws], got shape {tuple(s.shape)}")
+    if not (s[0].is_contiguous() and (s.shape[0] == 1 or s.stride(0) >= s[0].numel())):
+        s = s.contiguous()
+    K, Hs, Ws = (int(d) for d in s.shape)
+    if not 1 <= K <= _lib.HSR_MAX_SRF_BANDS:
+        raise ValueError(f"{name} must hold 1..{_lib.HSR_MAX_SRF_BANDS} planes, got {K}")
+    return s, K, Hs, Ws, int(s.stride(0)) if K > 1 else Hs * Ws
+
+
+def _factor(factor) -> int:
+    f = int(factor)
+    if f < 1 or f != factor:
+        raise ValueError(f"factor must be an integer >= 1, got {factor!r}")
+    return f
+
+
+def bilinear_fine_mask(src: torch.Tensor, factor: int, *, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """``mask10`` of s2_emit/poly_regression.py:159 without the fine planes: [Hs*factor, Ws*factor] bool =
+    ``isfinite(bilinear_upsample(src, factor)).all(0)`` (no nodata, no gate), from the [K, Hs, Ws] f32 planes."""
+    s, K, Hs, Ws, sps = _coarse_planes(src)
+    f = _factor(factor)
+    with torch.cuda.device_of(s):
+        if out is None:
+            out = torch.empty((Hs * f, Ws * f), dtype=torch.bool, device=s.device)
+        elif out.dtype != torch.bool or tuple(out.shape) != (Hs * f, Ws * f) or not out.is_contiguous():
+            raise ValueError(f"out must be a contiguous [{Hs * f}, {Ws * f}] bool tensor")
+        _lib.check(_lib.lib().hsr_bilinear_fine_mask_u8(s.data_ptr(), K, Hs, Ws, sps, f, _cuda(out.view(torch.uint8), "out", torch.uint8).data_ptr(),
+                                                        _stream()))
+    return out
+
+
+def bilinear_apply(src: torch.Tensor, factor: int, coeffs: torch.Tensor, *, x_stretch: Optional[torch.Tensor] = None,
+                   lo: float = 0.0, hi: float = 1.0, out: Optional[torch.Tensor] = None,
+                   mask_out: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Colour-matched planes on the ``factor``-times finer grid in one pass (s2_emit/poly_regression.py:150-162 on K
+    planes): ``x10 = bilinear_upsample(src, factor)``, ``mask10 = isfinite(x10).all(0)``, ``xs = x10`` stretched with
+    ``x_stretch`` ([K, 1, 2] f64 (lo, hi), optional) on every pixel, ``(f32) polyval_f64(coeffs[k], xs)`` where mask10,
+    then every pixel clipped to [lo, hi] (``lo > hi``: no clip).  Bit-identical to ``bilinear_upsample`` ->
+    ``fit_mask(gate_k=-1)`` -> ``poly_solve_apply`` with the moments that gave ``coeffs``; the fine intermediates are
+    never written.  Returns ``(out [K, Hs*factor, Ws*factor] f32 padded planes, mask10 [Hs*factor, Ws*factor] bool)``."""
+    s, K, Hs, Ws, sps = _coarse_planes(src)
+    f = _factor(factor)
+    co = _cuda(coeffs, "coeffs", torch.float64).contiguous()
+    if co.dim() != 2 or co.shape[0] != K or not 2 <= co.shape[1] <= _lib.HSR_MAX_POLY_DEG + 1:
+        raise ValueError(f"coeffs must be [K={K}, deg+1] with 1 <= deg <= {_lib.HSR_MAX_POLY_DEG}, got {tuple(co.shape)}")
+    deg = int(co.shape[1]) - 1
+    xst = _stretch_arg(x_stretch, K, 1, "x_stretch")
+    Hd, Wd = Hs * f, Ws * f
+    with torch.cuda.device_of(s):
+        if out is None:
+            out = alloc_planes(K, (Hd, Wd), s.device)
+        else:
+            _cuda(out, "out", torch.float32)
+            if tuple(out.shape) != (K, Hd, Wd):
+                raise ValueError(f"out must be [{K}, {Hd}, {Wd}], got {tuple(out.shape)}")
+        ops = _plane_stride(out, K, Hd * Wd, "out")
+        if mask_out is None:
+            mask_out = torch.empty((Hd, Wd), dtype=torch.bool, device=s.device)
+        elif mask_out.dtype != torch.bool or tuple(mask_out.shape) != (Hd, Wd) or not mask_out.is_contiguous():
+            raise ValueError(f"mask_out must be a contiguous [{Hd}, {Wd}] bool tensor")
+        m = _cuda(mask_out.view(torch.uint8), "mask_out", torch.uint8)
+        _lib.check(_lib.lib().hsr_bilinear_apply_f32(s.data_ptr(), K, Hs, Ws, sps, f, co.data_ptr(), deg, _ptr(xst),
+                                                     float(lo), float(hi), out.data_ptr(), max(ops, Hd * Wd),
+                                                     m.data_ptr(), _stream()))
+    return out, mask_out
 
 
 # --------------------------------------------------------------------------------------- general grid warp

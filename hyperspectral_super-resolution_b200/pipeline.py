@@ -15,6 +15,10 @@ from HBM once:
 of the K planes onto the S2 grid (``warp_planes``), then the same fit and solve / apply.  ``synthesize_sharded`` takes
 granules with an S2 target too, and ``synthesize_slab_on_s2_grid`` runs one band of target rows of a mosaic, staging only
 the ortho and raw rows that band reads.
+
+``matched_fine`` takes a result to the Sentinel-2 10 m resolution as the reference script's last step does
+(poly_regression.py:150-162): bilinear x factor of the planes, mask, the stretch with the percentiles of the fine planes
+and the 60 m polynomial — a fine mask, a union select over the fine values computed on the fly, and one fused apply.
 """
 from __future__ import annotations
 
@@ -54,6 +58,16 @@ class PairResult:
     raw_rows: Optional[tuple] = None         # synthesize_slab: the [row0, row1) raw rows that were staged
     grid: Optional[S2Target] = None          # synthesize_on_s2_grid: the S2 grid of bands / matched / valid / fit_mask
     ortho_rows: Optional[tuple] = None       # synthesize_slab_on_s2_grid: the [row0, row1) ortho rows that were staged
+
+
+@dataclass
+class FineResult:
+    matched: torch.Tensor                    # [K, f*H, f*W] f32 colour-matched planes on the finer grid (padded planes)
+    mask: torch.Tensor                       # [f*H, f*W] bool: mask10, every fine value finite
+    x_limits: Optional[torch.Tensor]         # [K, 1, 2] f64 (lo, hi) percentiles of the fine planes, None without a stretch
+    factor: int
+    s2_window: Optional[tuple] = None        # the target's s2_window x factor: (row, col) of the top-left fine pixel in
+                                             # the S2 grid at the fine resolution (None off the S2 grid)
 
 
 class PairSynthesizer:
@@ -436,6 +450,64 @@ class PairSynthesizer:
             out.append(PairResult(bands, matched, coeffs.view(self.K, self.deg + 1), valid, fm.view(valid.shape), diag,
                                   mom, None, self.band_names, xl, yl, grid=target))
         return out
+
+
+    # ------------------------------------------------------------------ the step to the finer (S2 10 m) resolution
+    def matched_fine(self, results, factor: int = 6, *, group=None, out=None):
+        """Colour-matched planes on the ``factor``-times finer aligned grid — the reference script's last step
+        (s2_emit/poly_regression.py:150-162), for the K planes of a pair result: ``x10 = bilinear x factor`` of the
+        result's (unstretched) ``bands``, ``mask10 = isfinite(x10).all(0)``, with ``stretch`` the percentiles of x10
+        under mask10 (``lim10``) and ``xs = clip((x10 - lo) / (hi - lo + 1e-12), 0, 1)`` on every pixel (else
+        ``xs = x10``), ``(f32) polyval(coeffs[k], xs)`` where mask10, then every pixel clipped to ``clip``.  On an S2
+        target grid (snapped to the S2 origin at an integer ratio) factor 6 gives the S2 10 m grid.  Fill pixels
+        (``fill_out``) are finite and therefore data here, as in the reference (DESIGN section 7).
+
+        ``results``: one ``PairResult`` -> one ``FineResult``; a sequence of the results of ONE global fit (e.g.
+        ``synthesize_sharded``, possibly empty on a rank that holds no granule) -> a list.  The 10 m limits follow the
+        60 m ones: one result has its own; several (``stretch_scope="fit"``) share the union over all of them and, with
+        ``group``, over every rank of the group — every rank must then call, also with no result.  The fine planes are
+        never materialised: a fine mask, a union select over fine values formed from the 60 m planes in each of its
+        four passes, and one fused apply (``kernels.bilinear_fine_mask``, ``kernels.masked_percentiles_union(factor=)``,
+        ``kernels.bilinear_apply``).  ``out``: a [K, f*H, f*W] f32 tensor (one result) or a list of them.
+        Raises ``ValueError`` for tile batches, row slabs (the upsample at a slab edge needs the neighbouring slab's
+        rows) and ``factor < 1``."""
+        single = isinstance(results, PairResult)
+        rs = [results] if single else list(results)
+        f = int(factor)
+        if f < 1 or f != factor:
+            raise ValueError(f"factor must be an integer >= 1, got {factor!r}")
+        for r in rs:
+            if r.coeffs.dim() != 2 or r.bands.dim() != 3:
+                raise ValueError("matched_fine takes granule results: tile batches (coeffs [K, T, deg+1]) are not covered")
+            if r.raw_rows is not None or r.ortho_rows is not None:
+                raise ValueError("matched_fine does not take row slabs: the upsample at a slab edge needs the "
+                                 "neighbouring slab's rows")
+        outs = [out] if single else (list(out) if out is not None else [None] * len(rs))
+        if len(outs) != len(rs):
+            raise ValueError(f"out holds {len(outs)} tensors for {len(rs)} results")
+        with torch.cuda.device(self.device):
+            # the select needs mask10 before the apply; without a stretch the apply writes it
+            masks = [kernels.bilinear_fine_mask(r.bands, f) if self.stretch is not None else
+                     torch.empty((r.bands.shape[1] * f, r.bands.shape[2] * f), dtype=torch.bool, device=self.device)
+                     for r in rs]
+            xl = None
+            if self.stretch is not None:
+                world = hdist.group_size(group) if group is not None else 1
+                if len(rs) > 1 or world > 1:
+                    self._no_global_stretch("matched_fine over several results / ranks")
+                reduce = self._global_reduce(group) if group is not None else None
+                xl = kernels.masked_percentiles_union([(r.bands, m) for r, m in zip(rs, masks)], self.stretch,
+                                                      reduce=reduce or _no_reduce, K=self.K, pair=False,
+                                                      device=self.device, factor=f)
+            lo, hi = self.clip if self.clip is not None else (1.0, 0.0)
+            fine = []
+            for r, m, o in zip(rs, masks, outs):
+                matched, _ = kernels.bilinear_apply(r.bands, f, r.coeffs, x_stretch=xl, lo=lo, hi=hi, out=o, mask_out=m)
+                win = None
+                if r.grid is not None:
+                    win = (int(r.grid.s2_window[0]) * f, int(r.grid.s2_window[1]) * f)
+                fine.append(FineResult(matched, m, xl, f, win))
+        return fine[0] if single else fine
 
 
 def _as_tensor(raw):

@@ -383,6 +383,19 @@ HSR_API int hsr_union_select_step(int Q, int S, int pass, void* state, double* h
                           void* stream);
 
 /*
+ * hsr_union_select_count_bilinear: hsr_union_select_count for a unit whose K series (x only: S = K) are the VIRTUAL
+ * planes bilinear x factor of the coarse planes src (K planes [Hs, Ws] f32, plane stride src_plane_stride): sample i of
+ * series k is fine pixel i of hsr_bilinear_upsample_f32(src[k], factor) without nodata (same bits), formed where
+ * mask[i] != 0 (mask nullable [Hs*factor, Ws*factor]) and never written.  The fine planes of s2_emit/poly_regression.py
+ * :150-161 (2 GB at 10 m for a granule) are not materialised; the 60 m planes stay in L2 across the four passes.
+ * factor^2 * Hs * Ws < 2^32 (HSR_ERANGE otherwise).  Takes the place of hsr_union_select_count in the sequence above;
+ * begin, step and the all-reduce are unchanged, and units of both kinds may be counted into one select.
+ */
+HSR_API int hsr_union_select_count_bilinear(const float* src, int64_t src_plane_stride, int64_t Hs, int64_t Ws,
+                                    int factor, const uint8_t* mask, int K, int Q, int pass, void* state,
+                                    double* hist, void* stream);
+
+/*
  * Optimal-transport targets of fit_ot_poly_rgb, s2_emit/poly_regression.py:31-60.  POT (`import ot`) is an
  * un-vendored, un-pinned dependency of the reference; these entry points follow its published algorithms
  * (ot.dist "sqeuclidean" = |x|^2 + |y|^2 - 2 x.y clamped at 0; ot.sinkhorn = sinkhorn_knopp), all in fp64.
@@ -475,6 +488,25 @@ HSR_API int hsr_block_average_f32(const void* src, int src_dtype, int C, int64_t
  */
 HSR_API int hsr_bilinear_upsample_f32(const float* src, int C, int64_t Hs, int64_t Ws, int64_t src_plane_stride, int factor,
                               int has_nodata, float nodata, float* dst, int64_t dst_plane_stride, void* stream);
+
+/*
+ * Colour-matched planes at the finer resolution, s2_emit/poly_regression.py:150-162 on K planes, without the fine
+ * intermediates.  src: K <= HSR_MAX_SRF_BANDS coarse planes [Hs, Ws] f32 (plane stride src_plane_stride); fine pixel i
+ * of plane k is x10[k][i] = hsr_bilinear_upsample_f32(src[k], factor) without nodata (same bits).
+ * hsr_bilinear_fine_mask_u8: mask [Hs*factor, Ws*factor] u8 = all_k isfinite(x10[k]) (hsr_fit_mask_u8 with no gate).
+ * hsr_bilinear_apply_f32:    dst[k] = xs = x10[k], stretched first with x_stretch (nullable [K][2] f64 (lo, hi), the
+ *                            on-the-fly stretch of hsr_poly_solve_apply_f32) on every pixel; where mask10:
+ *                            (f32) polyval_f64(coeffs[k], xs) (coeffs [K, deg+1] f64, highest power first); then every
+ *                            pixel clipped to [lo, hi] (lo > hi: no clip).  Bit-identical to hsr_bilinear_upsample_f32
+ *                            -> hsr_fit_mask_u8 (gate_k < 0) -> hsr_poly_solve_apply_f32 with the moments that gave
+ *                            coeffs.  dst: K planes of Hs*factor*Ws*factor, plane stride dst_plane_stride (16-byte
+ *                            stores where dst and the stride allow); mask_out nullable: receives mask10.
+ */
+HSR_API int hsr_bilinear_fine_mask_u8(const float* src, int K, int64_t Hs, int64_t Ws, int64_t src_plane_stride,
+                              int factor, uint8_t* mask, void* stream);
+HSR_API int hsr_bilinear_apply_f32(const float* src, int K, int64_t Hs, int64_t Ws, int64_t src_plane_stride,
+                           int factor, const double* coeffs, int deg, const double* x_stretch, float lo, float hi,
+                           float* dst, int64_t dst_plane_stride, uint8_t* mask_out, void* stream);
 
 /*
  * robust_norm / robust_norm_rgb of s2_emit/color.py:6-23, whose results are float64:
