@@ -124,6 +124,10 @@ SIGNATURES = {
     "hsr_sinkhorn_workspace_bytes": (_c.c_size_t, [_int, _int]),
     "hsr_sinkhorn_barycentric_f64": (_int, [_p, _p, _int, _int, _int, _c.c_double, _int, _c.c_double, _p, _p, _p, _p]),
     "hsr_polyfit_moments_f64in": (_int, [_p, _p, _i64, _int, _int, _p, _p]),
+    "hsr_compact_planes_pair_workspace_bytes": (_c.c_size_t, [_i64]),
+    "hsr_compact_planes_pair": (_int, [_p, _i64, _p, _p, _i64, _p, _p, _i64, _int, _p, _p, _p, _p, _p, _p]),
+    "hsr_gather_planes_f64": (_int, [_p, _i64, _int, _p, _p, _p, _i64, _p, _p, _p]),
+    "hsr_sinkhorn_barycentric_k_f64": (_int, [_p, _p, _int, _int, _int, _c.c_double, _int, _c.c_double, _p, _p, _p, _p]),
     "hsr_black_mask_f32": (_int, [_p, _i64, _i64, _i64, _int, _int, _int, _f32, _f32, _f32, _f32, _f32, _p, _p, _p]),
     "hsr_quantize_u16_f32": (_int, [_p, _i64, _int, _f32, _f32, _int, _p, _p]),
     "hsr_tile_sums_u8": (_int, [_p, _i64, _i64, _int, _int, _int, _int, _p, _p]),

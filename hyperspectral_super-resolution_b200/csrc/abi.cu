@@ -138,6 +138,13 @@ int gather_rows_impl(const float*, const int*, const long long*, long long, int,
 size_t sinkhorn_workspace(int ns, int nt);
 int sinkhorn_barycentric_impl(const double*, const double*, int, int, int, double, int, double, void*, double*, double*,
                               cudaStream_t);
+size_t compact_planes_pair_workspace(long long n);
+int compact_planes_pair_impl(const float*, long long, const double*, const float*, long long, const double*,
+                             const uint8_t*, long long, int, void*, int*, long long*, int*, long long*, cudaStream_t);
+int gather_planes_impl(const float*, long long, int, const int*, const long long*, const long long*, long long,
+                       const double*, double*, cudaStream_t);
+int sinkhorn_barycentric_k_impl(const double*, const double*, int, int, int, double, int, double, void*, double*,
+                                double*, cudaStream_t);
 int polyfit_f64_moments_impl(const double*, const double*, long long, int, int, double*, cudaStream_t);
 
 int black_mask_impl(const float*, long long, long long, long long, int, int, int, float, float, float, float, float,
@@ -314,6 +321,30 @@ int hsr_sinkhorn_barycentric_f64(const double* X, const double* Y, int ns, int n
                                  double stop_thr, void* workspace, double* ybar, double* info, void* stream) {
     return hsr::sinkhorn_barycentric_impl(X, Y, ns, nt, C, reg, num_iter_max, stop_thr, workspace, ybar, info,
                                           (cudaStream_t)stream);
+}
+
+size_t hsr_compact_planes_pair_workspace_bytes(int64_t n) { return hsr::compact_planes_pair_workspace(n); }
+
+int hsr_compact_planes_pair(const float* x, int64_t x_plane_stride, const double* x_stretch, const float* y,
+                            int64_t y_plane_stride, const double* y_stretch, const uint8_t* mask, int64_t n, int K,
+                            void* workspace, int32_t* idx_x, int64_t* count_x, int32_t* idx_y, int64_t* count_y,
+                            void* stream) {
+    return hsr::compact_planes_pair_impl(x, x_plane_stride, x_stretch, y, y_plane_stride, y_stretch, mask, n, K, workspace,
+                                         idx_x, reinterpret_cast<long long*>(count_x), idx_y,
+                                         reinterpret_cast<long long*>(count_y), (cudaStream_t)stream);
+}
+
+int hsr_gather_planes_f64(const float* planes, int64_t plane_stride, int K, const int32_t* idx, const int64_t* sel,
+                          const int64_t* dst, int64_t ns, const double* stretch, double* out, void* stream) {
+    return hsr::gather_planes_impl(planes, plane_stride, K, idx, reinterpret_cast<const long long*>(sel),
+                                   reinterpret_cast<const long long*>(dst), ns, stretch, out, (cudaStream_t)stream);
+}
+
+int hsr_sinkhorn_barycentric_k_f64(const double* X, const double* Y, int ns, int nt, int C, double reg,
+                                   int num_iter_max, double stop_thr, void* workspace, double* ybar, double* info,
+                                   void* stream) {
+    return hsr::sinkhorn_barycentric_k_impl(X, Y, ns, nt, C, reg, num_iter_max, stop_thr, workspace, ybar, info,
+                                            (cudaStream_t)stream);
 }
 
 int hsr_polyfit_moments_f64in(const double* x, const double* y, int64_t n, int S, int deg, double* moments,

@@ -26,6 +26,7 @@ namespace hsr {
 namespace {
 
 constexpr int OT_MAXC = 4;       // channels per sample (RGB = 3)
+constexpr int OT_MAXC_WIDE = HSR_MAX_SRF_BANDS;   // hsr_sinkhorn_barycentric_k_f64: the K planes of a pair synthesis
 constexpr int COL_THREADS = 128;
 constexpr int OT_PARTS_MAX = 160;   // column-pass partial rows: <= 32 chunks, or one per SM in the fused kernel
 
@@ -116,24 +117,153 @@ __global__ void gather_rows_kernel(const float* __restrict__ img, const int* __r
     out[t] = (double)__ldg(img + (long long)idx[sel[r]] * C + c);
 }
 
+// ---------------------------------------------------------------------------------- planar pair compaction / gather
+// The pair pipeline holds its samples as K planes (plane k at p + k * ks, any stride >= n: padded or dense) for both
+// the synthesised bands X and the reference Y, under one fit mask.  X rows and Y rows are filtered independently
+// (:33-36), so one pass over the mask and both plane sets yields two index lists.  With a stretch ([K][2] (lo, hi)) a
+// row is judged on its stretched values, as fit_ot_poly_rgb judges the stretched image it is handed.
+struct PlanePair {
+    const float* x;
+    long long xks;
+    const double* xst;  // nullable [K][2]
+    const float* y;
+    long long yks;
+    const double* yst;
+    const uint8_t* mask;  // nullable
+    long long n;
+    int K;
+};
+
+// color.py:33 with the true fp64 division of hsr_stretch_f32 (stretch_kernel in select.cu), so that a stretched
+// sample carries the bits of the stretched plane
+__device__ __forceinline__ float stretch_exact(float v, const double* __restrict__ st, int k) {
+    const double lo = __ldg(st + 2 * k), den = __ldg(st + 2 * k + 1) - lo + 1e-12;
+    double r = ((double)v - lo) / den;
+    r = r < 0.0 ? 0.0 : (r > 1.0 ? 1.0 : r);  // NaN survives, as np.clip
+    return (float)r;
+}
+
+// Whether stretch_exact(v) is finite: the clip maps +-Inf into [0, 1], so only a NaN quotient is not, and IEEE
+// division gives NaN exactly for NaN operands, Inf / Inf and 0 / 0 — decided without the division (whose slow path is
+// a call that would spill in the compaction kernels).
+__device__ __forceinline__ bool stretched_finite(float v, const double* __restrict__ st, int k) {
+    const double lo = __ldg(st + 2 * k), den = __ldg(st + 2 * k + 1) - lo + 1e-12;
+    const double a = (double)v - lo;
+    return !(isnan(a) || isnan(den) || (isinf(a) && isinf(den)) || (a == 0.0 && den == 0.0));
+}
+
+__device__ __forceinline__ bool planes_row_finite(const float* __restrict__ p, long long ks, const double* __restrict__ st,
+                                                  int K, long long i) {
+    bool f = true;
+    for (int k = 0; k < K; ++k) {
+        const float v = __ldg(p + k * ks + i);
+        f = f && (st ? stretched_finite(v, st, k) : finite_f32(v));
+    }
+    return f;
+}
+
+__global__ void __launch_bounds__(256) compact_pair_count_kernel(const PlanePair P, int rows_per_block,
+                                                                 unsigned int* __restrict__ count_x,
+                                                                 unsigned int* __restrict__ count_y) {
+    const long long r0 = (long long)blockIdx.x * rows_per_block;
+    unsigned int cx = 0, cy = 0;
+    for (long long i = r0 + threadIdx.x; i < r0 + rows_per_block && i < P.n; i += 256) {
+        const bool m = P.mask == nullptr || P.mask[i] != 0;
+        cx += (m && planes_row_finite(P.x, P.xks, P.xst, P.K, i)) ? 1u : 0u;
+        cy += (m && planes_row_finite(P.y, P.yks, P.yst, P.K, i)) ? 1u : 0u;
+    }
+    __shared__ unsigned int red[2][8];
+    cx = (unsigned int)warp_sum((int)cx);
+    cy = (unsigned int)warp_sum((int)cy);
+    if ((threadIdx.x & 31) == 0) red[0][threadIdx.x >> 5] = cx, red[1][threadIdx.x >> 5] = cy;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned int tx = 0, ty = 0;
+        for (int w = 0; w < 8; ++w) tx += red[0][w], ty += red[1][w];
+        count_x[blockIdx.x] = tx;
+        count_y[blockIdx.x] = ty;
+    }
+}
+
+__global__ void __launch_bounds__(256) compact_pair_scatter_kernel(const PlanePair P, int rows_per_block,
+                                                                   const long long* __restrict__ base_x,
+                                                                   const long long* __restrict__ base_y,
+                                                                   int* __restrict__ idx_x, int* __restrict__ idx_y) {
+    __shared__ unsigned int wcount[2][8];
+    __shared__ long long base_s[2];
+    const long long r0 = (long long)blockIdx.x * rows_per_block;
+    if (threadIdx.x == 0) base_s[0] = base_x[blockIdx.x], base_s[1] = base_y[blockIdx.x];
+    __syncthreads();
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    for (long long s0 = r0; s0 < r0 + rows_per_block && s0 < P.n; s0 += 256) {
+        const long long i = s0 + threadIdx.x;
+        const bool m = i < P.n && i < r0 + rows_per_block && (P.mask == nullptr || P.mask[i] != 0);
+        const bool fx = m && planes_row_finite(P.x, P.xks, P.xst, P.K, i);
+        const bool fy = m && planes_row_finite(P.y, P.yks, P.yst, P.K, i);
+        const unsigned int bx = __ballot_sync(0xffffffffu, fx), by = __ballot_sync(0xffffffffu, fy);
+        if (lane == 0) wcount[0][warp] = __popc(bx), wcount[1][warp] = __popc(by);
+        __syncthreads();
+        long long ox = base_s[0], oy = base_s[1];
+        for (int w = 0; w < warp; ++w) ox += wcount[0][w], oy += wcount[1][w];
+        const unsigned int below = (1u << lane) - 1u;
+        if (fx) idx_x[ox + __popc(bx & below)] = (int)i;
+        if (fy) idx_y[oy + __popc(by & below)] = (int)i;
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            unsigned int tx = 0, ty = 0;
+            for (int w = 0; w < 8; ++w) tx += wcount[0][w], ty += wcount[1][w];
+            base_s[0] += tx;
+            base_s[1] += ty;
+        }
+        __syncthreads();
+    }
+}
+
+// out[dst[r], k] = (f64) stretch(planes[k, idx[sel[r]]])   (dst nullable: row r) — the union's sample rows, each
+// rank writing the rows it owns into a buffer the caller prefilled
+__global__ void gather_planes_kernel(const float* __restrict__ planes, long long ks, int K, const int* __restrict__ idx,
+                                     const long long* __restrict__ sel, const long long* __restrict__ dst, long long ns,
+                                     const double* __restrict__ st, double* __restrict__ out) {
+    const long long t = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (t >= ns * K) return;
+    const long long r = t / K;
+    const int k = (int)(t - r * K);
+    float v = __ldg(planes + k * ks + idx[sel[r]]);
+    if (st) v = stretch_exact(v, st, k);
+    out[(dst ? dst[r] : r) * K + k] = (double)v;
+}
+
 // ---------------------------------------------------------------------------------- Sinkhorn
+// Channel loops of the two Sinkhorn kernels that depend on C.  The narrow cap (OT_MAXC, the C <= 4 entry) runs them to
+// the runtime C, as it always has; the wide cap runs them to the cap itself with a guard, so that they unroll and the
+// per-channel arrays stay in registers (a runtime-indexed 16-entry array would live in local memory).
+template <int MAXC>
+__device__ __forceinline__ int channel_bound(int C) {
+    return MAXC > OT_MAXC ? MAXC : C;
+}
+
 // K[i, j] = exp(max(|x_i|^2 + |y_j|^2 - 2 x_i.y_j, 0) / -reg)      (ot.dist + the first line of sinkhorn_knopp)
+template <int MAXC>
 __global__ void __launch_bounds__(256) ot_kernel_matrix(const double* __restrict__ X, const double* __restrict__ Y,
                                                         int ns, int nt, int C, double reg, double* __restrict__ K) {
     const int j = blockIdx.x * 256 + threadIdx.x;
     const int i0 = blockIdx.y * 16;
     if (j >= nt) return;
-    double y[OT_MAXC], b2 = 0.0;
-    for (int c = 0; c < C; ++c) {
-        y[c] = Y[(long long)j * C + c];
-        b2 = fma(y[c], y[c], b2);
+    double y[MAXC], b2 = 0.0;
+    for (int c = 0; c < channel_bound<MAXC>(C); ++c) {
+        if (c < C) {
+            y[c] = Y[(long long)j * C + c];
+            b2 = fma(y[c], y[c], b2);
+        }
     }
     for (int i = i0; i < i0 + 16 && i < ns; ++i) {
         double a2 = 0.0, d = 0.0;
-        for (int c = 0; c < C; ++c) {
-            const double x = X[(long long)i * C + c];
-            a2 = fma(x, x, a2);
-            d = fma(x, y[c], d);
+        for (int c = 0; c < channel_bound<MAXC>(C); ++c) {
+            if (c < C) {
+                const double x = X[(long long)i * C + c];
+                a2 = fma(x, x, a2);
+                d = fma(x, y[c], d);
+            }
         }
         double m = (-2.0 * d + a2) + b2;
         m = m > 0.0 ? m : 0.0;
@@ -442,6 +572,7 @@ __global__ void ot_finish_kernel(int num_iter, OtState* st) {
 }
 
 // Ybar[i, c] = sum_j P[i, j] Y[j, c] / (sum_j P[i, j] + 1e-32),  P[i, j] = u[i] K[i, j] v[j]     (:55-56)
+template <int MAXC>
 __global__ void __launch_bounds__(256) ot_barycentric_kernel(const double* __restrict__ K, const double* __restrict__ ubuf,
                                                              const double* __restrict__ vbuf, const double* __restrict__ Y,
                                                              int ns, int nt, int C, const OtState* st,
@@ -453,18 +584,19 @@ __global__ void __launch_bounds__(256) ot_barycentric_kernel(const double* __res
     const double ui = ubuf[(long long)par * ns + row];
     const double* v = vbuf + (long long)par * nt;
     const double* kr = K + (long long)row * nt;
-    double sp = 0.0, sy[OT_MAXC];
-    for (int c = 0; c < OT_MAXC; ++c) sy[c] = 0.0;
+    double sp = 0.0, sy[MAXC];
+    for (int c = 0; c < MAXC; ++c) sy[c] = 0.0;
     for (int j = lane; j < nt; j += 32) {
         const double p = (ui * kr[j]) * v[j];
         sp += p;
-        for (int c = 0; c < OT_MAXC; ++c)
+        for (int c = 0; c < MAXC; ++c)
             if (c < C) sy[c] = fma(p, Y[(long long)j * C + c], sy[c]);
     }
     sp = warp_sum(sp);
-    for (int c = 0; c < OT_MAXC; ++c) sy[c] = warp_sum(sy[c]);
+    for (int c = 0; c < MAXC; ++c) sy[c] = warp_sum(sy[c]);
     if (lane == 0)
-        for (int c = 0; c < C; ++c) ybar[(long long)row * C + c] = sy[c] / (sp + 1e-32);
+        for (int c = 0; c < channel_bound<MAXC>(C); ++c)
+            if (c < C) ybar[(long long)row * C + c] = sy[c] / (sp + 1e-32);
 }
 
 // ---------------------------------------------------------------------------------- fp64 polyfit of the targets
@@ -554,6 +686,45 @@ int gather_rows_impl(const float* img, const int* idx, const long long* sel, lon
     return HSR_OK;
 }
 
+size_t compact_planes_pair_workspace(long long n) { return 2 * compact_workspace(n); }
+
+int compact_planes_pair_impl(const float* x, long long xks, const double* xst, const float* y, long long yks,
+                             const double* yst, const uint8_t* mask, long long n, int K, void* workspace, int* idx_x,
+                             long long* count_x, int* idx_y, long long* count_y, cudaStream_t stream) {
+    HSR_REQUIRE(((x && y) || n == 0) && workspace && idx_x && count_x && idx_y && count_y, HSR_EINVAL,
+                "null planes / workspace / idx / count pointer");
+    HSR_REQUIRE(n >= 0 && n < 2147483647LL && K >= 1 && K <= HSR_MAX_SRF_BANDS, HSR_ERANGE,
+                "bad n = %lld or K = %d (K <= %d)", n, K, HSR_MAX_SRF_BANDS);
+    HSR_REQUIRE(n == 0 || K == 1 || (xks >= n && yks >= n), HSR_EINVAL, "plane strides %lld, %lld < n = %lld", xks, yks, n);
+    HSR_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, HSR_EALIGN, "workspace not 256-byte aligned");
+    const size_t half = compact_workspace(n);
+    unsigned char* w = reinterpret_cast<unsigned char*>(workspace);
+    const int nb = (int)((n + COMPACT_ROWS - 1) / COMPACT_ROWS);
+    const size_t counts = align_up((size_t)(nb + 1) * sizeof(unsigned int), 256);
+    unsigned int* bcx = reinterpret_cast<unsigned int*>(w);
+    long long* bbx = reinterpret_cast<long long*>(w + counts);
+    unsigned int* bcy = reinterpret_cast<unsigned int*>(w + half);
+    long long* bby = reinterpret_cast<long long*>(w + half + counts);
+    const PlanePair P{x, xks, xst, y, yks, yst, mask, n, K};
+    if (nb > 0) compact_pair_count_kernel<<<nb, 256, 0, stream>>>(P, COMPACT_ROWS, bcx, bcy);
+    compact_scan_kernel<<<1, 32, 0, stream>>>(bcx, nb, bbx, count_x);
+    compact_scan_kernel<<<1, 32, 0, stream>>>(bcy, nb, bby, count_y);
+    if (nb > 0) compact_pair_scatter_kernel<<<nb, 256, 0, stream>>>(P, COMPACT_ROWS, bbx, bby, idx_x, idx_y);
+    HSR_CUDA(cudaGetLastError());
+    return HSR_OK;
+}
+
+int gather_planes_impl(const float* planes, long long ks, int K, const int* idx, const long long* sel, const long long* dst,
+                       long long ns, const double* st, double* out, cudaStream_t stream) {
+    HSR_REQUIRE(planes && idx && sel && out, HSR_EINVAL, "null planes / idx / sel / out pointer");
+    HSR_REQUIRE(ns >= 0 && K >= 1 && K <= HSR_MAX_SRF_BANDS, HSR_ERANGE, "bad ns = %lld or K = %d", ns, K);
+    if (ns == 0) return HSR_OK;
+    gather_planes_kernel<<<(unsigned int)((ns * K + 255) / 256), 256, 0, stream>>>(planes, ks, K, idx, sel, dst, ns, st,
+                                                                                 out);
+    HSR_CUDA(cudaGetLastError());
+    return HSR_OK;
+}
+
 size_t sinkhorn_workspace(int ns, int nt) {
     if (ns < 1 || nt < 1) return 0;
     size_t b = align_up(sizeof(OtState), 256);
@@ -565,10 +736,12 @@ size_t sinkhorn_workspace(int ns, int nt) {
     return b;
 }
 
-int sinkhorn_barycentric_impl(const double* X, const double* Y, int ns, int nt, int C, double reg, int num_iter_max,
-                              double stop_thr, void* workspace, double* ybar, double* info, cudaStream_t stream) {
-    HSR_REQUIRE(X && Y && workspace && ybar, HSR_EINVAL, "null X / Y / workspace / ybar pointer");
-    HSR_REQUIRE(ns >= 1 && nt >= 1 && C >= 1 && C <= OT_MAXC, HSR_ERANGE, "bad ns = %d, nt = %d or C = %d", ns, nt, C);
+namespace {
+
+// The Sinkhorn loop of both entries; only the kernel matrix and the barycentric step depend on the channel cap
+// (OT_MAXC, or OT_MAXC_WIDE for 4 < C <= 16).
+int sinkhorn_run(bool wide, const double* X, const double* Y, int ns, int nt, int C, double reg, int num_iter_max,
+                 double stop_thr, void* workspace, double* ybar, double* info, cudaStream_t stream) {
     HSR_REQUIRE(reg > 0.0 && num_iter_max >= 0, HSR_EINVAL, "reg must be > 0 and numItermax >= 0");
     HSR_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, HSR_EALIGN, "workspace not 256-byte aligned");
     unsigned char* w = reinterpret_cast<unsigned char*>(workspace);
@@ -588,7 +761,10 @@ int sinkhorn_barycentric_impl(const double* X, const double* Y, int ns, int nt, 
     const int nmax = ns > nt ? ns : nt;
     ot_init_kernel<<<(nmax + 255) / 256, 256, 0, stream>>>(u, v, ns, nt, st);
     dim3 gk((nt + 255) / 256, (ns + 15) / 16);
-    ot_kernel_matrix<<<gk, 256, 0, stream>>>(X, Y, ns, nt, C, reg, K);
+    if (wide)
+        ot_kernel_matrix<OT_MAXC_WIDE><<<gk, 256, 0, stream>>>(X, Y, ns, nt, C, reg, K);
+    else
+        ot_kernel_matrix<OT_MAXC><<<gk, 256, 0, stream>>>(X, Y, ns, nt, C, reg, K);
     const int nchunks = col_chunks(ns);
     const int rpc = (ns + nchunks - 1) / nchunks;
     dim3 gc((nt + COL_THREADS - 1) / COL_THREADS, nchunks);
@@ -667,13 +843,33 @@ int sinkhorn_barycentric_impl(const double* X, const double* Y, int ns, int nt, 
         }
     }
     ot_finish_kernel<<<1, 32, 0, stream>>>(num_iter_max, st);
-    ot_barycentric_kernel<<<(ns + 7) / 8, 256, 0, stream>>>(K, u, v, Y, ns, nt, C, st, ybar);
+    if (wide)
+        ot_barycentric_kernel<OT_MAXC_WIDE><<<(ns + 7) / 8, 256, 0, stream>>>(K, u, v, Y, ns, nt, C, st, ybar);
+    else
+        ot_barycentric_kernel<OT_MAXC><<<(ns + 7) / 8, 256, 0, stream>>>(K, u, v, Y, ns, nt, C, st, ybar);
     HSR_CUDA(cudaGetLastError());
     if (info) {  // {final iteration, last evaluated error, iteration it was evaluated at, numerical-error flag}
         ot_info_kernel<<<1, 1, 0, stream>>>(st, info);
         HSR_CUDA(cudaGetLastError());
     }
     return HSR_OK;
+}
+
+}  // namespace
+
+int sinkhorn_barycentric_impl(const double* X, const double* Y, int ns, int nt, int C, double reg, int num_iter_max,
+                              double stop_thr, void* workspace, double* ybar, double* info, cudaStream_t stream) {
+    HSR_REQUIRE(X && Y && workspace && ybar, HSR_EINVAL, "null X / Y / workspace / ybar pointer");
+    HSR_REQUIRE(ns >= 1 && nt >= 1 && C >= 1 && C <= OT_MAXC, HSR_ERANGE, "bad ns = %d, nt = %d or C = %d", ns, nt, C);
+    return sinkhorn_run(false, X, Y, ns, nt, C, reg, num_iter_max, stop_thr, workspace, ybar, info, stream);
+}
+
+int sinkhorn_barycentric_k_impl(const double* X, const double* Y, int ns, int nt, int C, double reg, int num_iter_max,
+                                double stop_thr, void* workspace, double* ybar, double* info, cudaStream_t stream) {
+    HSR_REQUIRE(X && Y && workspace && ybar, HSR_EINVAL, "null X / Y / workspace / ybar pointer");
+    HSR_REQUIRE(ns >= 1 && nt >= 1 && C >= 1 && C <= OT_MAXC_WIDE, HSR_ERANGE, "bad ns = %d, nt = %d or C = %d (C <= %d)",
+                ns, nt, C, OT_MAXC_WIDE);
+    return sinkhorn_run(C > OT_MAXC, X, Y, ns, nt, C, reg, num_iter_max, stop_thr, workspace, ybar, info, stream);
 }
 
 int polyfit_f64_moments_impl(const double* x, const double* y, long long n, int S, int deg, double* moments,

@@ -881,10 +881,77 @@ def gather_rows_f64(img: torch.Tensor, idx: torch.Tensor, sel: torch.Tensor) -> 
     return out
 
 
+def compact_planes_pair(x: torch.Tensor, y: torch.Tensor, mask: Optional[torch.Tensor], *,
+                        x_stretch: Optional[torch.Tensor] = None, y_stretch: Optional[torch.Tensor] = None):
+    """The two row filters of s2_emit/poly_regression.py:33-36 on K planes (hsr_compact_planes_pair): ``idx_x`` holds
+    the row-major indices of the pixels with ``mask`` set and all K planes of ``x`` finite, ``idx_y`` likewise for
+    ``y``, independently.  x, y: [K, ...] f32 planes (padded or dense); mask: one entry per pixel, or None;
+    ``x_stretch`` / ``y_stretch``: [K, 1, 2] f64 (lo, hi) — the planes are judged as the percentile stretch of
+    color.py:33 leaves them.  Returns ``(idx_x int32 [n], count_x int64[1], idx_y, count_y)`` on the device (the first
+    ``count`` entries of each list are valid)."""
+    xs, K, n, xks, _ = _series(x, "x", "planar")
+    ys, Ky, ny, yks, _ = _series(y, "y", "planar")
+    if (K, n) != (Ky, ny):
+        raise ValueError(f"x and y disagree: {K}x{n} vs {Ky}x{ny}")
+    m = None
+    if mask is not None:
+        m = mask.view(torch.uint8) if mask.dtype == torch.bool else mask
+        m = _cuda(m, "mask", torch.uint8).contiguous()
+        if m.numel() != n:
+            raise ValueError("mask must have one entry per pixel")
+    xst, yst = _stretch_arg(x_stretch, K, 1, "x_stretch"), _stretch_arg(y_stretch, K, 1, "y_stretch")
+    lib = _lib.lib()
+    with torch.cuda.device_of(xs):
+        work, wptr = _aligned_workspace(lib.hsr_compact_planes_pair_workspace_bytes(n), xs.device)
+        idx = torch.empty((2, max(n, 1)), dtype=torch.int32, device=xs.device)
+        count = torch.zeros(2, dtype=torch.int64, device=xs.device)
+        _lib.check(lib.hsr_compact_planes_pair(xs.data_ptr(), xks, _ptr(xst), ys.data_ptr(), yks, _ptr(yst), _ptr(m), n, K,
+                                               wptr, idx[0].data_ptr(), count[0:1].data_ptr(), idx[1].data_ptr(),
+                                               count[1:2].data_ptr(), _stream()))
+        work.record_stream(torch.cuda.current_stream())
+    return idx[0], count[0:1], idx[1], count[1:2]
+
+
+def gather_planes_f64(planes: torch.Tensor, idx: torch.Tensor, sel: torch.Tensor, *,
+                      stretch: Optional[torch.Tensor] = None, dst: Optional[torch.Tensor] = None,
+                      out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Sample rows of K planes (hsr_gather_planes_f64): ``out[dst[r], k] = float64(s(planes[k, idx[sel[r]]]))``, ``s``
+    the percentile stretch of color.py:33 with ``stretch`` [K, 1, 2] f64 (lo, hi) (bit-identical to
+    ``stretch_apply``), or none.  Without ``dst`` row r is written to row r of a new [len(sel), K] f64 tensor; with it
+    (int64, one per ``sel``, each in [0, rows); checked on the host, one synchronisation) into ``out`` [rows, K] f64,
+    whose other rows keep what the caller put there."""
+    xs, K, n, ks, _ = _series(planes, "planes", "planar")
+    ix = _cuda(idx, "idx", torch.int32).contiguous()
+    se = _cuda(sel, "sel", torch.int64).contiguous()
+    ns = se.numel()
+    st = _stretch_arg(stretch, K, 1, "stretch")
+    ds = None
+    if dst is not None:
+        ds = _cuda(dst, "dst", torch.int64).contiguous()
+        if ds.numel() != ns:
+            raise ValueError("dst must hold one row per sel entry")
+        if out is None:
+            raise ValueError("dst= writes into a caller's out= buffer")
+        if ns:
+            lo, hi = (int(v) for v in torch.aminmax(ds))
+            if lo < 0 or hi >= out.shape[0]:
+                raise IndexError(f"dst holds rows in [{lo}, {hi}], out has {out.shape[0]} rows")
+    with torch.cuda.device_of(xs):
+        if out is None:
+            out = torch.empty((ns, K), dtype=torch.float64, device=xs.device)
+        _cuda(out, "out", torch.float64)
+        if out.dim() != 2 or out.shape[1] != K or not out.is_contiguous() or (ds is None and out.shape[0] < ns):
+            raise ValueError(f"out must be a contiguous [rows, K={K}] f64 tensor")
+        _lib.check(_lib.lib().hsr_gather_planes_f64(xs.data_ptr(), ks, K, ix.data_ptr(), se.data_ptr(), _ptr(ds), ns,
+                                                    _ptr(st), out.data_ptr(), _stream()))
+    return out
+
+
 def sinkhorn_barycentric(X: torch.Tensor, Y: torch.Tensor, reg: float = 0.05, numItermax: int = 300,
                          stopThr: float = 1e-6):
     """``Ybar = (P @ Y) / (P.sum(1) + 1e-32)``, ``P = ot.sinkhorn(1/ns, 1/nt, ot.dist(X, Y), reg, ...)``
-    (poly_regression.py:49-56), fp64.  X [ns, C], Y [nt, C] f64.
+    (poly_regression.py:49-56), fp64.  X [ns, C], Y [nt, C] f64, C <= 16 (hsr_sinkhorn_barycentric_k_f64; C <= 4 runs
+    the kernels of hsr_sinkhorn_barycentric_f64, bit for bit).
     Returns ``(Ybar [ns, C] f64, info f64[4] = (iteration used, last error, iteration of that check, numerical flag))``."""
     Xd = _cuda(X, "X", torch.float64).contiguous()
     Yd = _cuda(Y, "Y", torch.float64).contiguous()
@@ -896,16 +963,16 @@ def sinkhorn_barycentric(X: torch.Tensor, Y: torch.Tensor, reg: float = 0.05, nu
         work, wptr = _aligned_workspace(_lib.lib().hsr_sinkhorn_workspace_bytes(ns, nt), Xd.device)
         ybar = torch.empty((ns, C), dtype=torch.float64, device=Xd.device)
         info = torch.zeros(4, dtype=torch.float64, device=Xd.device)
-        _lib.check(_lib.lib().hsr_sinkhorn_barycentric_f64(Xd.data_ptr(), Yd.data_ptr(), ns, nt, C, float(reg),
-                                                           int(numItermax), float(stopThr), wptr, ybar.data_ptr(),
-                                                           info.data_ptr(), _stream()))
+        _lib.check(_lib.lib().hsr_sinkhorn_barycentric_k_f64(Xd.data_ptr(), Yd.data_ptr(), ns, nt, C, float(reg),
+                                                             int(numItermax), float(stopThr), wptr, ybar.data_ptr(),
+                                                             info.data_ptr(), _stream()))
         work.record_stream(torch.cuda.current_stream())
     return ybar, info
 
 
-def polyfit_f64(x: torch.Tensor, y: torch.Tensor, deg: int, min_count: int = 0, return_moments: bool = False):
-    """``coeffs[c] = np.polyfit(x[:, c], y[:, c], deg)`` for the columns of two [n, S] f64 arrays
-    (poly_regression.py:58-60): fp64 moments + the warp solve."""
+def polyfit_moments_f64(x: torch.Tensor, y: torch.Tensor, deg: int) -> torch.Tensor:
+    """The [S, 3*deg+2] fp64 normal-equation moments of the columns of two [n, S] f64 arrays
+    (hsr_polyfit_moments_f64in; the layout ``poly_solve`` / ``poly_solve_apply`` take)."""
     xd = _cuda(x, "x", torch.float64).contiguous()
     yd = _cuda(y, "y", torch.float64).contiguous()
     if xd.shape != yd.shape or xd.dim() != 2:
@@ -915,6 +982,13 @@ def polyfit_f64(x: torch.Tensor, y: torch.Tensor, deg: int, min_count: int = 0, 
         mom = torch.empty((S, 3 * int(deg) + 2), dtype=torch.float64, device=xd.device)
         _lib.check(_lib.lib().hsr_polyfit_moments_f64in(xd.data_ptr(), yd.data_ptr(), n, S, int(deg), mom.data_ptr(),
                                                         _stream()))
+    return mom
+
+
+def polyfit_f64(x: torch.Tensor, y: torch.Tensor, deg: int, min_count: int = 0, return_moments: bool = False):
+    """``coeffs[c] = np.polyfit(x[:, c], y[:, c], deg)`` for the columns of two [n, S] f64 arrays
+    (poly_regression.py:58-60): fp64 moments + the warp solve."""
+    mom = polyfit_moments_f64(x, y, deg)
     co = poly_solve(mom, deg, min_count)
     return (co, mom) if return_moments else co
 

@@ -16,6 +16,11 @@ of the K planes onto the S2 grid (``warp_planes``), then the same fit and solve 
 granules with an S2 target too, and ``synthesize_slab_on_s2_grid`` runs one band of target rows of a mosaic, staging only
 the ortho and raw rows that band reads.
 
+``targets="ot"`` fits the polynomial against the optimal-transport barycentric targets of the reference script
+(poly_regression.py:129-137, ``fit_ot_poly_rgb``) instead of the pixel-paired ones: a planar compaction of the fit
+mask, the sample draw on the host, a planar gather, the fp64 Sinkhorn and the moments of (X, Ybar) feeding the same
+solve / apply (``_ot_fit_apply``; DESIGN section 4.9).
+
 ``matched_fine`` takes a result to the Sentinel-2 10 m resolution as the reference script's last step does
 (poly_regression.py:150-162): bilinear x factor of the planes, mask, the stretch with the percentiles of the fine planes
 and the 60 m polynomial — a fine mask, a union select over the fine values computed on the fly, and one fused apply.
@@ -25,6 +30,7 @@ from __future__ import annotations
 from dataclasses import dataclass
 from typing import Dict, List, Optional, Sequence
 
+import numpy as np
 import torch
 
 from . import dist as hdist
@@ -35,6 +41,7 @@ from .s2_emit.srf import srf_fold_weights
 
 NO_DATA_VALUE = kernels.NO_DATA_VALUE
 STRETCH_SCOPES = ("granule", "fit")
+TARGETS = ("paired", "ot")
 
 
 def _no_reduce(t):
@@ -58,6 +65,8 @@ class PairResult:
     raw_rows: Optional[tuple] = None         # synthesize_slab: the [row0, row1) raw rows that were staged
     grid: Optional[S2Target] = None          # synthesize_on_s2_grid: the S2 grid of bands / matched / valid / fit_mask
     ortho_rows: Optional[tuple] = None       # synthesize_slab_on_s2_grid: the [row0, row1) ortho rows that were staged
+    ot_info: Optional[tuple] = None          # targets="ot": (iterations, err, err_iteration, numerical) of the Sinkhorn
+                                             # (fit_ot_poly_rgb's return_info); None for paired fits and the identity
 
 
 @dataclass
@@ -75,7 +84,9 @@ class PairSynthesizer:
 
     def __init__(self, emit_w, srf_dict: Dict[str, tuple], good_mask=None, *, deg: int = 2,
                  fill: float = NO_DATA_VALUE, min_count: int = 200, gate_band: Optional[str] = None,
-                 clip=(0.0, 1.0), y_finite: bool = False, stretch=None, stretch_scope: str = "granule", device=None):
+                 clip=(0.0, 1.0), y_finite: bool = False, stretch=None, stretch_scope: str = "granule", device=None,
+                 targets: str = "paired", n_samples: int = 5000, reg: float = 0.05, numItermax: int = 300,
+                 stopThr: float = 1e-6, seed=0):
         """``stretch=(pmin, pmax)`` inserts the shared percentile stretch of s2_emit/color.py:25-34 between the
         SRF synthesis and the fit, as the reference's script does (poly_regression.py:126-127): both images are
         stretched with their own masked percentiles, the fit and the apply then run on the stretched values
@@ -85,7 +96,16 @@ class PairSynthesizer:
         global fit (``synthesize_sharded``, ``exchange=`` / ``allreduce=True``) with a stretch raises ``ValueError``.
         "fit": over exactly the pixels the fit is taken over — one granule, each tile of ``synthesize_tiles``, or the
         union of every granule / slab on every rank of a global fit (exact: np.percentile of the concatenation, the
-        same limits on every rank)."""
+        same limits on every rank).
+
+        ``targets``: "paired" (default) fits every masked pixel against the reference at that pixel; "ot" fits against
+        the optimal-transport barycentric targets of ``fit_ot_poly_rgb`` (poly_regression.py:129-137) with its
+        ``n_samples``, ``reg``, ``numItermax``, ``stopThr`` and ``seed``, jointly over the K planes: X rows (all K planes
+        finite, after the stretch if any) and Y rows (likewise) of the fit mask, the identity when either count is
+        below ``min_count``, else ``default_rng(seed).choice`` samples of each, the fp64 Sinkhorn and the per-plane
+        polynomial of X against the targets.  A global fit (``synthesize_sharded``, ``allreduce=True``) is that fit
+        over the concatenation of every unit's rows in (rank, unit) order.  ``exchange=``, ``synthesize_tiles`` and
+        ``HostGranuleStream`` raise ``ValueError`` with "ot" (DESIGN section 4.9)."""
         if stretch_scope not in STRETCH_SCOPES:
             raise ValueError(f"stretch_scope must be one of {STRETCH_SCOPES}, got {stretch_scope!r}")
         self.device = torch.device(device) if device is not None else cuda_device()
@@ -103,6 +123,24 @@ class PairSynthesizer:
         self.y_finite = bool(y_finite)
         self.stretch = None if stretch is None else (float(stretch[0]), float(stretch[1]))
         self.stretch_scope = stretch_scope
+        if targets not in TARGETS:
+            raise ValueError(f"targets must be one of {TARGETS}, got {targets!r}")
+        self.targets = targets
+        if targets == "ot":
+            if int(n_samples) != n_samples or n_samples < 1:
+                raise ValueError(f"n_samples must be an integer >= 1, got {n_samples!r}")
+            if not (float(reg) > 0.0 and np.isfinite(reg)):
+                raise ValueError(f"reg must be a finite number > 0, got {reg!r}")
+            if int(numItermax) != numItermax or numItermax < 0:
+                raise ValueError(f"numItermax must be an integer >= 0, got {numItermax!r}")
+            if np.isnan(float(stopThr)):
+                raise ValueError("stopThr must not be NaN")
+            try:
+                np.random.default_rng(seed)
+            except (TypeError, ValueError) as e:
+                raise ValueError(f"seed {seed!r} is not a valid numpy.random.default_rng seed: {e}") from None
+        self.n_samples, self.reg, self.numItermax = int(n_samples), float(reg), int(numItermax)
+        self.stopThr, self.seed = float(stopThr), seed
 
     @property
     def K(self) -> int:
@@ -161,11 +199,18 @@ class PairSynthesizer:
 
     def _check_global(self, exchange, allreduce) -> bool:
         """Whether a call's fit is global across ranks (``exchange=`` / ``allreduce=True`` with more than one
-        process); raises for a stretch whose limits would be per granule."""
+        process); raises for a stretch whose limits would be per granule, and for ``exchange=`` with OT targets."""
+        self._no_ot_exchange(exchange)
         global_fit = (exchange is not None and exchange.world > 1) or (allreduce and hdist.world()[1] > 1)
         if global_fit:
             self._no_global_stretch("exchange= / allreduce=True")
         return global_fit
+
+    def _no_ot_exchange(self, exchange) -> None:
+        """The peer exchange carries moment sums; an OT fit forms no per-rank moments that could be summed."""
+        if exchange is not None and self.targets == "ot":
+            raise ValueError("exchange= cannot carry an OT fit (targets=\"ot\"): the peer exchange sums moments, and the "
+                             "OT targets are drawn over the union of every rank's rows; use allreduce=True / group=")
 
     def _global_reduce(self, group):
         """The SUM all-reduce of the percentile histograms of a global fit (None for one process)."""
@@ -208,6 +253,9 @@ class PairSynthesizer:
     def _fit_apply(self, bands, s2_ref, valid, fm, diag, *, matched_out=None, ex=None, reduce=None,
                    allreduce=False, group=None, ortho=None, grid=None) -> PairResult:
         """The tail of one image: fit (+ all-reduce), then solve / apply."""
+        if self.targets == "ot":
+            return self._ot_fit_apply([(bands, s2_ref, valid, fm, diag, ortho, grid, matched_out)], reduce=reduce,
+                                      group=group, union=allreduce)[0]
         mom, fm, xl, yl = self.fit(bands, s2_ref, valid, fm, exchange=ex, reduce=reduce)
         if allreduce and ex is None:
             hdist.allreduce_moments(mom, group)
@@ -373,6 +421,9 @@ class PairSynthesizer:
         per-tile 1-based indices, s2_ref [K, T, h, w].  One launch per stage; T*K independent fits.
         The tiles are stacked along rows; the kernel itself offsets tile t's GLT rows by t*h and keeps an entry that
         points past its own tile out of bounds (hsr_raw_view_t.batch_*), so the GLT is used as delivered."""
+        if self.targets == "ot":
+            raise ValueError("synthesize_tiles fits T * K independent pixel-paired series; OT targets (targets=\"ot\") "
+                             "are not available for tile batches")
         T, h, w, B = raw_tiles.shape
         gy = glt_y.reshape(T * h, w)
         gx = glt_x.reshape(T * h, w)
@@ -396,8 +447,10 @@ class PairSynthesizer:
         over NVLink peer memory when ``exchange`` (a ``dist.PeerExchange``) is given, else one all-reduce (NCCL /
         gloo) — and solved redundantly.  A rank that was dealt no granule still takes part in the exchange.
         With ``stretch_scope="fit"`` the stretch limits are the percentiles of every granule on every rank (their
-        histograms are summed over ``group`` with ``dist.all_reduce`` also when the moments go through ``exchange``)."""
+        histograms are summed over ``group`` with ``dist.all_reduce`` also when the moments go through ``exchange``).
+        With ``targets="ot"`` the fit is the OT fit over every granule's rows on every rank (``exchange`` raises)."""
         self._no_global_stretch("synthesize_sharded")
+        self._no_ot_exchange(exchange)
         stage = []
         for g in granules:
             target = g.get("target")
@@ -413,6 +466,9 @@ class PairSynthesizer:
             if self.stretch is not None:
                 fm = self.stretch_mask(bands, g["s2_ref"], valid, fm)
             stage.append((bands, valid, diag, fm, g["s2_ref"], target))
+        if self.targets == "ot":
+            return self._ot_fit_apply([(b, y, v, m, d, None, t, None) for b, v, d, m, y, t in stage],
+                                      reduce=self._global_reduce(group), group=group, union=True)
         xl = yl = None
         if self.stretch is not None:
             xl, yl = self.stretch_limits([(s[0], s[4], s[3]) for s in stage], self._global_reduce(group))
@@ -451,6 +507,75 @@ class PairSynthesizer:
                                   mom, None, self.band_names, xl, yl, grid=target))
         return out
 
+
+    # ------------------------------------------------------------------ OT targets
+    def _ot_fit_apply(self, units, *, reduce=None, group=None, union=False) -> List[PairResult]:
+        """The OT tail of every entry point: ``units`` = this rank's [(bands, s2_ref, valid, fit_mask, diag, ortho,
+        grid, matched_out)].  The fit mask (rebuilt with ``y_finite``), the stretch limits (over every unit and, with
+        ``reduce``, every rank), then :meth:`_ot_moments` over the union of the units (and of every rank of ``group``
+        when ``union``) and one solve / apply per unit with those moments."""
+        masks = [self.stretch_mask(u[0], u[1], u[2], u[3]) for u in units]
+        xl = yl = None
+        if self.stretch is not None:
+            xl, yl = self.stretch_limits([(u[0], u[1], m) for u, m in zip(units, masks)], reduce)
+        with torch.cuda.device(self.device):
+            mom, min_count, info = self._ot_moments([(u[0], u[1], m) for u, m in zip(units, masks)], xl, yl,
+                                                    group, union)
+            lo, hi = self.clip if self.clip is not None else (1.0, 0.0)
+            out = []
+            for (bands, s2_ref, valid, _, diag, ortho, grid, matched_out), m in zip(units, masks):
+                coeffs, matched = kernels.poly_solve_apply(bands, mom, m, self.deg, min_count=min_count, lo=lo, hi=hi,
+                                                           out=matched_out, x_stretch=xl)
+                out.append(PairResult(bands, matched, coeffs.view(self.K, self.deg + 1), valid, m.view(valid.shape), diag,
+                                      mom, ortho, self.band_names, xl, yl, grid=grid, ot_info=info))
+        return out
+
+    def _ot_moments(self, units, xl, yl, group, union):
+        """``fit_ot_poly_rgb`` over the concatenation, in (rank, unit) order, of the rows of ``units`` ([(bands,
+        s2_ref, mask)]) of this process or, with ``union``, of every rank of ``group``.  Returns ``(moments [K,
+        3*deg+2], min_count, ot_info)`` for ``poly_solve_apply``: the moments of (X, Ybar) with min_count 0, or zeros
+        with min_count 1 (the identity) when the union has fewer than ``min_count`` X or Y rows.
+
+        Each unit's rows are compacted on the device; the per-unit counts come to the host and the per-rank totals are
+        summed with one all-reduce ([world, 2], each rank filling its own row), so every rank knows where every rank's
+        rows start in the union and draws the same samples.  Each rank gathers the samples it owns into [ns, K] / [nt, K]
+        buffers prefilled with -0.0 and one SUM all-reduce assembles them: -0.0 + v == v for every v, so each row
+        arrives with its owner's bits whatever the reduction order."""
+        K, dev = self.K, self.device
+        world = hdist.group_size(group) if union else 1
+        rank = torch.distributed.get_rank(group) if world > 1 else 0
+        lists = [kernels.compact_planes_pair(b, y, m, x_stretch=xl, y_stretch=yl) for b, y, m in units]
+        cnt = torch.stack([torch.cat([cx, cy]) for _, cx, _, cy in lists]) if lists else \
+            torch.zeros((0, 2), dtype=torch.int64, device=dev)
+        tot = torch.zeros((world, 2), dtype=torch.float64, device=dev)
+        tot[rank] = cnt.sum(0).to(torch.float64)
+        if world > 1:
+            hdist.allreduce_moments(tot, group)
+        cnt_h = cnt.tolist()
+        tot_h = [[int(v) for v in row] for row in tot.tolist()]
+        nx, ny = sum(r[0] for r in tot_h), sum(r[1] for r in tot_h)
+        M = 3 * self.deg + 2
+        if nx < self.min_count or ny < self.min_count:                    # poly_regression.py:38-41
+            return torch.zeros((K, M), dtype=torch.float64, device=dev), 1, None
+        rng = np.random.default_rng(self.seed)                            # :31
+        ns, nt = min(self.n_samples, nx), min(self.n_samples, ny)
+        sel = (rng.choice(nx, size=ns, replace=False).astype(np.int64),   # :46-47
+               rng.choice(ny, size=nt, replace=False).astype(np.int64))
+        buf = torch.full(((ns + nt) * K,), -0.0, dtype=torch.float64, device=dev)
+        XY = (buf[:ns * K].view(ns, K), buf[ns * K:].view(nt, K))
+        for side in (0, 1):                                               # X from the bands, Y from the reference
+            owned = ot_owned_rows(sel[side], [r[side] for r in tot_h], rank, [c[side] for c in cnt_h])
+            for (bands, s2_ref, _), lst, (rows, local) in zip(units, lists, owned):
+                if rows.size:
+                    kernels.gather_planes_f64((bands, s2_ref)[side], lst[2 * side], torch.from_numpy(local).to(dev),
+                                              stretch=(xl, yl)[side], dst=torch.from_numpy(rows).to(dev), out=XY[side])
+        if world > 1:
+            hdist.allreduce_moments(buf, group)
+        if not units:                                                     # nothing to apply on this rank
+            return torch.zeros((K, M), dtype=torch.float64, device=dev), 1, None
+        ybar, info = kernels.sinkhorn_barycentric(XY[0], XY[1], self.reg, self.numItermax, self.stopThr)   # :49-56
+        mom = kernels.polyfit_moments_f64(XY[0], ybar, self.deg)                                            # :58-60
+        return mom, 0, tuple(info.tolist())
 
     # ------------------------------------------------------------------ the step to the finer (S2 10 m) resolution
     def matched_fine(self, results, factor: int = 6, *, group=None, out=None):
@@ -510,6 +635,21 @@ class PairSynthesizer:
         return fine[0] if single else fine
 
 
+def ot_owned_rows(sel, rank_counts, rank: int, unit_counts):
+    """The samples of a union draw that one rank's units own.  ``sel``: indices into the concatenation of every rank's
+    rows in (rank, unit) order; ``rank_counts``: rows per rank; ``unit_counts``: rows per unit of ``rank``.  Returns one
+    ``(rows, local)`` pair per unit: the positions r in ``sel`` whose row lies in that unit, and the row's index within
+    the unit (``sel[rows] - unit offset``), both int64."""
+    sel = np.asarray(sel, dtype=np.int64)
+    off = int(sum(rank_counts[:rank]))
+    out = []
+    for c in unit_counts:
+        rows = np.flatnonzero((sel >= off) & (sel < off + int(c))).astype(np.int64)
+        out.append((rows, sel[rows] - off))
+        off += int(c)
+    return out
+
+
 def _as_tensor(raw):
     """A numpy raw mosaic as a (host) tensor; tensors pass through."""
     import numpy as np
@@ -534,6 +674,10 @@ class HostGranuleStream:
 
     def __init__(self, ps: PairSynthesizer, raw_shape, ortho_shape, *, depth: int = 2, allreduce: bool = False,
                  exchange=None):
+        if ps.targets == "ot":
+            raise ValueError("HostGranuleStream overlaps upload, compute and download on three streams; an OT fit "
+                             "(targets=\"ot\") needs a host round trip per granule for the sample draw, so nothing "
+                             "would overlap: call synthesize per granule instead")
         self.ps, self.depth, self.allreduce, self.exchange = ps, int(depth), bool(allreduce), exchange
         dev = ps.device
         Hr, Wr, B = raw_shape

@@ -414,6 +414,22 @@ HSR_API int hsr_union_select_count_bilinear(const float* src, int64_t src_plane_
  *   bytes, 256-byte aligned (holds the ns x nt fp64 kernel matrix).  C <= 4.
  * hsr_polyfit_moments_f64in: normal-equation moments (layout of hsr_poly_moments_f64) of S series of n fp64
  *   samples stored [n, S] (the columns of X and ybar); solve with hsr_poly_solve_f64 -> np.polyfit of :58-60.
+ *
+ * The same stage on the K planes of a pair synthesis (PairSynthesizer(targets="ot")), padded or dense:
+ * hsr_compact_planes_pair: one count / scan / scatter over the mask and both plane sets x, y (K planes each, plane k
+ *   at x + k * x_plane_stride; strides >= n, any value when K = 1).  idx_x = row-major indices of the pixels whose mask
+ *   byte is set (mask nullable: every pixel) and whose K x values are all finite, count_x[0] = how many; idx_y /
+ *   count_y likewise for y — the two filters of :33-36, independent of each other.  x_stretch / y_stretch: nullable
+ *   [K][2] f64 (lo, hi); given, a value is judged after the percentile stretch of color.py:33 (true division, as
+ *   hsr_stretch_f32).  n < 2^31, 1 <= K <= HSR_MAX_SRF_BANDS.  workspace: hsr_compact_planes_pair_workspace_bytes(n)
+ *   bytes, 256-byte aligned.
+ * hsr_gather_planes_f64: out[dst[r], k] = (f64) s(planes[k, idx[sel[r]]]) for r < ns, k < K (out row-major with K
+ *   columns; dst nullable: row r), s the stretch of color.py:33 with stretch [K][2] (lo, hi), or none when stretch is
+ *   null — the stretched samples carry the bits of hsr_stretch_f32.  Rows of out that no r maps to are not written:
+ *   a buffer prefilled with -0.0 (the additive identity of IEEE sums: -0.0 + v == v for every v, +0.0 included) can
+ *   hold the rows one rank owns and be SUM-all-reduced into the union's rows bit for bit.
+ * hsr_sinkhorn_barycentric_k_f64: hsr_sinkhorn_barycentric_f64 for C <= HSR_MAX_SRF_BANDS channels (same workspace,
+ *   same loop).  C <= 4 runs the kernels of hsr_sinkhorn_barycentric_f64, so its results are bit-identical to it.
  */
 HSR_API size_t hsr_compact_workspace_bytes(int64_t n);
 HSR_API int hsr_compact_finite_rows(const float* img, const uint8_t* mask, int64_t n, int C, void* workspace,
@@ -426,6 +442,17 @@ HSR_API int hsr_sinkhorn_barycentric_f64(const double* X, const double* Y, int n
                                  double* info, void* stream);
 HSR_API int hsr_polyfit_moments_f64in(const double* x, const double* y, int64_t n, int S, int deg,
                               double* moments, void* stream);
+HSR_API size_t hsr_compact_planes_pair_workspace_bytes(int64_t n);
+HSR_API int hsr_compact_planes_pair(const float* x, int64_t x_plane_stride, const double* x_stretch, const float* y,
+                            int64_t y_plane_stride, const double* y_stretch, const uint8_t* mask, int64_t n,
+                            int K, void* workspace, int32_t* idx_x, int64_t* count_x, int32_t* idx_y,
+                            int64_t* count_y, void* stream);
+HSR_API int hsr_gather_planes_f64(const float* planes, int64_t plane_stride, int K, const int32_t* idx,
+                          const int64_t* sel, const int64_t* dst, int64_t ns, const double* stretch, double* out,
+                          void* stream);
+HSR_API int hsr_sinkhorn_barycentric_k_f64(const double* X, const double* Y, int ns, int nt, int C, double reg,
+                                   int num_iter_max, double stop_thr, void* workspace, double* ybar,
+                                   double* info, void* stream);
 
 /*
  * Tile validity and uint16 quantisation, tiles_helpers/utils.py (the step after orthorectification in the
