@@ -19,7 +19,10 @@ the ortho and raw rows that band reads.
 ``targets="ot"`` fits the polynomial against the optimal-transport barycentric targets of the reference script
 (poly_regression.py:129-137, ``fit_ot_poly_rgb``) instead of the pixel-paired ones: a planar compaction of the fit
 mask, the sample draw on the host, a planar gather, the fp64 Sinkhorn and the moments of (X, Ybar) feeding the same
-solve / apply (``_ot_fit_apply``; DESIGN section 4.9).
+solve / apply (``_ot_moments``; DESIGN section 4.9).
+
+Every ``synthesize*`` entry point produces its planes and masks as units and hands them to one fit-and-apply tail
+(``_fit_apply``).
 
 ``matched_fine`` takes a result to the Sentinel-2 10 m resolution as the reference script's last step does
 (poly_regression.py:150-162): bilinear x factor of the planes, mask, the stretch with the percentiles of the fine planes
@@ -27,8 +30,8 @@ and the 60 m polynomial — a fine mask, a union select over the fine values com
 """
 from __future__ import annotations
 
-from dataclasses import dataclass
-from typing import Dict, List, Optional, Sequence
+from dataclasses import dataclass, replace
+from typing import Dict, Iterable, List, Optional, Sequence
 
 import numpy as np
 import torch
@@ -77,6 +80,19 @@ class FineResult:
     factor: int
     s2_window: Optional[tuple] = None        # the target's s2_window x factor: (row, col) of the top-left fine pixel in
                                              # the S2 grid at the fine resolution (None off the S2 grid)
+
+
+@dataclass
+class _Unit:
+    """One image of a fit, as an entry point produced it: the fields of its PairResult before the fit."""
+    bands: torch.Tensor                 # [K, Ho, Wo] (tile batches: [K, T, h, w]) f32 planes
+    s2_ref: torch.Tensor
+    valid: torch.Tensor                 # shaped as the result's valid / fit_mask
+    fit_mask: torch.Tensor              # from glt_srf / warp_planes
+    diag: torch.Tensor
+    ortho: Optional[torch.Tensor] = None
+    grid: Optional[S2Target] = None
+    matched_out: Optional[torch.Tensor] = None
 
 
 class PairSynthesizer:
@@ -166,19 +182,21 @@ class PairSynthesizer:
         several streams / threads.  With a stretch: mask first, then the limits, then the moments; ``reduce``
         (a global fit with stretch_scope="fit") sums the percentile histograms across processes, so the limits are
         those of every process's masked pixels."""
+        xl = yl = None
         if self.stretch is not None:
-            fm = self.stretch_mask(bands, s2_ref, valid, fit_mask, groups=groups)
-            xl, yl = self.stretch_limits([(bands, s2_ref, fm)], reduce, groups=groups)
-            mom, fm = kernels.fit_moments(bands, s2_ref, fm, self.deg, groups=groups, mask_given=True,
-                                          x_stretch=xl, y_stretch=yl, exchange=exchange)
-            return mom, fm, xl, yl
-        if self.y_finite:
-            mom, fm = kernels.fit_moments(bands, s2_ref, valid, self.deg, groups=groups, gate_k=self.gate_k,
-                                          gate_gt=0.0, y_finite=True, exchange=exchange)
-        else:
-            mom, fm = kernels.fit_moments(bands, s2_ref, fit_mask, self.deg, groups=groups, mask_given=True,
-                                          exchange=exchange)
-        return mom, fm, None, None
+            fit_mask = self.stretch_mask(bands, s2_ref, valid, fit_mask, groups=groups)
+            xl, yl = self.stretch_limits([(bands, s2_ref, fit_mask)], reduce, groups=groups)
+        mom, fm = self._fit_moments(bands, s2_ref, valid, fit_mask, xl, yl, groups=groups, exchange=exchange)
+        return mom, fm, xl, yl
+
+    def _fit_moments(self, bands, s2_ref, valid, fit_mask, xl, yl, *, groups=1, exchange=None):
+        """``(moments, fit_mask)``: with ``y_finite`` and no stretch the moment kernel builds the mask from ``valid``
+        (no separate mask launch); otherwise ``fit_mask`` is the mask, with the stretch limits ``xl`` / ``yl`` if any."""
+        if self.y_finite and self.stretch is None:
+            return kernels.fit_moments(bands, s2_ref, valid, self.deg, groups=groups, gate_k=self.gate_k, gate_gt=0.0,
+                                       y_finite=True, exchange=exchange)
+        return kernels.fit_moments(bands, s2_ref, fit_mask, self.deg, groups=groups, mask_given=True, x_stretch=xl,
+                                   y_stretch=yl, exchange=exchange)
 
     def stretch_mask(self, bands, s2_ref, valid, fit_mask, *, groups=1):
         """The pixels the stretch percentiles and the fit are taken over (with ``y_finite``: rebuilt so that
@@ -227,8 +245,70 @@ class PairSynthesizer:
                              "stretch_scope=\"fit\" for limits over the whole fit, fit per granule, or stretch with "
                              "limits of your own before calling")
 
-    def moments(self, bands, s2_ref, fit_mask, mask_rows="auto"):
-        return kernels.poly_moments(bands, s2_ref, fit_mask, self.deg, mask_rows=mask_rows)
+    @property
+    def _clip_bounds(self) -> tuple:
+        """``(lo, hi)`` of the apply's clip; lo > hi (``clip=None``) clips nothing."""
+        return self.clip if self.clip is not None else (1.0, 0.0)
+
+    # ------------------------------------------------------------------ the fit and apply of every entry point
+    def _fit_apply(self, units: Iterable[_Unit], *, groups: int = 1, global_fit: bool = False, group=None,
+                   exchange=None, allreduce: bool = False, summed: bool = False) -> List[PairResult]:
+        """Fit and solve / apply ``units`` (this rank's images of one fit, in order) -> one PairResult per unit.
+
+        With a stretch or OT targets each unit's fit mask is taken as the unit arrives (:meth:`stretch_mask`).  The
+        stretch limits cover every unit and, with ``global_fit``, every rank of ``group``.  The moments are the one
+        unit's (``groups`` series per plane for a tile batch), the fixed-order sum of the units' with ``summed``, or
+        :meth:`_ot_moments` (over every rank of ``group`` with ``allreduce``).  Paired moments are made global by
+        ``exchange`` (a ``dist.PeerExchange``: the moment kernel, or with ``summed`` the sum, publishes; the first
+        solve / apply consumes and returns the global sums for the other units; a rank with no unit still consumes)
+        or else, with ``allreduce``, by one all-reduce over ``group``."""
+        if self.stretch is not None or self.targets == "ot":
+            units = (replace(u, fit_mask=self.stretch_mask(u.bands, u.s2_ref, u.valid, u.fit_mask, groups=groups))
+                     for u in units)
+        units = list(units)
+        ex = exchange.next() if exchange is not None and exchange.world > 1 else None
+        xl = yl = None
+        if self.stretch is not None:
+            reduce = self._global_reduce(group) if global_fit else None
+            xl, yl = self.stretch_limits([(u.bands, u.s2_ref, u.fit_mask) for u in units], reduce, groups=groups)
+        min_count, info = self.min_count, None
+        with torch.cuda.device(self.device):
+            if self.targets == "ot":
+                mom, min_count, info = self._ot_moments([(u.bands, u.s2_ref, u.fit_mask) for u in units], xl, yl,
+                                                        group, allreduce)
+            else:
+                moms = []
+                for u in units:
+                    m, u.fit_mask = self._fit_moments(u.bands, u.s2_ref, u.valid, u.fit_mask, xl, yl, groups=groups,
+                                                      exchange=None if summed else ex)
+                    moms.append(m)
+                if summed:
+                    like = torch.empty((self.K, 3 * self.deg + 2), dtype=torch.float64, device=self.device)
+                    mom = kernels.moments_sum([m.view(self.K, -1) for m in moms], like=like, exchange=ex)
+                else:
+                    (mom,) = moms
+                if allreduce and ex is None:
+                    hdist.allreduce_moments(mom, group)
+            lo, hi = self._clip_bounds
+            if ex is not None and not units:
+                # nothing to apply here, but the exchange must be consumed (the slot parity protocol lets a rank run at
+                # most one epoch ahead of its own consumption)
+                x0 = torch.zeros((self.K, 1), dtype=torch.float32, device=self.device)
+                m0 = torch.zeros(1, dtype=torch.uint8, device=self.device)
+                kernels.poly_solve_apply(x0, mom, m0, self.deg, min_count=min_count, lo=lo, hi=hi, exchange=ex)
+            out = []
+            for u in units:
+                gmom = torch.empty_like(mom) if ex is not None else None
+                coeffs, matched = kernels.poly_solve_apply(u.bands, mom, u.fit_mask, self.deg, groups=groups,
+                                                           min_count=min_count, lo=lo, hi=hi, out=u.matched_out,
+                                                           x_stretch=xl, exchange=ex, moments_out=gmom)
+                if gmom is not None:          # the global sums: the later units solve them without the exchange
+                    mom, ex = gmom, None
+                lead = u.bands.shape[1:-2]    # (T,) for a tile batch
+                out.append(PairResult(u.bands, matched, coeffs.view(self.K, *lead, self.deg + 1), u.valid,
+                                      u.fit_mask.view(u.valid.shape), u.diag, mom.view(self.K, *lead, -1), u.ortho,
+                                      self.band_names, xl, yl, grid=u.grid, ot_info=info))
+        return out
 
     # ------------------------------------------------------------------ one granule
     def synthesize(self, raw: torch.Tensor, glt_x: torch.Tensor, glt_y: torch.Tensor, s2_ref: torch.Tensor, *,
@@ -240,33 +320,17 @@ class PairSynthesizer:
         Global fit across ranks: ``exchange`` (a ``dist.PeerExchange``: moments travel over NVLink peer memory
         inside the finalize / solve kernels) or ``allreduce=True`` (one NCCL all-reduce between the two)."""
         global_fit = self._check_global(exchange, allreduce)
+        unit = self._planes(raw, glt_x, glt_y, s2_ref, transpose_raw_yx, materialize_ortho=materialize_ortho,
+                            bands_out=bands_out, raw_row0=raw_row0, raw_rows_total=raw_rows_total)
+        unit.matched_out = matched_out
+        return self._fit_apply([unit], global_fit=global_fit, group=group, exchange=exchange, allreduce=allreduce)[0]
+
+    def _planes(self, raw, glt_x, glt_y, s2_ref, transpose_raw_yx=False, **kw) -> _Unit:
+        """glt_srf with the fit mask, on the ortho grid."""
         fm = torch.empty(glt_x.shape, dtype=torch.bool, device=raw.device)
         bands, valid, diag, ortho = self.bands_from_raw(raw, glt_x, glt_y, transpose_raw_yx=transpose_raw_yx,
-                                                        materialize_ortho=materialize_ortho, bands_out=bands_out,
-                                                        fit_mask_out=fm, raw_row0=raw_row0,
-                                                        raw_rows_total=raw_rows_total)
-        ex = exchange.next() if exchange is not None and exchange.world > 1 else None
-        reduce = self._global_reduce(group) if global_fit else None
-        return self._fit_apply(bands, s2_ref, valid, fm, diag, matched_out=matched_out, ex=ex, reduce=reduce,
-                               allreduce=allreduce, group=group, ortho=ortho)
-
-    def _fit_apply(self, bands, s2_ref, valid, fm, diag, *, matched_out=None, ex=None, reduce=None,
-                   allreduce=False, group=None, ortho=None, grid=None) -> PairResult:
-        """The tail of one image: fit (+ all-reduce), then solve / apply."""
-        if self.targets == "ot":
-            return self._ot_fit_apply([(bands, s2_ref, valid, fm, diag, ortho, grid, matched_out)], reduce=reduce,
-                                      group=group, union=allreduce)[0]
-        mom, fm, xl, yl = self.fit(bands, s2_ref, valid, fm, exchange=ex, reduce=reduce)
-        if allreduce and ex is None:
-            hdist.allreduce_moments(mom, group)
-        lo, hi = self.clip if self.clip is not None else (1.0, 0.0)
-        gmom = torch.empty_like(mom) if ex is not None else None
-        coeffs, matched = kernels.poly_solve_apply(bands, mom, fm, self.deg, min_count=self.min_count, lo=lo, hi=hi,
-                                                   out=matched_out, x_stretch=xl, exchange=ex, moments_out=gmom)
-        if gmom is not None:
-            mom = gmom
-        return PairResult(bands, matched, coeffs.view(self.K, self.deg + 1), valid, fm.view(valid.shape), diag,
-                          mom.view(self.K, -1), ortho, self.band_names, xl, yl, grid=grid)
+                                                        fit_mask_out=fm, **kw)
+        return _Unit(bands, s2_ref, valid, fm, diag, ortho)
 
     # ------------------------------------------------------------------ one granule on the Sentinel-2 grid
     def synthesize_on_s2_grid(self, raw: torch.Tensor, glt_x: torch.Tensor, glt_y: torch.Tensor, s2_ref: torch.Tensor,
@@ -286,25 +350,24 @@ class PairSynthesizer:
         in some or all of its bands is used as data (DESIGN section 7)."""
         self._check_s2_ref(s2_ref, target.shape)
         global_fit = self._check_global(exchange, allreduce)
-        bands, dvalid, fm, diag = self._planes_on_grid(raw, glt_x, glt_y, target, transpose_raw_yx, bands_out)
-        ex = exchange.next() if exchange is not None and exchange.world > 1 else None
-        reduce = self._global_reduce(group) if global_fit else None
-        return self._fit_apply(bands, s2_ref, dvalid, fm, diag, matched_out=matched_out, ex=ex, reduce=reduce,
-                               allreduce=allreduce, group=group, grid=target)
+        unit = self._planes_on_grid(raw, glt_x, glt_y, s2_ref, target, transpose_raw_yx, bands_out)
+        unit.matched_out = matched_out
+        return self._fit_apply([unit], global_fit=global_fit, group=group, exchange=exchange, allreduce=allreduce)[0]
 
     def _check_s2_ref(self, s2_ref, shape) -> None:
         Hd, Wd = shape
         if tuple(s2_ref.shape) != (self.K, Hd, Wd):
             raise ValueError(f"s2_ref must be [K={self.K}, {Hd}, {Wd}] on the target grid, got {tuple(s2_ref.shape)}")
 
-    def _planes_on_grid(self, raw, glt_x, glt_y, target: S2Target, transpose_raw_yx=False, bands_out=None):
-        """glt_srf, then the plane warp onto ``target``: (bands, dst_valid, fit_mask, diag)."""
+    def _planes_on_grid(self, raw, glt_x, glt_y, s2_ref, target: S2Target, transpose_raw_yx=False,
+                        bands_out=None) -> _Unit:
+        """glt_srf, then the plane warp onto ``target``."""
         src, valid, diag, _ = self.bands_from_raw(raw, glt_x, glt_y, transpose_raw_yx=transpose_raw_yx)
         fm = torch.empty(target.shape, dtype=torch.bool, device=src.device)
         bands, dvalid, fm = kernels.warp_planes(src, valid, target.coords(src.device), target.scales,
                                                 kernel=target.kernel, fill_out=self.fill_out, gate_k=self.gate_k,
                                                 gate_gt=0.0, out=bands_out, fit_mask_out=fm)
-        return bands, dvalid, fm, diag
+        return _Unit(bands, s2_ref, dvalid, fm, diag, grid=target)
 
     # ------------------------------------------------------------------ a row slab of a mosaic
     def synthesize_slab(self, raw, glt_x: torch.Tensor, glt_y: torch.Tensor, s2_ref: torch.Tensor, *,
@@ -318,23 +381,19 @@ class PairSynthesizer:
         reference planes.  ``stage``: optional preallocated CUDA buffer the window is copied into (flat f32, at least
         rows * Wr * B elements).  Other keywords as :meth:`synthesize` (``exchange=`` / ``allreduce=`` make the fit
         global over the slabs).  The result's ``raw_rows`` holds the staged [row0, row1) range."""
+        with torch.cuda.device(self.device):
+            win, lo, hi, d0 = self._stage_raw(raw, glt_x, glt_y, transpose_raw_yx, stage)
+            res = self.synthesize(win, glt_x, glt_y, s2_ref, transpose_raw_yx=transpose_raw_yx, raw_row0=lo,
+                                  raw_rows_total=d0, **kw)
+            return _slab_checked(res, (lo, hi))
+
+    def _stage_raw(self, raw, glt_x, glt_y, transpose_raw_yx, stage):
+        """(window on the device, lo, hi, raw rows): the raw rows [lo, hi) of ``raw`` (a numpy array or a host / CUDA
+        tensor of ``raw rows`` rows) that the GLT rows reference, copied into ``stage`` (or a new device buffer) when
+        ``raw`` is in host memory."""
         raw = _as_tensor(raw)
         d0, d1 = int(raw.shape[0]), int(raw.shape[1])
         Hr, Wr = (d1, d0) if transpose_raw_yx else (d0, d1)
-        with torch.cuda.device(self.device):
-            lo, hi, win = self._stage_raw(raw, glt_x, glt_y, Hr, Wr, transpose_raw_yx, stage)
-            res = self.synthesize(win, glt_x, glt_y, s2_ref, transpose_raw_yx=transpose_raw_yx, raw_row0=lo,
-                                  raw_rows_total=d0, **kw)
-            outside = int(res.diag[3])
-            if outside:
-                raise RuntimeError(f"{outside} valid GLT entries fell outside the staged raw rows [{lo}, {hi})")
-        res.diag = res.diag[:3]
-        res.raw_rows = (lo, hi)
-        return res
-
-    def _stage_raw(self, raw, glt_x, glt_y, Hr, Wr, transpose_raw_yx, stage):
-        """(lo, hi, window on the device): the raw rows [lo, hi) the GLT rows reference, copied into ``stage`` (or a
-        new device buffer) when ``raw`` is in host memory."""
         lo, hi = kernels.glt_row_range(glt_x, glt_y, Hr, Wr, transpose_raw_yx=transpose_raw_yx).tolist()
         if hi == 0:                       # no valid entry in this slab: any one row will do
             lo, hi = 0, 1
@@ -347,7 +406,7 @@ class PairSynthesizer:
             dst = buf.view(-1)[:n].view(win.shape)
             dst.copy_(win, non_blocking=win.is_pinned())
             win = dst
-        return lo, hi, win
+        return win, lo, hi, d0
 
     # ------------------------------------------------------------------ a row band of a mosaic on the Sentinel-2 grid
     def synthesize_slab_on_s2_grid(self, raw, glt_x: torch.Tensor, glt_y: torch.Tensor, s2_ref: torch.Tensor,
@@ -378,9 +437,6 @@ class PairSynthesizer:
             raise ValueError(f"rows must satisfy 0 <= t0 < t1 <= {Hd}, got {tuple(rows)}")
         self._check_s2_ref(s2_ref, (t1 - t0, Wd))
         global_fit = self._check_global(exchange, allreduce)
-        raw = _as_tensor(raw)
-        d0, d1 = int(raw.shape[0]), int(raw.shape[1])
-        Hr, Wr = (d1, d0) if transpose_raw_yx else (d0, d1)
         Ho, Wo = glt_x.shape
         with torch.cuda.device(self.device):
             coords = target.coords(self.device, rows=(t0, t1))
@@ -392,7 +448,7 @@ class PairSynthesizer:
                 diag = torch.zeros(4, dtype=torch.int64, device=self.device)
             else:
                 gx, gy = glt_x[o0:o1], glt_y[o0:o1]
-                lo, hi, win = self._stage_raw(raw, gx, gy, Hr, Wr, transpose_raw_yx, stage)
+                win, lo, hi, d0 = self._stage_raw(raw, gx, gy, transpose_raw_yx, stage)
                 src, valid, diag, _ = self.bands_from_raw(win, gx, gy, transpose_raw_yx=transpose_raw_yx, raw_row0=lo,
                                                           raw_rows_total=d0)
             outside = torch.zeros(1, dtype=torch.int64, device=self.device)
@@ -400,19 +456,9 @@ class PairSynthesizer:
             bands, dvalid, fm = kernels.warp_planes(src, valid, coords, target.scales, kernel=target.kernel,
                                                     fill_out=self.fill_out, gate_k=self.gate_k, gate_gt=0.0,
                                                     fit_mask_out=fm, src_row0=o0, src_rows_total=Ho, outside=outside)
-            ex = exchange.next() if exchange is not None and exchange.world > 1 else None
-            reduce = self._global_reduce(group) if global_fit else None
-            res = self._fit_apply(bands, s2_ref, dvalid, fm, diag, ex=ex, reduce=reduce, allreduce=allreduce,
-                                  group=group, grid=target)
-            raw_missed, tap_missed = torch.cat([res.diag[3:], outside]).tolist()
-            if raw_missed:
-                raise RuntimeError(f"{raw_missed} valid GLT entries fell outside the staged raw rows [{lo}, {hi})")
-            if tap_missed:
-                raise RuntimeError(f"{tap_missed} target pixels needed ortho rows outside the staged rows [{o0}, {o1})")
-        res.diag = res.diag[:3]
-        res.raw_rows = (lo, hi)
-        res.ortho_rows = (o0, o1)
-        return res
+            res = self._fit_apply([_Unit(bands, s2_ref, dvalid, fm, diag, grid=target)], global_fit=global_fit,
+                                  group=group, exchange=exchange, allreduce=allreduce)[0]
+            return _slab_checked(res, (lo, hi), (o0, o1), outside)
 
     # ------------------------------------------------------------------ a batch of equal tiles
     def synthesize_tiles(self, raw_tiles: torch.Tensor, glt_x: torch.Tensor, glt_y: torch.Tensor,
@@ -425,18 +471,11 @@ class PairSynthesizer:
             raise ValueError("synthesize_tiles fits T * K independent pixel-paired series; OT targets (targets=\"ot\") "
                              "are not available for tile batches")
         T, h, w, B = raw_tiles.shape
-        gy = glt_y.reshape(T * h, w)
-        gx = glt_x.reshape(T * h, w)
-        raw = raw_tiles.reshape(T * h, w, B)
-        fm = torch.empty(gx.shape, dtype=torch.bool, device=raw.device)
-        bands, valid, diag, _ = self.bands_from_raw(raw, gx, gy, fit_mask_out=fm, tile_rows=(h, h))   # [K, T*h, w]
-        diag = diag[:3]
-        mom, fm, xl, yl = self.fit(bands, s2_ref, valid, fm.view(T, h * w), groups=T)
-        lo, hi = self.clip if self.clip is not None else (1.0, 0.0)
-        coeffs, matched = kernels.poly_solve_apply(bands, mom, fm, self.deg, groups=T, min_count=self.min_count,
-                                                   lo=lo, hi=hi, x_stretch=xl)
-        return PairResult(bands.view(self.K, T, h, w), matched.view(self.K, T, h, w), coeffs, valid.view(T, h, w),
-                          fm.view(T, h, w), diag, mom, None, self.band_names, xl, yl)
+        u = self._planes(raw_tiles.reshape(T * h, w, B), glt_x.reshape(T * h, w), glt_y.reshape(T * h, w), s2_ref,
+                         tile_rows=(h, h))
+        u = replace(u, bands=u.bands.view(self.K, T, h, w), valid=u.valid.view(T, h, w),
+                    fit_mask=u.fit_mask.view(T, h, w), diag=u.diag[:3])
+        return self._fit_apply([u], groups=T)[0]
 
     # ------------------------------------------------------------------ many granules, one global fit
     def synthesize_sharded(self, granules: Sequence[dict], *, group=None, exchange=None) -> List[PairResult]:
@@ -451,85 +490,18 @@ class PairSynthesizer:
         With ``targets="ot"`` the fit is the OT fit over every granule's rows on every rank (``exchange`` raises)."""
         self._no_global_stretch("synthesize_sharded")
         self._no_ot_exchange(exchange)
-        stage = []
-        for g in granules:
-            target = g.get("target")
-            if target is not None:
-                self._check_s2_ref(g["s2_ref"], target.shape)
-                bands, valid, fm, diag = self._planes_on_grid(g["raw"], g["glt_x"], g["glt_y"], target,
-                                                              g.get("transpose_raw_yx", False))
-            else:
-                fm = torch.empty(g["glt_x"].shape, dtype=torch.bool, device=self.device)
-                bands, valid, diag, _ = self.bands_from_raw(g["raw"], g["glt_x"], g["glt_y"],
-                                                            transpose_raw_yx=g.get("transpose_raw_yx", False),
-                                                            fit_mask_out=fm)
-            if self.stretch is not None:
-                fm = self.stretch_mask(bands, g["s2_ref"], valid, fm)
-            stage.append((bands, valid, diag, fm, g["s2_ref"], target))
-        if self.targets == "ot":
-            return self._ot_fit_apply([(b, y, v, m, d, None, t, None) for b, v, d, m, y, t in stage],
-                                      reduce=self._global_reduce(group), group=group, union=True)
-        xl = yl = None
-        if self.stretch is not None:
-            xl, yl = self.stretch_limits([(s[0], s[4], s[3]) for s in stage], self._global_reduce(group))
-        moms = []
-        for i, (bands, valid, diag, fm, s2_ref, target) in enumerate(stage):
-            if self.stretch is not None:
-                mom, _ = kernels.fit_moments(bands, s2_ref, fm, self.deg, mask_given=True, x_stretch=xl, y_stretch=yl)
-            else:
-                mom, fm, _, _ = self.fit(bands, s2_ref, valid, fm)
-            moms.append(mom.view(self.K, -1))
-            stage[i] = (bands, valid, diag, fm, target)
-        ex = exchange.next() if exchange is not None and exchange.world > 1 else None
-        like = torch.empty((self.K, 3 * self.deg + 2), dtype=torch.float64, device=self.device)
-        with torch.cuda.device(self.device):
-            mom = kernels.moments_sum(moms, like=like, exchange=ex)
-        if ex is None:
-            hdist.allreduce_moments(mom, group)
-        lo, hi = self.clip if self.clip is not None else (1.0, 0.0)
-        out = []
-        if ex is not None and not stage:
-            # nothing to apply here, but the exchange must be consumed (the slot parity protocol lets a rank run at
-            # most one epoch ahead of its own consumption)
-            x0 = torch.zeros((self.K, 1), dtype=torch.float32, device=self.device)
-            m0 = torch.zeros(1, dtype=torch.uint8, device=self.device)
-            kernels.poly_solve_apply(x0, mom, m0, self.deg, min_count=self.min_count, lo=lo, hi=hi, exchange=ex)
-        for i, (bands, valid, diag, fm, target) in enumerate(stage):
-            if i == 0 and ex is not None:
-                gmom = torch.empty_like(mom)
-                coeffs, matched = kernels.poly_solve_apply(bands, mom, fm, self.deg, min_count=self.min_count, lo=lo,
-                                                           hi=hi, x_stretch=xl, exchange=ex, moments_out=gmom)
-                mom = gmom.view(self.K, -1)
-            else:
-                coeffs, matched = kernels.poly_solve_apply(bands, mom, fm, self.deg, min_count=self.min_count, lo=lo,
-                                                           hi=hi, x_stretch=xl)
-            out.append(PairResult(bands, matched, coeffs.view(self.K, self.deg + 1), valid, fm.view(valid.shape), diag,
-                                  mom, None, self.band_names, xl, yl, grid=target))
-        return out
 
+        def unit(g):
+            target, tr = g.get("target"), g.get("transpose_raw_yx", False)
+            if target is None:
+                return self._planes(g["raw"], g["glt_x"], g["glt_y"], g["s2_ref"], tr)
+            self._check_s2_ref(g["s2_ref"], target.shape)
+            return self._planes_on_grid(g["raw"], g["glt_x"], g["glt_y"], g["s2_ref"], target, tr)
+        # a generator: each granule's fit mask is taken right after its planes
+        return self._fit_apply((unit(g) for g in granules), global_fit=True, group=group, exchange=exchange,
+                               allreduce=True, summed=True)
 
     # ------------------------------------------------------------------ OT targets
-    def _ot_fit_apply(self, units, *, reduce=None, group=None, union=False) -> List[PairResult]:
-        """The OT tail of every entry point: ``units`` = this rank's [(bands, s2_ref, valid, fit_mask, diag, ortho,
-        grid, matched_out)].  The fit mask (rebuilt with ``y_finite``), the stretch limits (over every unit and, with
-        ``reduce``, every rank), then :meth:`_ot_moments` over the union of the units (and of every rank of ``group``
-        when ``union``) and one solve / apply per unit with those moments."""
-        masks = [self.stretch_mask(u[0], u[1], u[2], u[3]) for u in units]
-        xl = yl = None
-        if self.stretch is not None:
-            xl, yl = self.stretch_limits([(u[0], u[1], m) for u, m in zip(units, masks)], reduce)
-        with torch.cuda.device(self.device):
-            mom, min_count, info = self._ot_moments([(u[0], u[1], m) for u, m in zip(units, masks)], xl, yl,
-                                                    group, union)
-            lo, hi = self.clip if self.clip is not None else (1.0, 0.0)
-            out = []
-            for (bands, s2_ref, valid, _, diag, ortho, grid, matched_out), m in zip(units, masks):
-                coeffs, matched = kernels.poly_solve_apply(bands, mom, m, self.deg, min_count=min_count, lo=lo, hi=hi,
-                                                           out=matched_out, x_stretch=xl)
-                out.append(PairResult(bands, matched, coeffs.view(self.K, self.deg + 1), valid, m.view(valid.shape), diag,
-                                      mom, ortho, self.band_names, xl, yl, grid=grid, ot_info=info))
-        return out
-
     def _ot_moments(self, units, xl, yl, group, union):
         """``fit_ot_poly_rgb`` over the concatenation, in (rank, unit) order, of the rows of ``units`` ([(bands,
         s2_ref, mask)]) of this process or, with ``union``, of every rank of ``group``.  Returns ``(moments [K,
@@ -624,7 +596,7 @@ class PairSynthesizer:
                 xl = kernels.masked_percentiles_union([(r.bands, m) for r, m in zip(rs, masks)], self.stretch,
                                                       reduce=reduce or _no_reduce, K=self.K, pair=False,
                                                       device=self.device, factor=f)
-            lo, hi = self.clip if self.clip is not None else (1.0, 0.0)
+            lo, hi = self._clip_bounds
             fine = []
             for r, m, o in zip(rs, masks, outs):
                 matched, _ = kernels.bilinear_apply(r.bands, f, r.coeffs, x_stretch=xl, lo=lo, hi=hi, out=o, mask_out=m)
@@ -652,9 +624,22 @@ def ot_owned_rows(sel, rank_counts, rank: int, unit_counts):
 
 def _as_tensor(raw):
     """A numpy raw mosaic as a (host) tensor; tensors pass through."""
-    import numpy as np
-
     return torch.from_numpy(raw) if isinstance(raw, np.ndarray) else raw
+
+
+def _slab_checked(res: PairResult, raw_rows: tuple, ortho_rows: Optional[tuple] = None,
+                  outside: Optional[torch.Tensor] = None) -> PairResult:
+    """A row slab's result: raises ``RuntimeError`` when a valid GLT entry (``diag[3]``) or, on the S2 grid, a filter
+    tap (``outside``) fell outside the staged rows — only now, after the fit and apply, so that no rank is left waiting
+    in the exchange — then keeps the three GLT diagnostics and records the staged ranges."""
+    raw_missed, *tap_missed = torch.cat([res.diag[3:]] + ([outside] if outside is not None else [])).tolist()
+    if raw_missed:
+        raise RuntimeError(f"{raw_missed} valid GLT entries fell outside the staged raw rows [{raw_rows[0]}, {raw_rows[1]})")
+    if tap_missed and tap_missed[0]:
+        raise RuntimeError(f"{tap_missed[0]} target pixels needed ortho rows outside the staged rows "
+                           f"[{ortho_rows[0]}, {ortho_rows[1]})")
+    res.diag, res.raw_rows, res.ortho_rows = res.diag[:3], raw_rows, ortho_rows
+    return res
 
 
 class HostGranuleStream:
